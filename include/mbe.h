@@ -173,7 +173,8 @@ int mbe_abi_version(void);
 const char* mbe_build_info(void);
 const char* mbe_last_error(void);
 /* sizeof of the ABI structs as the library was compiled (0 mbe_config, 1 mbe_buffers, 2 mbe_link_class,
- * 3 mbe_ue_class, 4 mbe_rollout_out; -1 otherwise): lets a binding in another language check its layout */
+ * 3 mbe_ue_class, 4 mbe_rollout_out, 5 mbe_render_style; -1 otherwise): lets a binding in another
+ * language check its layout */
 int mbe_struct_size(int which);
 
 /* replaces MComCore.__init__ (base.py:32-100): validates, copies the constant tables */
@@ -226,6 +227,23 @@ typedef struct mbe_rollout_out {
  * what `steps` calls of mbe_step would have left.  Shapes without the fused kernel run the same
  * episode as a sequence of step launches (same results). */
 int mbe_rollout(mbe_env* env, int steps, float* qoe_acc, float threshold, const mbe_rollout_out* out, void* stream);
+
+/* Map-panel frames (DESIGN.md section 9).  palette rows: 0 background, 1..3 coverage by 1 / 2 / >= 3
+ * BSs, 4 BS square, 5 unconnected UE, 6..261 utility ramp (index clamp(floor((u + 1) * 128), 0, 255)). */
+enum { MBE_RENDER_PALETTE = 262, MBE_RENDER_MAX_STYLE_PX = 64 };
+typedef struct mbe_render_style {
+  int32_t height, width;                  /* 8..4096, width % 4 == 0 */
+  int32_t ue_radius, bs_half, line_width; /* pixels, 0..MBE_RENDER_MAX_STYLE_PX */
+  uint8_t palette[MBE_RENDER_PALETTE][3]; /* RGB */
+} mbe_render_style;
+
+/* Frames of envs env_ids[0..n) (DEVICE int32, NULL = envs 0..n-1) into out uint8 [steps, n, H, W, 3]
+ * (DEVICE, 4-byte aligned), one launch.  series == NULL: the bound state (steps must be 1).
+ * series != NULL (FORK): the pos / assoc / utility series [steps, E, U(,2)] that mbe_rollout wrote,
+ * one frame per step.  BS layouts, nbs and link classes are the handle's bound ones, so a series
+ * should not cross an episode boundary.  An env id outside 0..E-1 gives a background-only frame. */
+int mbe_render(mbe_env* env, const int32_t* env_ids, int n, const mbe_rollout_out* series, int steps,
+               const mbe_render_style* style, uint8_t* out, void* stream);
 
 /* number of kernel launches this handle has enqueued so far */
 int64_t mbe_launch_count(const mbe_env* env);

@@ -20,6 +20,7 @@ MAX_UE_CLASSES = 8
 FLAG_GENERIC_KERNEL = 1
 FLAG_SHARED_TRAJECTORY = 2
 PHASE_MOVE, PHASE_PRE, PHASE_CLOCK, PHASE_POST, PHASE_ALL = 1, 2, 4, 8, 15
+RENDER_PALETTE = 262
 
 
 class BsClass(C.Structure):
@@ -108,6 +109,13 @@ class RolloutOut(C.Structure):
                 ("utility", C.c_void_p)]
 
 
+class RenderStyle(C.Structure):
+    """mbe_render_style: frame size, entity sizes in pixels and the palette (rows: see render.py)."""
+
+    _fields_ = [("height", C.c_int32), ("width", C.c_int32), ("ue_radius", C.c_int32), ("bs_half", C.c_int32),
+                ("line_width", C.c_int32), ("palette", (C.c_uint8 * 3) * RENDER_PALETTE)]
+
+
 # every symbol include/mbe.h declares: (name, restype, argtypes)
 SYMBOLS = [
     ("mbe_abi_version", C.c_int, []),
@@ -125,6 +133,8 @@ SYMBOLS = [
     ("mbe_observe", C.c_int, [C.c_void_p, C.c_void_p]),
     ("mbe_accumulate_qoe", C.c_int, [C.c_void_p, C.c_void_p, C.c_float, C.c_void_p]),
     ("mbe_rollout", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_float, C.POINTER(RolloutOut), C.c_void_p]),
+    ("mbe_render", C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(RolloutOut), C.c_int,
+                             C.POINTER(RenderStyle), C.c_void_p, C.c_void_p]),
     ("mbe_launch_count", C.c_int64, [C.c_void_p]),
     ("mbe_step_kernel_name", C.c_char_p, [C.c_void_p]),
     ("mbe_step_host", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -154,7 +164,7 @@ def load():
         fn.argtypes = args
     if lib.mbe_abi_version() != MBE_ABI_VERSION:
         raise MbeError(f"libmbe ABI {lib.mbe_abi_version()} != binding {MBE_ABI_VERSION}")
-    for which, struct in enumerate((Config, Buffers, BsClass, UeClass, RolloutOut)):
+    for which, struct in enumerate((Config, Buffers, BsClass, UeClass, RolloutOut, RenderStyle)):
         if lib.mbe_struct_size(which) != C.sizeof(struct):
             raise MbeError(f"struct layout mismatch: {struct.__name__} is {C.sizeof(struct)} bytes here, "
                            f"{lib.mbe_struct_size(which)} in {LIB_PATH}")

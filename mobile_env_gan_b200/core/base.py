@@ -253,7 +253,7 @@ class MComCore:
     # ---------------------------------------------------------------------- construction --
     def __init__(self, stations: List[BaseStation], users: List[UserEquipment], config=None, render_mode=None):
         assert render_mode in self.metadata["render_modes"] + [None]
-        self.render_mode = render_mode  # rendering is out of scope (base.py:466-753)
+        self.render_mode = render_mode  # "rgb_array": render() returns env 0's map panel (render_frames)
         config = deep_dict_merge(self.default_config(), config or {})
         config = self.seeding(config)
         self.config = config
@@ -621,6 +621,48 @@ class MComCore:
         ptr = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
         _lib.check(self._lib.mbe_step_host(self._handle, ptr(actions_host), ptr(obs_host), ptr(reward_host),
                                            ptr(done_host), self._stream()))
+
+    def render(self):
+        """Gymnasium ``render``: with ``render_mode="rgb_array"`` env 0's map panel as numpy uint8
+        ``[H, W, 3]`` (slow path: synchronises and copies, like ``view``); ``None`` without a render mode.
+        The reference's metric dashboard is not drawn (DESIGN.md section 9)."""
+        if self.render_mode is None:
+            return None
+        if self.render_mode == "human":
+            raise NotImplementedError('render_mode="human" needs a display backend, which this build does not have; '
+                                      'use "rgb_array" and show the frames yourself')
+        return self.render_frames([0])[0].cpu().numpy()
+
+    def render_frames(self, envs=None, size=None, series=None):
+        """Map-panel frames in one launch (``mbe_render``), as a device tensor uint8 ``[N, H, W, 3]`` of the
+        current state of ``envs`` (index tensor or list, default all), or ``[T, N, H, W, 3]`` from ``series``,
+        the dict of ``rollout(..., record=("pos", "assoc", "utility"))`` (FORK mode).  ``size`` = (height,
+        width) pixels (default ``render.DEFAULT_SIZE``).  Series frames use the BS layouts bound now, so a
+        series should stay within one episode (with ``autoreset`` the step that ends it draws new layouts)."""
+        from .. import render as _render
+
+        if envs is None:
+            n, ids = self.num_envs, None
+        else:
+            ids = torch.as_tensor(envs).to(device=self.device, dtype=torch.int32).reshape(-1).contiguous()
+            n = ids.numel()
+            if n == 0:
+                raise ValueError("render_frames: envs is empty")
+            if bool(((ids < 0) | (ids >= self.num_envs)).any()):
+                raise IndexError(f"render_frames: env ids must lie in 0..{self.num_envs - 1}")
+        st = _render.style(size)
+        steps, ro = 1, None
+        if series is not None:
+            ro = _lib.RolloutOut()
+            for name in ("pos", "assoc", "utility"):
+                if name in series:
+                    setattr(ro, name, series[name].data_ptr())
+            steps = int(next(iter(series.values())).shape[0]) if series else 0
+        out = torch.empty((max(steps, 1), n, st.height, st.width, 3), dtype=torch.uint8, device=self.device)
+        _lib.check(self._lib.mbe_render(self._handle, None if ids is None else C.c_void_p(ids.data_ptr()), int(n),
+                                        None if ro is None else C.byref(ro), int(steps), C.byref(st),
+                                        C.c_void_p(out.data_ptr()), self._stream()))
+        return out if series is not None else out[0]
 
     @property
     def launch_count(self) -> int:

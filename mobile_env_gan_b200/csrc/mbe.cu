@@ -18,6 +18,7 @@
 #include "mbe_step_upt.cuh"
 #include "mbe_step_tpe.cuh"
 #include "mbe_host_wire.cuh"
+#include "mbe_render.cuh"
 
 #include <memory>
 #include <sched.h>
@@ -186,6 +187,7 @@ int mbe_struct_size(int which) {
     case 2: return (int)sizeof(mbe_link_class);
     case 3: return (int)sizeof(mbe_ue_class);
     case 4: return (int)sizeof(mbe_rollout_out);
+    case 5: return (int)sizeof(mbe_render_style);
     default: return -1;
   }
 }
@@ -836,6 +838,57 @@ int mbe_rollout(mbe_env* env, int steps, float* qoe_acc, float threshold, const 
     if (o.rate) MBE_CUDA(cudaMemcpyAsync(o.rate + EU * s, a0.rate, EU * 8, cudaMemcpyDeviceToDevice, st));
     if (o.utility) MBE_CUDA(cudaMemcpyAsync(o.utility + EU * s, a0.utility, EU * 4, cudaMemcpyDeviceToDevice, st));
   }
+  return 0;
+}
+
+int mbe_render(mbe_env* env, const int32_t* env_ids, int n, const mbe_rollout_out* series, int steps,
+               const mbe_render_style* style, uint8_t* out, void* stream) {
+  if (!env || !style || !out) return fail("mbe_render: null argument");
+  if (!env->bound) return fail("mbe_bind has not been called");
+  const int H = style->height, W = style->width;
+  if (H < 8 || H > 4096 || W < 8 || W > 4096 || W % 4)
+    return fail("mbe_render: frame %d x %d out of range (8..4096 each, width a multiple of 4)", H, W);
+  const int lim = MBE_RENDER_MAX_STYLE_PX;
+  if (style->ue_radius < 0 || style->ue_radius > lim || style->bs_half < 0 || style->bs_half > lim ||
+      style->line_width < 0 || style->line_width > lim)
+    return fail("mbe_render: ue_radius, bs_half and line_width must be in 0..%d pixels", lim);
+  if (n < 1) return fail("mbe_render: n must be positive");
+  if (steps < 1) return fail("mbe_render: steps must be positive");
+  if (steps > 1 && !series) return fail("mbe_render: steps > 1 needs a series");
+  const bool gym = env->cfg.mode == MBE_MODE_GYM;
+  if (series && gym) return fail("mbe_render: series are FORK-mode only (there is no connection series in GYM mode)");
+  if (series && (!series->pos || !series->assoc || !series->utility))
+    return fail("mbe_render: a series needs pos, assoc and utility");
+  if ((uintptr_t)out & 3) return fail("mbe_render: out must be 4-byte aligned");
+  const mbe::StepArgs& s = env->args;
+  const int Wm = (int)env->cfg.width, Hm = (int)env->cfg.height;
+  if (Wm < 1 || Hm < 1) return fail("mbe_render: the map must be at least 1 x 1 in integer units");
+  mbe::RenderArgs a = {};
+  a.pos = series ? reinterpret_cast<const uint32_t*>(series->pos) : s.pos;
+  a.conn = s.conn;
+  a.assoc = series ? series->assoc : s.assoc;
+  a.utility = series ? series->utility : s.utility;
+  a.bs_xy = s.bs_xy;
+  a.nbs = s.nbs;
+  a.bs_class = s.bs_class;
+  a.env_ids = env_ids;
+  a.out = out;
+  a.step_eu = series ? (long long)s.E * s.U : 0;
+  a.E = s.E, a.U = s.U, a.B = s.B, a.MW = (s.B + 31) >> 5, a.n = n, a.gym = gym, a.bs_per_env = s.bs_per_env;
+  a.Wm = Wm, a.Hm = Hm;
+  const int nuc = s.n_ue_classes;
+  for (int c = 0; c < env->cfg.num_classes; ++c) a.cov_d2max[c] = env->cfg.classes[c * nuc].d2max;
+  a.band_rows = std::min(H, std::max(4, (mbe::kRenderBandPixels / W) & ~3));
+  a.bands = (H + a.band_rows - 1) / a.band_rows;
+  a.seg_cap = mbe::kRenderSegUes * s.B;
+  const long long blocks = (long long)steps * n * a.bands;
+  if (blocks > 0x7fffffffll) return fail("mbe_render: %lld CTAs exceed one launch", blocks);
+  const size_t smem = mbe::render_smem_layout(s.U, W, a.band_rows, a.seg_cap).total;
+  MBE_ON_DEVICE(env->cfg.device);
+  MBE_CUDA(cudaFuncSetAttribute((const void*)mbe::render_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  mbe::render_kernel<<<(unsigned)blocks, mbe::kRenderThreads, smem, static_cast<cudaStream_t>(stream)>>>(a, *style);
+  MBE_CUDA(cudaGetLastError());
+  env->launches += 1;
   return 0;
 }
 
