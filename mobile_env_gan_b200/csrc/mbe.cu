@@ -17,11 +17,7 @@
 #include "mbe_step_big.cuh"
 #include "mbe_step_upt.cuh"
 #include "mbe_step_tpe.cuh"
-#include "mbe_host_wire.cuh"
 #include "mbe_render.cuh"
-
-#include <memory>
-#include <sched.h>
 
 namespace {
 
@@ -81,9 +77,6 @@ struct mbe_env {
   // specialised fused kernel for this shape (nullptr: generic kernel only)
   void (*spec)(mbe::StepArgs) = nullptr;
   size_t spec_smem = 0;
-  void (*pipe)(mbe::StepArgs) = nullptr;
-  size_t pipe_smem = 0;
-  int pipe_grid = 0;
   bool big = false;  // block-per-env kernel (wide shapes, ProportionalFair)
   // several-UEs-per-thread kernel (GYM scenario shapes, shared layout)
   void (*upt)(mbe::StepArgs) = nullptr;
@@ -103,12 +96,6 @@ struct mbe_env {
   // mbe_step_host pipeline: second stream + fork/join events (created on first use)
   cudaStream_t host_stream = nullptr;
   cudaEvent_t host_fork = nullptr, host_join = nullptr;
-  // compact observation wire format of mbe_step_host (mbe_host_wire.cuh; created on first use)
-  mbe::WireShape wire_shape = {};
-  unsigned char* wire_dev = nullptr;     // [E * bytes_per_env]
-  unsigned char* wire_pinned = nullptr;  // the same, pinned host staging
-  std::vector<cudaEvent_t> wire_events;  // one per env window
-  std::unique_ptr<mbe::ExpandCrew> wire_pool;
 };
 
 namespace {
@@ -133,17 +120,13 @@ struct SpecEntry {
   int mode, handler, U, B, per_env;
   void (*fn)(mbe::StepArgs);
   size_t smem;
-  void (*pipe_fn)(mbe::StepArgs);  // persistent, TMA-pipelined variant (E % EPB == 0)
-  size_t pipe_smem;
-  void (*mc_fn)(mbe::StepArgs);    // several BS classes in a shared layout (nullptr for per-env layouts)
+  void (*mc_fn)(mbe::StepArgs);  // several BS classes in a shared layout (nullptr for per-env layouts)
 };
 
 #define MBE_SPEC(MODE, HANDLER, U, B, PE)                                             \
   SpecEntry {                                                                         \
     MODE, HANDLER, U, B, PE, mbe::step_spec_kernel<MODE, HANDLER, U, B, (PE != 0)>,   \
         mbe::spec_smem_bytes<HANDLER, U, B, (PE != 0)>(MODE == 1),                    \
-        mbe::step_pipe_kernel<MODE, HANDLER, U, B, (PE != 0)>,                        \
-        mbe::pipe_smem_bytes<HANDLER, U, B, (PE != 0)>(MODE == 1),                    \
         mbe::spec_mc_kernel<MODE, HANDLER, U, B, (PE != 0)>()                         \
   }
 
@@ -156,11 +139,8 @@ struct UptEntry {
 };
 #define MBE_UPT(HANDLER, U, B, K) \
   UptEntry { HANDLER, U, B, K, mbe::step_upt_kernel<HANDLER, U, B, K>, mbe::upt_smem_bytes<HANDLER, U, B, K>() }
-#ifndef MBE_UPT_K_MEDIUM
-#define MBE_UPT_K_MEDIUM 5
-#endif
 // (small 5x3 with K=1 and large 30x13 with K=10 were measured slower than one thread per UE)
-const UptEntry kUpts[] = {MBE_UPT(0, 15, 4, MBE_UPT_K_MEDIUM), MBE_UPT(1, 15, 4, MBE_UPT_K_MEDIUM)};
+const UptEntry kUpts[] = {MBE_UPT(0, 15, 4, 5), MBE_UPT(1, 15, 4, 5)};
 
 const SpecEntry kSpecs[] = {
     MBE_SPEC(1, 0, 5, 3, 0),  MBE_SPEC(1, 1, 5, 3, 0),  MBE_SPEC(1, 0, 15, 4, 0),  MBE_SPEC(1, 1, 15, 4, 0),
@@ -408,10 +388,6 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
         if (cfg->num_classes > 1 && !sp.mc_fn) break;  // per-env layouts have one class: generic kernel
         env->spec = cfg->num_classes > 1 ? sp.mc_fn : sp.fn;
         env->spec_smem = sp.smem;
-        if (a.E % a.epb == 0 && cfg->num_classes == 1) {
-          env->pipe = sp.pipe_fn;
-          env->pipe_smem = sp.pipe_smem;
-        }
         break;
       }
   }
@@ -449,13 +425,11 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
       } else if (a.U == 15 && a.B == 4) {
         env->tpe_rollout = mbe::step_tpe_fork_kernel<15, 4, true, true>;
         env->tpe_rollout_smem = sizeof(mbe::TpeRolloutSmem<15, 4>);
-      } else if (a.U == 30 && a.B == 13 && std::getenv("MBE_TPE_LARGE") && std::getenv("MBE_TPE_LARGE")[0] == '1') {
-        // opt-in: one env per lane walks 30 x 13 pairs in scalar code at 208 registers -- 1.43 ms per
-        // 20-step episode of 65,536 envs against 0.83 ms for 20 launches of the warp-segment kernel
-        // (profiles/r02_j_fork_rollout.txt); the small and medium shapes win 7.1x and 1.8x
-        env->tpe_rollout = mbe::step_tpe_fork_kernel<30, 13, true, true>;
-        env->tpe_rollout_smem = sizeof(mbe::TpeRolloutSmem<30, 13>);
       } else {
+        // other shapes step episodes launch by launch.  A fused 30 x 13 episode (one env per lane walking
+        // 30 x 13 pairs in scalar code at 208 registers) took 1.43 ms per 20-step episode of 65,536 envs
+        // against 0.83 ms for 20 launches of the warp-segment kernel (profiles/r02_j_fork_rollout.txt);
+        // the small and medium shapes win 7.1x and 1.8x
         env->tpe_shared = false;
       }
     }
@@ -477,16 +451,12 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
                        : (const void*)mbe::step_kernel<0, 0>;
   cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->smem);
   if (e == cudaSuccess && env->big) {
-    // UEs per thread held in registers: 2 (64 registers, 4 CTAs per SM) up to 512 UEs, else 4
-// 1 = always the 4-UEs-per-thread instance (80 registers, 3 CTAs per SM).  With the observation rows
-// leaving as aligned bulk tiles the 2-UEs-per-thread instance for U <= 512 (64 registers, 4 CTAs per SM,
-// smaller shared-memory arrays) is the faster one: 802 vs 920 us per 16,384-env synthetic step
-// (profiles/r02_zb_variants.txt); while the rows were direct 4-byte stores it was the slower one
-// (1105 vs 1046 us, r02_q): more resident CTAs only meant more contention on misaligned sectors
-#ifndef MBE_BIG_FORCE_MAXI4
-#define MBE_BIG_FORCE_MAXI4 0
-#endif
-    const bool two = a.U <= 2 * mbe::kBigThreads && !MBE_BIG_FORCE_MAXI4;
+    // UEs per thread held in registers: 2 (64 registers, 4 CTAs per SM) up to 512 UEs, else 4 (80 registers,
+    // 3 CTAs per SM).  With the observation rows leaving as aligned bulk tiles the 2-UEs-per-thread instance
+    // is the faster one where both fit: 802 vs 920 us per 16,384-env synthetic step
+    // (profiles/r02_zb_variants.txt); while the rows were direct 4-byte stores it was the slower one
+    // (1105 vs 1046 us, r02_q): more resident CTAs only meant more contention on misaligned sectors
+    const bool two = a.U <= 2 * mbe::kBigThreads;
     env->big_fn = gym ? (ma ? (two ? mbe::step_big_kernel<1, 1, 2> : mbe::step_big_kernel<1, 1, 4>)
                             : (two ? mbe::step_big_kernel<1, 0, 2> : mbe::step_big_kernel<1, 0, 4>))
                       : (two ? mbe::step_big_kernel<0, 0, 2> : mbe::step_big_kernel<0, 0, 4>);
@@ -503,22 +473,6 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
   if (e == cudaSuccess && env->tpe_rollout)
     e = cudaFuncSetAttribute((const void*)env->tpe_rollout, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)env->tpe_rollout_smem);
-  if (e == cudaSuccess && env->pipe) {
-    // measured slower than the one-chunk-per-CTA kernel on B200 (profiles/README.md): opt-in only
-    const char* v = std::getenv("MBE_PIPE");
-    if (!(v && v[0] == '1')) env->pipe = nullptr;
-  }
-  if (e == cudaSuccess && env->pipe) {
-    e = cudaFuncSetAttribute((const void*)env->pipe, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)env->pipe_smem);
-    int per_sm = 0, sms = 0;
-    if (e == cudaSuccess)
-      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)env->pipe, mbe::kThreads,
-                                                        env->pipe_smem);
-    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cfg->device);
-    // persistent grid: one full wave of resident CTAs, never more CTAs than chunks
-    env->pipe_grid = std::max(1, std::min(a.E / a.epb, per_sm * sms));
-  }
   if (e == cudaSuccess) {
     // L2 prefetch distance: 0.75 waves of resident CTAs (measured best of 0.25 .. 2 waves on B200,
     // profiles/README.md); MBE_PREFETCH=0 turns it off, MBE_PREFETCH=n sets the distance in CTAs
@@ -550,10 +504,6 @@ void mbe_destroy(mbe_env* env) {
   if (env->host_stream) cudaStreamDestroy(env->host_stream);
   if (env->host_fork) cudaEventDestroy(env->host_fork);
   if (env->host_join) cudaEventDestroy(env->host_join);
-  env->wire_pool.reset();
-  for (cudaEvent_t e : env->wire_events) cudaEventDestroy(e);
-  if (env->wire_dev) cudaFree(env->wire_dev);
-  if (env->wire_pinned) cudaFreeHost(env->wire_pinned);
   delete env;
 }
 
@@ -714,18 +664,17 @@ static int launch(mbe_env* env, int op, int phases, const uint8_t* mask, void* s
   {
     const bool pdl = gym ? pdl_enabled_gym() : pdl_enabled();
     cudaLaunchConfig_t lc = {};
-    const bool use_pipe = env->pipe != nullptr && !window;
     a.pf_dist = env->pf_bound_ok ? env->spec_pf : 0;
-    lc.gridDim = dim3(use_pipe ? env->pipe_grid : grid);
+    lc.gridDim = dim3(grid);
     lc.blockDim = dim3(mbe::kThreads);
-    lc.dynamicSmemBytes = use_pipe ? env->pipe_smem : env->spec_smem;
+    lc.dynamicSmemBytes = env->spec_smem;
     lc.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     lc.attrs = attr;
     lc.numAttrs = pdl ? 1 : 0;
-    MBE_CUDA(cudaLaunchKernelEx(&lc, use_pipe ? env->pipe : env->spec, a));
+    MBE_CUDA(cudaLaunchKernelEx(&lc, env->spec, a));
   }
   else if (!gym)
     mbe::step_kernel<0, 0><<<grid, mbe::kThreads, env->smem, st>>>(a);
@@ -899,7 +848,7 @@ const char* mbe_step_kernel_name(const mbe_env* env) {  // mirrors the dispatch 
   if (env->big) return "step_big_kernel";
   if (env->tpe && (!env->bound || env->tpe_bound_ok) && !env->args.dbg_snr) return "step_tpe_fork_kernel";
   if (env->upt && !env->args.dbg_snr) return "step_upt_kernel";
-  if (env->spec && !env->args.dbg_snr) return env->pipe ? "step_pipe_kernel" : "step_spec_kernel";
+  if (env->spec && !env->args.dbg_snr) return "step_spec_kernel";
   return "step_kernel";
 }
 
@@ -916,68 +865,19 @@ int mbe_step_host(mbe_env* env, const int32_t* actions_host, float* obs_host, fl
   // Env windows on two streams: the action upload and the step of window c+1 overlap the result
   // download of window c (PCIe is full duplex).  With observations the call is bound by their
   // download: plain FP32 rows by DMA straight into obs_host (48 GB/s on the B200 box, no host thread
-  // touches them).  MBE_HOST_WIRE=compact ships them in the compact wire format instead
-  // (mbe_host_wire.cuh, a third fewer bytes) and host threads expand window c into obs_host while
-  // window c+1 is still arriving: that pays only on a host whose cores can write the FP32 rows faster
-  // than PCIe delivers them -- on the 16-vCPU B200 box it measured 0.52-0.70x the DMA path
-  // (profiles/README.md), hence opt-in.  MBE_HOST_WINDOWS / MBE_HOST_THREADS override the defaults.
-  const char* wire_v = std::getenv("MBE_HOST_WIRE");
-  const bool compact = obs_host != nullptr && wire_v && std::strcmp(wire_v, "compact") == 0;
+  // touches them).  A compact wire format (a third fewer bytes, expanded into obs_host by host threads)
+  // measured 0.52-0.70x this DMA path on the 16-vCPU B200 box (profiles/README.md): the host must still
+  // write the FP32 rows.  MBE_HOST_WINDOWS overrides the number of windows.
   const char* wv = std::getenv("MBE_HOST_WINDOWS");
-  const int want = wv ? std::max(1, std::atoi(wv)) : (obs_host ? (compact ? 8 : 4) : 1);
+  const int want = wv ? std::max(1, std::atoi(wv)) : (obs_host ? 4 : 1);
   constexpr int kAlign = 384;  // multiple of every kernel's envs-per-CTA and of 32 (16-byte aligned slices)
   int windows = std::min(want, std::max(1, a.E / (env->big ? kAlign : 8 * kAlign)));
   const int per = ((a.E + windows - 1) / windows + kAlign - 1) / kAlign * kAlign;
   windows = (a.E + per - 1) / per;
-  if (compact && !env->wire_dev) {
-    mbe::WireShape& w = env->wire_shape;
-    w.U = a.U, w.B = a.B, w.F = a.F, w.MW = (a.B + 31) >> 5, w.ma = ma ? 1 : 0;
-    w.W = w.MW * (ma ? 2 : 1);
-    const size_t bytes = (size_t)a.E * w.bytes_per_env();
-    MBE_CUDA(cudaMalloc(&env->wire_dev, bytes));
-    MBE_CUDA(cudaMemset(env->wire_dev, 0, bytes));
-    MBE_CUDA(cudaHostAlloc(&env->wire_pinned, bytes, cudaHostAllocDefault));
-    const char* tv = std::getenv("MBE_HOST_THREADS");
-    cpu_set_t set;
-    int cpus = (sched_getaffinity(0, sizeof set, &set) == 0) ? CPU_COUNT(&set) : (int)std::thread::hardware_concurrency();
-    // spinning workers: keep clear of oversubscription (driver threads, other ranks); 8 threads expand a
-    // 65,536-env medium batch in 0.3 ms on the B200 box's host (profiles/host_expand_bench.cu)
-    const int threads = tv ? std::max(1, std::atoi(tv)) : std::max(1, std::min(cpus / 2, 8));
-    env->wire_pool.reset(new mbe::ExpandCrew(threads - 1));  // the calling thread is the last worker
-  }
-  if (compact)
-    while ((int)env->wire_events.size() < windows) {
-      cudaEvent_t e;
-      MBE_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      env->wire_events.push_back(e);
-    }
   if (windows > 1 && !env->host_stream) {
     MBE_CUDA(cudaStreamCreateWithFlags(&env->host_stream, cudaStreamNonBlocking));
     MBE_CUDA(cudaEventCreateWithFlags(&env->host_fork, cudaEventDisableTiming));
     MBE_CUDA(cudaEventCreateWithFlags(&env->host_join, cudaEventDisableTiming));
-  }
-  // the expansion crew is woken first: its wake-up overlaps the launches below.  Any early return
-  // (a failing CUDA call) releases it through the guard.
-  struct CrewGuard {
-    mbe::ExpandCrew* crew;
-    ~CrewGuard() {
-      if (crew) crew->abort();
-    }
-  } crew_guard{nullptr};
-  if (compact) {
-    mbe::ExpandCrew* crew = env->wire_pool.get();
-    if (windows > mbe::ExpandCrew::kMaxWindows) return fail("mbe_step_host: at most %d env windows", mbe::ExpandCrew::kMaxWindows);
-    const mbe::WireShape ws = env->wire_shape;
-    const int chunks = std::max(1, 4 * (crew->size() + 1));
-    const unsigned char* pinned = env->wire_pinned;
-    const int E = a.E, UF = a.U * a.F;
-    crew->begin(windows, chunks, [=](int w, int c) {
-      const int first = w * per, count = std::min(per, E - first);
-      const int lo = (int)((long long)count * c / chunks), hi = (int)((long long)count * (c + 1) / chunks);
-      if (hi > lo)
-        mbe::wire_expand_any(pinned + (size_t)first * ws.bytes_per_env(), obs_host + (size_t)first * UF, count, lo, hi, ws);
-    });
-    crew_guard.crew = crew;
   }
   if (windows > 1) {  // the side stream starts after everything already queued on the caller's stream
     MBE_CUDA(cudaEventRecord(env->host_fork, st));
@@ -994,17 +894,8 @@ int mbe_step_host(mbe_env* env, const int32_t* actions_host, float* obs_host, fl
     if (int rc = (windows > 1 ? launch(env, mbe::OP_STEP, MBE_PHASE_ALL, nullptr, s, (size_t)first, count)
                               : launch(env, mbe::OP_STEP, MBE_PHASE_ALL, nullptr, s)))
       return rc;
-    if (compact) {
-      const mbe::WireShape& ws = env->wire_shape;
-      const size_t off = (size_t)first * ws.bytes_per_env(), len = (size_t)count * ws.bytes_per_env();
-      const int rows = count * a.U;
-      mbe::wire_pack_kernel<<<(rows + 255) / 256, 256, 0, s>>>(env->bufs.obs, env->wire_dev + off, first, count, ws);
-      MBE_CUDA(cudaGetLastError());
-      MBE_CUDA(cudaMemcpyAsync(env->wire_pinned + off, env->wire_dev + off, len, cudaMemcpyDeviceToHost, s));
-      MBE_CUDA(cudaEventRecord(env->wire_events[w], s));  // the window's observation bytes have landed
-    } else if (obs_host) {
+    if (obs_host)
       MBE_CUDA(cudaMemcpyAsync(obs_host + fu * a.F, env->bufs.obs + fu * a.F, cu * a.F * 4, cudaMemcpyDeviceToHost, s));
-    }
     if (reward_host) {
       const size_t f = ma ? fu : (size_t)first, c = ma ? cu : (size_t)count;
       MBE_CUDA(cudaMemcpyAsync(reward_host + f, env->bufs.reward + f, c * 4, cudaMemcpyDeviceToHost, s));
@@ -1015,16 +906,6 @@ int mbe_step_host(mbe_env* env, const int32_t* actions_host, float* obs_host, fl
   if (windows > 1) {
     MBE_CUDA(cudaEventRecord(env->host_join, env->host_stream));
     MBE_CUDA(cudaStreamWaitEvent(st, env->host_join, 0));
-  }
-  if (compact) {
-    // publish window after window as it lands; the crew expands window c while window c+1 is in flight
-    mbe::ExpandCrew* crew = env->wire_pool.get();
-    for (int w = 0; w < windows; ++w) {
-      MBE_CUDA(cudaEventSynchronize(env->wire_events[w]));
-      crew->publish(w + 1);
-    }
-    crew->finish();
-    crew_guard.crew = nullptr;
   }
   MBE_CUDA(cudaStreamSynchronize(st));
   return 0;

@@ -18,10 +18,6 @@
 #include <type_traits>
 #include "mbe_device.cuh"
 
-// 1 = the central handler tests connectivity only for the connected BSs and the action's BS (experiment switch)
-#ifndef MBE_BIG_SPARSE_PRE
-#define MBE_BIG_SPARSE_PRE 1
-#endif
 #ifndef MBE_BIG_MIN_BLOCKS
 #define MBE_BIG_MIN_BLOCKS 3
 #endif
@@ -290,7 +286,7 @@ __global__ void __launch_bounds__(kBigThreads, MAXI <= 2 ? MBE_BIG_MIN_BLOCKS + 
       float bestf = 3.0e38f;
       int act = 0;
       if (GYM) act = a.actions[idx];
-      if (MBE_BIG_SPARSE_PRE && GYM && !MA && !a.dbg_snr) {
+      if (GYM && !MA && !a.dbg_snr) {
         // The central handler only ever asks "is BS b connectable" for the BSs the UE is connected to
         // (update_connections, base.py:221-227) and for the BS its action names: test those few pairs
         // instead of all B (the multi-agent reward and the FORK association need every pair).  Only

@@ -46,20 +46,11 @@ struct ChunkMem {
   uint32_t* bs;    // [EPB*B] per-env BS table (PER_ENV)
   float* bsu;      // [EPB*B] multi-agent BS utilities
   int* bsn;        // [EPB*B] multi-agent BS connection counts
-  // state staged in shared memory by bulk async copies (PIPE), else unused
-  const uint32_t* st_pos;
-  const uint32_t* st_wp;
-  const uint32_t* st_conn;
-  const int32_t* st_act;
-  const int32_t* st_t;
-  const int32_t* st_epi;
-  const int32_t* st_nbs;
 };
 
-// One fused step of the EPB envs starting at env_base.  PIPE: the state comes from shared memory
-// (ChunkMem::st_*), otherwise straight from global memory.  The observation block is left in
-// m.obs; the caller stores it.
-template <int MODE, int HANDLER, int U, int B, bool PER_ENV, bool PIPE, bool MC = false>
+// One fused step of the EPB envs starting at env_base, state straight from global memory.  The
+// observation block is left in m.obs; the caller stores it.
+template <int MODE, int HANDLER, int U, int B, bool PER_ENV, bool MC = false>
 __device__ __forceinline__ void step_chunk(const StepArgs& a, const int env_base, const ChunkMem& m) {
   constexpr bool GYM = (MODE == 1);
   constexpr bool MA = (HANDLER == 1);
@@ -95,20 +86,18 @@ __device__ __forceinline__ void step_chunk(const StepArgs& a, const int env_base
   auto SL = [&](int b) -> const SlotDev& { return a.slot[MC ? b : 0]; };
 
   // ---- load state (all loads issued before any use) ----
-  const unsigned lidx = valid ? (unsigned)(env_in_blk * U + u) : 0u;  // index inside the chunk
-  const int lenv = valid ? env_in_blk : 0;
-  const uint32_t pos_in = PIPE ? m.st_pos[lidx] : a.pos[idx];
-  const uint32_t wp_in = PIPE ? m.st_wp[lidx] : a.wp[idx];
+  const uint32_t pos_in = a.pos[idx];
+  const uint32_t wp_in = a.wp[idx];
   uint32_t conn = 0;
   int act = 0;
   if (GYM) {
-    conn = PIPE ? m.st_conn[lidx] : a.conn[idx];
-    act = PIPE ? m.st_act[lidx] : a.actions[idx];
+    conn = a.conn[idx];
+    act = a.actions[idx];
   }
-  int t_e = PIPE ? m.st_t[lenv] : a.t[env_ld];
-  int epi = PIPE ? m.st_epi[lenv] : a.episode[env_ld];
+  int t_e = a.t[env_ld];
+  int epi = a.episode[env_ld];
   int nb = B;
-  if (PER_ENV && a.nbs) nb = PIPE ? m.st_nbs[lenv] : a.nbs[env_ld];
+  if (PER_ENV && a.nbs) nb = a.nbs[env_ld];
   int x, y, wx, wy;
   unpack_xy(pos_in, x, y);
   unpack_xy(wp_in, wx, wy);
@@ -347,7 +336,7 @@ __device__ __forceinline__ void step_chunk(const StepArgs& a, const int env_base
   }
 }
 
-// ---- one chunk per CTA (works for any E; also the fallback of the pipelined kernel) ----
+// ---- one chunk per CTA (works for any E) ----
 template <int MODE, int HANDLER, int U, int B, bool PER_ENV, bool MC = false>
 __global__ void __launch_bounds__(kThreads, MBE_SPEC_MIN_BLOCKS(MODE, HANDLER, B)) step_spec_kernel(const __grid_constant__ StepArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -375,7 +364,7 @@ __global__ void __launch_bounds__(kThreads, MBE_SPEC_MIN_BLOCKS(MODE, HANDLER, B
     for (int i = threadIdx.x; i < n; i += kThreads) m.bs[i] = g[i];
     __syncthreads();
   }
-  step_chunk<MODE, HANDLER, U, B, PER_ENV, false, MC>(a, env_base, m);
+  step_chunk<MODE, HANDLER, U, B, PER_ENV, MC>(a, env_base, m);
   if (GYM) store_obs_block(a, m.obs, env_base, threadIdx.x, true);
 }
 
@@ -384,154 +373,6 @@ template <int MODE, int HANDLER, int U, int B, bool PER_ENV>
 constexpr auto spec_mc_kernel() -> void (*)(StepArgs) {
   if constexpr (PER_ENV) return nullptr;
   else return step_spec_kernel<MODE, HANDLER, U, B, false, true>;
-}
-
-// ---- persistent, software-pipelined variant (E must be a multiple of EPB) ----
-// Every CTA walks the env chunks with a grid stride.  While chunk k is computed, the state slices
-// of chunk k+1 ([EPB,U] words of pos / wp / conn / actions, [EPB] clocks, per-env BS tables) are
-// already in flight into the other shared-memory stage as bulk async copies (TMA) that signal an
-// mbarrier, and the observation block of chunk k-1 is still draining from its own buffer as a bulk
-// async store.  Global-memory latency is thus off the critical path of every chunk but the first.
-template <int HANDLER, int U, int B, bool PER_ENV>
-__host__ __device__ constexpr size_t pipe_stage_bytes(bool gym) {
-  constexpr int EPB = (32 / U) * kWarpsPerBlock;
-  size_t n = (size_t)EPB * U * 4 * (gym ? 4 : 2);  // pos, wp (, conn, actions)
-  n += (size_t)EPB * 4 * 3;                        // t, episode, nbs
-  if (PER_ENV) n += (size_t)EPB * B * 4;
-  return (n + 15) & ~(size_t)15;
-}
-template <int HANDLER, int U, int B, bool PER_ENV>
-__host__ __device__ constexpr size_t pipe_smem_bytes(bool gym) {
-  constexpr int EPB = (32 / U) * kWarpsPerBlock;
-  constexpr int F = (HANDLER == 1 ? 4 : 2) * B + 1;
-  size_t obs = gym ? (((size_t)EPB * U * F * 4 + 15) & ~(size_t)15) : 0;
-  size_t ma = (gym && HANDLER == 1) ? (size_t)EPB * B * 8 : 0;
-  return 2 * obs + ((ma + 15) & ~(size_t)15) + 2 * pipe_stage_bytes<HANDLER, U, B, PER_ENV>(gym) + 16;
-}
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bar)),
-               "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = (uint32_t)__cvta_generic_to_shared(bar);
-  uint32_t ok = 0;
-  while (!ok) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.b32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(addr), "r"(parity)
-        : "memory");
-  }
-}
-__device__ __forceinline__ void bulk_load(void* sdst, const void* gsrc, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   (uint32_t)__cvta_generic_to_shared(sdst)),
-               "l"(gsrc), "r"(bytes), "r"((uint32_t)__cvta_generic_to_shared(bar))
-               : "memory");
-}
-
-template <int MODE, int HANDLER, int U, int B, bool PER_ENV>
-__global__ void __launch_bounds__(kThreads, MBE_SPEC_MIN_BLOCKS(MODE, HANDLER, B)) step_pipe_kernel(const __grid_constant__ StepArgs a) {
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  constexpr bool GYM = (MODE == 1);
-  constexpr bool MA = (HANDLER == 1);
-  constexpr int EPB = (32 / U) * kWarpsPerBlock;
-  constexpr int F = GYM ? ((MA ? 4 : 2) * B + 1) : 0;
-  constexpr size_t OBS_BYTES = GYM ? (((size_t)EPB * U * F * 4 + 15) & ~(size_t)15) : 0;
-  constexpr size_t MA_BYTES = (((GYM && MA) ? (size_t)EPB * B * 8 : 0) + 15) & ~(size_t)15;
-  constexpr size_t STAGE_BYTES = pipe_stage_bytes<HANDLER, U, B, PER_ENV>(GYM);
-  constexpr uint32_t EU = EPB * U * 4;  // bytes of one [EPB,U] word slice
-  constexpr uint32_t EE = EPB * 4;      // bytes of one [EPB] word slice
-  const int tid = threadIdx.x;
-
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-
-  unsigned char* obs_buf[2] = {smem_raw, smem_raw + OBS_BYTES};
-  unsigned char* ma_buf = smem_raw + 2 * OBS_BYTES;
-  unsigned char* stage[2] = {ma_buf + MA_BYTES, ma_buf + MA_BYTES + STAGE_BYTES};
-  uint64_t* bar = reinterpret_cast<uint64_t*>(ma_buf + MA_BYTES + 2 * STAGE_BYTES);
-
-  auto issue_loads = [&](int chunk, int sidx) {  // thread 0 only
-    unsigned char* st = stage[sidx];
-    const size_t e0 = (size_t)chunk * EPB;
-    const uint32_t total = EU * (GYM ? 4 : 2) + EE * 2 + (PER_ENV ? EE + EPB * B * 4 : 0);
-    mbar_expect_tx(&bar[sidx], total);
-    bulk_load(st, a.pos + e0 * U, EU, &bar[sidx]);
-    bulk_load(st + EU, a.wp + e0 * U, EU, &bar[sidx]);
-    size_t off = 2 * (size_t)EU;
-    if (GYM) {
-      bulk_load(st + off, a.conn + e0 * U, EU, &bar[sidx]);
-      bulk_load(st + off + EU, a.actions + e0 * U, EU, &bar[sidx]);
-      off += 2 * (size_t)EU;
-    }
-    bulk_load(st + off, a.t + e0, EE, &bar[sidx]);
-    bulk_load(st + off + EE, a.episode + e0, EE, &bar[sidx]);
-    if (PER_ENV) {
-      bulk_load(st + off + 2 * EE, a.nbs + e0, EE, &bar[sidx]);
-      bulk_load(st + off + 3 * EE, a.bs_xy + e0 * B, EPB * B * 4, &bar[sidx]);
-    }
-  };
-
-  const int nchunks = a.E / EPB;
-  if (tid == 0) {
-    mbar_init(&bar[0], 1);
-    mbar_init(&bar[1], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    if ((int)blockIdx.x < nchunks) issue_loads(blockIdx.x, 0);
-  }
-  __syncthreads();
-
-  int it = 0;
-  for (int chunk = blockIdx.x; chunk < nchunks; chunk += gridDim.x, ++it) {
-    const int sidx = it & 1;
-    // the other stage was consumed in the previous iteration (its readers passed that iteration's
-    // barrier), so it can be refilled now for the next chunk
-    if (tid == 0 && chunk + (int)gridDim.x < nchunks) issue_loads(chunk + gridDim.x, sidx ^ 1);
-    mbar_wait(&bar[sidx], (uint32_t)((it >> 1) & 1));
-
-    unsigned char* st = stage[sidx];
-    ChunkMem m = {};
-    m.obs = reinterpret_cast<float*>(obs_buf[sidx]);
-    m.bsu = reinterpret_cast<float*>(ma_buf);
-    m.bsn = reinterpret_cast<int*>(ma_buf + (size_t)EPB * B * 4);
-    m.st_pos = reinterpret_cast<const uint32_t*>(st);
-    m.st_wp = reinterpret_cast<const uint32_t*>(st + EU);
-    size_t off = 2 * (size_t)EU;
-    if (GYM) {
-      m.st_conn = reinterpret_cast<const uint32_t*>(st + off);
-      m.st_act = reinterpret_cast<const int32_t*>(st + off + EU);
-      off += 2 * (size_t)EU;
-    }
-    m.st_t = reinterpret_cast<const int32_t*>(st + off);
-    m.st_epi = reinterpret_cast<const int32_t*>(st + off + EE);
-    if (PER_ENV) {
-      m.st_nbs = reinterpret_cast<const int32_t*>(st + off + 2 * EE);
-      m.bs = reinterpret_cast<uint32_t*>(st + off + 3 * EE);
-    }
-    step_chunk<MODE, HANDLER, U, B, PER_ENV, true>(a, chunk * EPB, m);
-
-    // the bulk store that last read this observation buffer was issued two iterations ago and
-    // waited for one iteration ago (below), so the rows written above raced with nothing
-    if (GYM) {
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      if (tid == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // previous chunk's store
-    }
-    __syncthreads();  // rows complete; stage sidx fully consumed
-    if (GYM && tid == 0) {
-      float* gdst = a.obs + (size_t)chunk * EPB * U * F;
-      asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst),
-                   "r"((uint32_t)__cvta_generic_to_shared(m.obs)), "r"((uint32_t)(EPB * U * F * 4))
-                   : "memory");
-      asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-    }
-  }
-  if (GYM && tid == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
 
 }  // namespace mbe

@@ -21,7 +21,6 @@
 // bases 16-byte aligned, nbs bound.
 #pragma once
 #include "mbe_device.cuh"
-#include "mbe_step_spec.cuh"  // mbar_* / bulk_load helpers
 #include <type_traits>
 
 namespace mbe {
@@ -78,6 +77,31 @@ __device__ __forceinline__ float tree_sum(float (&v)[U]) {
   return v[0];
 }
 
+__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
+  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bar)), "r"(count));
+}
+__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
+  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bar)),
+               "r"(bytes)
+               : "memory");
+}
+__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
+  const uint32_t addr = (uint32_t)__cvta_generic_to_shared(bar);
+  uint32_t ok = 0;
+  while (!ok) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.b32 %0, 1, 0, p;\n\t}"
+        : "=r"(ok)
+        : "r"(addr), "r"(parity)
+        : "memory");
+  }
+}
+__device__ __forceinline__ void bulk_load(void* sdst, const void* gsrc, uint32_t bytes, uint64_t* bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                   (uint32_t)__cvta_generic_to_shared(sdst)),
+               "l"(gsrc), "r"(bytes), "r"((uint32_t)__cvta_generic_to_shared(bar))
+               : "memory");
+}
 __device__ __forceinline__ void bulk_store(void* gdst, const void* ssrc, uint32_t bytes) {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst),
                "r"((uint32_t)__cvta_generic_to_shared(ssrc)), "r"(bytes)
@@ -92,40 +116,18 @@ __device__ __forceinline__ void bulk_store(void* gdst, const void* ssrc, uint32_
 #define MBE_TPE_ROLLOUT_BLOCKS 16
 #endif
 
-// |connections(b)| of one env, packed into 64-bit words: 4 bits per BS while a count cannot exceed 15,
-// else 8 bits (two words for more than 8 BSs)
+// |connections(b)| of one env, 4 bits per BS in one 64-bit word
 template <int U, int B>
 struct TpeCounts {
-  static constexpr int kBits = U <= 15 ? 4 : 8;
-  static constexpr int kPer = 64 / kBits;
-  static constexpr int kWords = (B + kPer - 1) / kPer;
-  unsigned long long w[kWords];
-  __device__ __forceinline__ void clear() {
-#pragma unroll
-    for (int i = 0; i < kWords; ++i) w[i] = 0ull;
-  }
-  __device__ __forceinline__ void add(int b) {
-    if (kWords == 1) {
-      w[0] += 1ull << (kBits * b);
-    } else {
-#pragma unroll
-      for (int i = 0; i < kWords; ++i)
-        if (b / kPer == i) w[i] += 1ull << (kBits * (b % kPer));
-    }
-  }
-  __device__ __forceinline__ unsigned get(int b) const {
-    unsigned long long v = w[0];
-    if (kWords > 1) {
-#pragma unroll
-      for (int i = 1; i < kWords; ++i)
-        if (b / kPer == i) v = w[i];
-    }
-    return (unsigned)(v >> (kBits * (b % kPer))) & ((1u << kBits) - 1u);
-  }
+  static_assert(U <= 15 && B <= 16, "a count must fit 4 bits and all BSs one word");
+  unsigned long long w;
+  __device__ __forceinline__ void clear() { w = 0ull; }
+  __device__ __forceinline__ void add(int b) { w += 1ull << (4 * b); }
+  __device__ __forceinline__ unsigned get(int b) const { return (unsigned)(w >> (4 * b)) & 15u; }
 };
 
 template <int U, int B, bool ROLLOUT = false, bool SHARED = false>
-__global__ void __launch_bounds__(32, ROLLOUT ? (U > 16 ? 8 : MBE_TPE_ROLLOUT_BLOCKS) : MBE_TPE_BLOCKS) step_tpe_fork_kernel(const __grid_constant__ StepArgs a) {
+__global__ void __launch_bounds__(32, ROLLOUT ? MBE_TPE_ROLLOUT_BLOCKS : MBE_TPE_BLOCKS) step_tpe_fork_kernel(const __grid_constant__ StepArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   using S = typename std::conditional<ROLLOUT, TpeRolloutSmem<U, B>, TpeForkSmem<U, B>>::type;
   static_assert(B <= 16, "the nearest-BS key keeps the BS index in 4 bits");

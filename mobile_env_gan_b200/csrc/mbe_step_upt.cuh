@@ -28,57 +28,7 @@
 #define MBE_UPT_WARPS 2
 #endif
 
-// experiment switches (profiles/variant_sweep.py): cache hints for the streamed state / the rate table
-#ifndef MBE_UPT_STREAM_HINTS
-#define MBE_UPT_STREAM_HINTS 0
-#endif
-// how the observation block leaves shared memory: 0 = one bulk async copy per CTA (thread 0 issues
-// and waits for the read), 1 = cooperative 16-byte copies by the whole CTA after a barrier,
-// 2 = every warp copies its own envs (8-byte units, no CTA barrier)
-#ifndef MBE_UPT_STORE
-#define MBE_UPT_STORE 0
-#endif
-// 1 = the rate-table gathers are issued, then the movement phase runs (it needs nothing from them),
-// then the gathered values are summed, so that the L2 latency of the gathers hides behind independent
-// work.  Measured and rejected (profiles/r02_h_variants.txt): the 24 registers of gathered doubles
-// held across the movement code spill at the 72-register budget (18.2 vs 16.3 us per medium-central
-// step) and a 6-CTA budget loses as much in occupancy (18.6 us).
-#ifndef MBE_UPT_EARLY_MOVE
-#define MBE_UPT_EARLY_MOVE 0
-#endif
-#ifndef MBE_UPT_LUT_HINT
-#define MBE_UPT_LUT_HINT 2  // read-only path for the rate table: measured -2.3% (multi-agent), neutral (central)
-#endif
-
 namespace mbe {
-
-template <typename T>
-__device__ __forceinline__ T upt_ld(const T* p) {
-#if MBE_UPT_STREAM_HINTS
-  return __ldcs(p);  // read once: do not keep the line
-#else
-  return *p;
-#endif
-}
-template <typename T>
-__device__ __forceinline__ void upt_st(T* p, T v) {
-#if MBE_UPT_STREAM_HINTS
-  __stcs(p, v);
-#else
-  *p = v;
-#endif
-}
-__device__ __forceinline__ double upt_lut(const double* p) {
-#if MBE_UPT_LUT_HINT == 1
-  double v;
-  asm("ld.global.nc.L1::evict_last.f64 %0, [%1];" : "=d"(v) : "l"(p));
-  return v;
-#elif MBE_UPT_LUT_HINT == 2
-  return __ldg(p);
-#else
-  return *p;
-#endif
-}
 
 template <int HANDLER, int U, int B, int K>
 __host__ __device__ constexpr size_t upt_smem_bytes() {
@@ -127,10 +77,10 @@ __global__ void __launch_bounds__(32 * MBE_UPT_WARPS, MBE_UPT_MIN_BLOCKS(HANDLER
 #pragma unroll
   for (int j = 0; j < UPT; ++j) {
     idx[j] = (unsigned)env_ld * U + (unsigned)(k + K * j);
-    pos_in[j] = upt_ld(a.pos + idx[j]);
-    wp_in[j] = upt_ld(a.wp + idx[j]);
-    conn[j] = valid ? upt_ld(a.conn + idx[j]) : 0u;
-    act[j] = valid ? upt_ld(a.actions + idx[j]) : 0;
+    pos_in[j] = a.pos[idx[j]];
+    wp_in[j] = a.wp[idx[j]];
+    conn[j] = valid ? a.conn[idx[j]] : 0u;
+    act[j] = valid ? a.actions[idx[j]] : 0;
   }
   int t_e = a.t[env_ld];
   int epi = a.episode[env_ld];
@@ -188,38 +138,18 @@ __global__ void __launch_bounds__(32 * MBE_UPT_WARPS, MBE_UPT_MIN_BLOCKS(HANDLER
   float util[UPT];
   float lu = 0.0f, lr = 0.0f;
   int ln = 0;
-#if MBE_UPT_EARLY_MOVE
-  double gv[UPT][B];
-#pragma unroll
-  for (int j = 0; j < UPT; ++j)
-#pragma unroll
-    for (int b = 0; b < B; ++b) {
-      const unsigned off = (unsigned)cnt[b] * stride + (unsigned)d2pre[j][b];
-      if (MA) gv[j][b] = ((conn[j] >> b) & 1u) ? upt_lut(lut + off) : 0.0;
-      else gv[j][b] = upt_lut(lut + (((conn[j] >> b) & 1u) ? off : stride - 1u));
-    }
-  // ---- move (movement.py:42-62): independent of the rates, runs while the gathers are in flight ----
-#pragma unroll
-  for (int j = 0; j < UPT; ++j) {
-    if (wx[j] < 0) next_waypoint(a, gid, (unsigned)(k + K * j), idx[j], t_e, epi, valid, wx[j], wy[j]);
-    if (move_ue(a.mv[0], x[j], y[j], wx[j], wy[j])) wx[j] = wy[j] = -1;
-  }
-#endif
 #pragma unroll
   for (int j = 0; j < UPT; ++j) {
     double r = 0.0;
 #pragma unroll
     for (int b = 0; b < B; ++b) {
-#if MBE_UPT_EARLY_MOVE
-      r += gv[j][b];  // (+0.0 for an unconnected BS: the sum's bits do not change)
-#else
+      // the rate table through the read-only path: measured -2.3% (multi-agent), neutral (central)
       if (MA) {  // measured: predicated gathers win with the multi-agent register budget ...
-        if ((conn[j] >> b) & 1u) r += upt_lut(lut + ((unsigned)cnt[b] * stride + (unsigned)d2pre[j][b]));
+        if ((conn[j] >> b) & 1u) r += __ldg(lut + ((unsigned)cnt[b] * stride + (unsigned)d2pre[j][b]));
       } else {   // ... unconditional ones (unconnected -> the table's 0.0 entry) for the central handler
         const unsigned off = (unsigned)cnt[b] * stride + (unsigned)d2pre[j][b];
-        r += upt_lut(lut + (((conn[j] >> b) & 1u) ? off : stride - 1u));
+        r += __ldg(lut + (((conn[j] >> b) & 1u) ? off : stride - 1u));
       }
-#endif
     }
     rate[j] = r;
     util[j] = scaled_utility(a, r);
@@ -252,8 +182,8 @@ __global__ void __launch_bounds__(32 * MBE_UPT_WARPS, MBE_UPT_MIN_BLOCKS(HANDLER
   if (valid) {
 #pragma unroll
     for (int j = 0; j < UPT; ++j) {
-      if (a.rate) upt_st(a.rate + idx[j], rate[j]);
-      upt_st(a.utility + idx[j], util[j]);
+      if (a.rate) a.rate[idx[j]] = rate[j];
+      a.utility[idx[j]] = util[j];
       if (MA) {
         float nu = 0.0f;
         int ncnt = 0;
@@ -275,14 +205,16 @@ __global__ void __launch_bounds__(32 * MBE_UPT_WARPS, MBE_UPT_MIN_BLOCKS(HANDLER
     }
   }
 
-#if !MBE_UPT_EARLY_MOVE
   // ---- move (movement.py:42-62) ----
+  // (Issuing the rate gathers before the move, to hide their L2 latency behind it, was measured and
+  // rejected, profiles/r02_h_variants.txt: the 24 registers of gathered doubles held across the
+  // movement code spill at the 72-register budget, 18.2 vs 16.3 us per medium-central step, and a
+  // 6-CTA budget loses as much in occupancy, 18.6 us.)
 #pragma unroll
   for (int j = 0; j < UPT; ++j) {
     if (wx[j] < 0) next_waypoint(a, gid, (unsigned)(k + K * j), idx[j], t_e, epi, valid, wx[j], wy[j]);
     if (move_ue(a.mv[0], x[j], y[j], wx[j], wy[j])) wx[j] = wy[j] = -1;
   }
-#endif
 
   // ---- clock, departures, same-step autoreset (base.py:280-291, 407-409; 172-209) ----
   t_e += 1;
@@ -368,35 +300,6 @@ __global__ void __launch_bounds__(32 * MBE_UPT_WARPS, MBE_UPT_MIN_BLOCKS(HANDLER
     }
     if (k == 0) a.t[env] = t_e;
   }
-#if MBE_UPT_STORE == 1
-  if (a.obs_bulk_ok && env_base + EPB <= a.E) {
-    constexpr int N16 = EPB * U * F / 4;
-    static_assert((EPB * U * F) % 4 == 0, "whole CTA blocks are multiples of 16 bytes");
-    __syncthreads();
-    float4* g = reinterpret_cast<float4*>(a.obs + (size_t)env_base * (U * F));
-    const float4* sv = reinterpret_cast<const float4*>(s_obs);
-#pragma unroll
-    for (int i = 0; i < (N16 + 32 * MBE_UPT_WARPS - 1) / (32 * MBE_UPT_WARPS); ++i) {
-      const int e = tid + i * 32 * MBE_UPT_WARPS;
-      if (e < N16) g[e] = sv[e];
-    }
-    return;
-  }
-#elif MBE_UPT_STORE == 2
-  if (a.obs_bulk_ok && env_base + EPB <= a.E) {
-    constexpr int N8 = EPW * U * F / 2;  // 8-byte units of one warp's envs
-    static_assert((EPW * U * F) % 2 == 0, "a warp's rows are a multiple of 8 bytes");
-    __syncwarp();
-    float2* g = reinterpret_cast<float2*>(a.obs + (size_t)(env_base + warp * EPW) * (U * F));
-    const float2* sv = reinterpret_cast<const float2*>(s_obs + warp * EPW * U * F);
-#pragma unroll
-    for (int i = 0; i < (N8 + 31) / 32; ++i) {
-      const int e = lane + i * 32;
-      if (e < N8) g[e] = sv[e];
-    }
-    return;
-  }
-#endif
   store_obs_block<32 * MBE_UPT_WARPS>(a, s_obs, env_base, tid, true);
 }
 

@@ -54,11 +54,11 @@ run(env, 22, False)
 env.rollout(23, qoe_acc=LayoutScorer(env).acc, record=("pos", "wp", "assoc", "rate", "utility"))
 env.step_window(32, 32)
 env.step_window(64, 17)
-os.environ["MBE_TPE_LARGE"] = "1"
 for cls in (MComSmall, MComMedium, MComLarge):
     fork = cls(config={"num_envs": 64, "autoreset": True, "mode": "fork"})
     run(fork, 3, False)
-    fork.rollout(23, qoe_acc=LayoutScorer(fork).acc, record=("pos", "rate"))
+    # 30 x 13 has no fused episode, and a stepped episode with autoreset cannot record positions
+    fork.rollout(23, qoe_acc=LayoutScorer(fork).acc, record=("rate",) if cls is MComLarge else ("pos", "rate"))
 # block-per-env kernel: split phases, observe, window, central handler
 big = mbe.make("mobile-synthetic-central-v0", num_envs=64, autoreset=True, config={"EP_MAX_TIME": 3, "arrival_params": {"ep_time": 3}})
 run(big, 4, True)
@@ -66,19 +66,14 @@ for ph in (2, 1, 4, 8):
     big.stage(ph)
 big.observe()
 big.step_window(32, 32)
-# host-buffer entry point, both wire formats
-for wire in ("raw", "compact"):
-    os.environ["MBE_HOST_WIRE"] = wire
-    os.environ["MBE_HOST_THREADS"] = "3"
-    for wid in ("mobile-medium-central-v0", "mobile-medium-ma-v0"):
-        h = mbe.make(wid, num_envs=6400, autoreset=True)
-        h.reset()
-        acts = torch.zeros(tuple(h.actions.shape), dtype=torch.int32).pin_memory()
-        obs_h = torch.empty(tuple(h.obs.shape), dtype=torch.float32).pin_memory()
-        rew_h = torch.empty(tuple(h.reward.shape), dtype=torch.float32).pin_memory()
-        done_h = torch.empty(6400, dtype=torch.uint8).pin_memory()
-        for _ in range(3):
-            h.step_host(acts, obs_h, rew_h, done_h)
-os.environ["MBE_PIPE"] = "1"
-run(mbe.make("mobile-medium-central-v0", num_envs=64, autoreset=True), 25, True)
+# host-buffer entry point
+for wid in ("mobile-medium-central-v0", "mobile-medium-ma-v0"):
+    h = mbe.make(wid, num_envs=6400, autoreset=True)
+    h.reset()
+    acts = torch.zeros(tuple(h.actions.shape), dtype=torch.int32).pin_memory()
+    obs_h = torch.empty(tuple(h.obs.shape), dtype=torch.float32).pin_memory()
+    rew_h = torch.empty(tuple(h.reward.shape), dtype=torch.float32).pin_memory()
+    done_h = torch.empty(6400, dtype=torch.uint8).pin_memory()
+    for _ in range(3):
+        h.step_host(acts, obs_h, rew_h, done_h)
 print("sanitize smoke done")

@@ -556,17 +556,13 @@ def test_readme_pathloss_example_runs_verbatim_and_matches_the_oracle():
     assert ranged > 0  # the threshold really cut links
 
 
-@pytest.mark.parametrize("wire", ["compact", "raw"])
 @pytest.mark.parametrize("handler", ["central", "ma"])
-def test_step_host_wire_formats_reproduce_the_device_observation(wire, handler, monkeypatch):
-    """mbe_step_host ships observations as plain FP32 rows by DMA (the default) or, with
-    MBE_HOST_WIRE=compact, in the compact wire format (mask bits + snr ratios + utility, per-env BS
-    utilities for the multi-agent handler) expanded by host threads.  Either way obs_host must equal the device tensor bit
-    for bit, including the all-zero rows of finished episodes (no autoreset) and fresh rows after a reset."""
+def test_step_host_reproduces_the_device_observation(handler):
+    """mbe_step_host ships observations as plain FP32 rows by DMA: obs_host must equal the device
+    tensor bit for bit, including the all-zero rows of finished episodes (no autoreset) and fresh rows
+    after a reset."""
     import mobile_env_gan_b200 as mbe
 
-    monkeypatch.setenv("MBE_HOST_WIRE", wire)
-    monkeypatch.setenv("MBE_HOST_THREADS", "5")
     E = 6400
     env = mbe.make(f"mobile-medium-{handler}-v0", num_envs=E, autoreset=False)
     env.reset()
@@ -582,16 +578,14 @@ def test_step_host_wire_formats_reproduce_the_device_observation(wire, handler, 
         acts = torch.randint(0, B + 1, (E, U), dtype=torch.int32, generator=gen).pin_memory()
         obs_h.fill_(7.0)
         env.step_host(acts, obs_h, rew_h, done_h)
-        assert torch.equal(obs_h, env.obs.cpu()), (wire, handler, k)
+        assert torch.equal(obs_h, env.obs.cpu()), (handler, k)
         assert torch.equal(rew_h, env.reward.cpu()) and torch.equal(done_h, env.done.cpu())
     assert bool((env.obs.view(E, -1).abs().sum(dim=1) == 0).any())  # inactive envs were part of the comparison
 
 
-def test_step_host_compact_wire_on_a_wide_shape(monkeypatch):
+def test_step_host_on_a_wide_shape():
     """Two mask words per UE (40 BSs), multi-agent, block-per-env kernel, env windows."""
     from test_gpu_parity import wide_env
-
-    monkeypatch.setenv("MBE_HOST_WIRE", "compact")
 
     env, B, U = wide_env("wide_pf", "gym", "ma", 800, autoreset=True)
     env.reset()
