@@ -5,10 +5,16 @@ whole 20-step epoch is one kernel launch (mbe_rollout) and the score statistics 
 
     python examples/layout_search.py --layouts 1000000 --rounds 5 --top 10
     torchrun --nproc-per-node 8 examples/layout_search.py --layouts 8388608   # layouts sharded over the GPUs
+    python examples/layout_search.py --layouts 1048576 --generations 50       # genetic search (LayoutEvolution)
 
 Multi-GPU: every rank scores its own contiguous slice of the global layout range (Philox layouts are
 keyed by the global env id, so the candidates do not depend on the number of GPUs); the only exchange
 is an all-gather of each rank's top-k (score, layout) rows per round.
+
+--generations N > 0 replaces the random rounds by N generations of LayoutEvolution: each generation scores
+the population, keeps the best layouts and breeds the rest from them on the GPU (mbe_evolve_layouts).
+Under torchrun every rank evolves its own island (Philox counters use global env ids; no migration) and
+the ranks' winners are gathered as above.
 """
 import argparse
 import os
@@ -20,7 +26,7 @@ import torch.distributed as dist
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from mobile_env_gan_b200.scenarios.custom import MComCustom  # noqa: E402
-from mobile_env_gan_b200.scoring import LayoutScorer  # noqa: E402
+from mobile_env_gan_b200.scoring import LayoutEvolution, LayoutScorer  # noqa: E402
 from mobile_env_gan_b200.sharding import sharded_config  # noqa: E402
 
 
@@ -29,6 +35,7 @@ def main():
     ap.add_argument("--layouts", type=int, default=1 << 20, help="candidate layouts per round (envs)")
     ap.add_argument("--rounds", type=int, default=3, help="each round draws fresh layouts (next episode)")
     ap.add_argument("--top", type=int, default=5)
+    ap.add_argument("--generations", type=int, default=0, help="> 0: genetic search instead of random rounds")
     args = ap.parse_args()
     world, rank, local = (int(os.environ.get(k, d)) for k, d in (("WORLD_SIZE", 1), ("RANK", 0), ("LOCAL_RANK", 0)))
     torch.cuda.set_device(local)
@@ -38,6 +45,8 @@ def main():
     # autoreset: the step that ends an epoch draws the next layout, like MComCustom.reset (custom.py:40-77)
     env = MComCustom(config={"autoreset": True, "device": f"cuda:{local}", **sharded_config(total, rank, world)})
     E, B = env.num_envs, env.plan.num_bs
+    if args.generations > 0:
+        return evolve(env, args, world, rank, total)
     scorer = LayoutScorer(env)
     env.reset()
     best = []
@@ -49,11 +58,7 @@ def main():
         scorer.run_episode()  # one launch: 20 steps x E envs + score statistics
         idx, score = scorer.best(min(args.top, E))
         rows = torch.cat([score[:, None], nbs[idx, None].float(), layouts[idx].reshape(len(idx), -1).float()], dim=1)
-        if world > 1:  # the only exchange: every rank's top-k rows
-            out = rows.new_empty((world * rows.shape[0], rows.shape[1]))
-            dist.all_gather_into_tensor(out, rows.contiguous())
-            rows = out
-        cand = [(float(row[0]), row[2:2 + 2 * int(row[1])].reshape(-1, 2).int().tolist()) for row in rows.cpu()]
+        cand = gather_rows(rows, world)
         best = sorted(best + cand, key=lambda c: -c[0])[: args.top]
         if rank == 0:
             top = max(cand, key=lambda c: c[0])
@@ -64,6 +69,40 @@ def main():
         n = args.rounds * total
         print(f"{n} layouts x {env.plan.ep_time} steps on {world} GPU(s) in {dt:.3f} s = "
               f"{n * env.plan.ep_time / dt:.3e} env-steps/s (wall clock, incl. top-k and gather)")
+        for s, xy in best:
+            print(f"{s:+.4f}  {xy}")
+    if world > 1:
+        dist.destroy_process_group()
+
+
+def gather_rows(rows, world):
+    if world > 1:  # the only exchange: every rank's top-k rows
+        out = rows.new_empty((world * rows.shape[0], rows.shape[1]))
+        dist.all_gather_into_tensor(out, rows.contiguous())
+        rows = out
+    return [(float(row[0]), row[2:2 + 2 * int(row[1])].reshape(-1, 2).int().tolist()) for row in rows.cpu()]
+
+
+def evolve(env, args, world, rank, total):
+    evo = LayoutEvolution(env)
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    for g in range(args.generations):
+        fit = evo.step()
+        best = fit.max().reshape(1)
+        if world > 1:
+            dist.all_reduce(best, op=dist.ReduceOp.MAX)
+        if rank == 0:
+            print(f"generation {g}: best score {float(best):+.4f}")
+    torch.cuda.synchronize()
+    dt = time.perf_counter() - t0
+    xy, nbs, score = evo.best(min(args.top, env.num_envs))
+    rows = torch.cat([score[:, None], nbs[:, None].float(), xy.reshape(len(score), -1).float()], dim=1)
+    best = sorted(gather_rows(rows, world), key=lambda c: -c[0])[: args.top]
+    if rank == 0:
+        n = args.generations * total
+        print(f"{n} layouts evaluated in {args.generations} generations on {world} GPU(s) in {dt:.3f} s "
+              f"(wall clock, incl. the per-generation print)")
         for s, xy in best:
             print(f"{s:+.4f}  {xy}")
     if world > 1:

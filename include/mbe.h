@@ -173,8 +173,8 @@ int mbe_abi_version(void);
 const char* mbe_build_info(void);
 const char* mbe_last_error(void);
 /* sizeof of the ABI structs as the library was compiled (0 mbe_config, 1 mbe_buffers, 2 mbe_link_class,
- * 3 mbe_ue_class, 4 mbe_rollout_out, 5 mbe_render_style; -1 otherwise): lets a binding in another
- * language check its layout */
+ * 3 mbe_ue_class, 4 mbe_rollout_out, 5 mbe_render_style, 6 mbe_evolve_params; -1 otherwise): lets a
+ * binding in another language check its layout */
 int mbe_struct_size(int which);
 
 /* replaces MComCore.__init__ (base.py:32-100): validates, copies the constant tables */
@@ -244,6 +244,25 @@ typedef struct mbe_render_style {
  * should not cross an episode boundary.  An env id outside 0..E-1 gives a background-only frame. */
 int mbe_render(mbe_env* env, const int32_t* env_ids, int n, const mbe_rollout_out* series, int steps,
                const mbe_render_style* style, uint8_t* out, void* stream);
+
+/* One generation of a genetic search over per-env BS layouts (DESIGN.md section 10).  Philox key = seed,
+ * counter (env_offset + child, generation, block, 3).  Probabilities are compared as r * 2^-32 < p. */
+typedef struct mbe_evolve_params {
+  uint64_t seed;
+  uint32_t generation;
+  int32_t tournament; /* candidates per tournament, 1..4 */
+  int32_t step;       /* largest per-axis move, 0..32767 */
+  int32_t reserved;
+  double p_cross, p_move, p_add, p_del; /* each in [0, 1] */
+} mbe_evolve_params;
+
+/* Breeds child_xy int16 [E,B,2] / child_nbs int32 [E] from parent_xy / parent_nbs and fitness f32 [E]
+ * (all DEVICE, 4-byte aligned; E, B and the layout ranges are the handle's, which needs random per-env
+ * layouts).  Child c < n_elite copies parent elite_ids[c] verbatim when that id is in 0..E-1.  The
+ * child buffers must not overlap any input.  One launch. */
+int mbe_evolve_layouts(mbe_env* env, const float* fitness, const int16_t* parent_xy, const int32_t* parent_nbs,
+                       const int32_t* elite_ids, int n_elite, const mbe_evolve_params* p, int16_t* child_xy,
+                       int32_t* child_nbs, void* stream);
 
 /* number of kernel launches this handle has enqueued so far */
 int64_t mbe_launch_count(const mbe_env* env);

@@ -116,6 +116,14 @@ class RenderStyle(C.Structure):
                 ("line_width", C.c_int32), ("palette", (C.c_uint8 * 3) * RENDER_PALETTE)]
 
 
+class EvolveParams(C.Structure):
+    """mbe_evolve_params: Philox seed and generation, tournament size, move step, operator probabilities."""
+
+    _fields_ = [("seed", C.c_uint64), ("generation", C.c_uint32), ("tournament", C.c_int32), ("step", C.c_int32),
+                ("reserved", C.c_int32), ("p_cross", C.c_double), ("p_move", C.c_double), ("p_add", C.c_double),
+                ("p_del", C.c_double)]
+
+
 # every symbol include/mbe.h declares: (name, restype, argtypes)
 SYMBOLS = [
     ("mbe_abi_version", C.c_int, []),
@@ -135,6 +143,8 @@ SYMBOLS = [
     ("mbe_rollout", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_float, C.POINTER(RolloutOut), C.c_void_p]),
     ("mbe_render", C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(RolloutOut), C.c_int,
                              C.POINTER(RenderStyle), C.c_void_p, C.c_void_p]),
+    ("mbe_evolve_layouts", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                     C.POINTER(EvolveParams), C.c_void_p, C.c_void_p, C.c_void_p]),
     ("mbe_launch_count", C.c_int64, [C.c_void_p]),
     ("mbe_step_kernel_name", C.c_char_p, [C.c_void_p]),
     ("mbe_step_host", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -164,7 +174,7 @@ def load():
         fn.argtypes = args
     if lib.mbe_abi_version() != MBE_ABI_VERSION:
         raise MbeError(f"libmbe ABI {lib.mbe_abi_version()} != binding {MBE_ABI_VERSION}")
-    for which, struct in enumerate((Config, Buffers, BsClass, UeClass, RolloutOut, RenderStyle)):
+    for which, struct in enumerate((Config, Buffers, BsClass, UeClass, RolloutOut, RenderStyle, EvolveParams)):
         if lib.mbe_struct_size(which) != C.sizeof(struct):
             raise MbeError(f"struct layout mismatch: {struct.__name__} is {C.sizeof(struct)} bytes here, "
                            f"{lib.mbe_struct_size(which)} in {LIB_PATH}")

@@ -18,6 +18,7 @@
 #include "mbe_step_upt.cuh"
 #include "mbe_step_tpe.cuh"
 #include "mbe_render.cuh"
+#include "mbe_evolve.cuh"
 
 namespace {
 
@@ -168,6 +169,7 @@ int mbe_struct_size(int which) {
     case 3: return (int)sizeof(mbe_ue_class);
     case 4: return (int)sizeof(mbe_rollout_out);
     case 5: return (int)sizeof(mbe_render_style);
+    case 6: return (int)sizeof(mbe_evolve_params);
     default: return -1;
   }
 }
@@ -836,6 +838,70 @@ int mbe_render(mbe_env* env, const int32_t* env_ids, int n, const mbe_rollout_ou
   MBE_ON_DEVICE(env->cfg.device);
   MBE_CUDA(cudaFuncSetAttribute((const void*)mbe::render_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   mbe::render_kernel<<<(unsigned)blocks, mbe::kRenderThreads, smem, static_cast<cudaStream_t>(stream)>>>(a, *style);
+  MBE_CUDA(cudaGetLastError());
+  env->launches += 1;
+  return 0;
+}
+
+namespace {
+bool ranges_overlap(const void* a, size_t na, const void* b, size_t nb) {
+  if (!a || !b) return false;
+  const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
+  return x < y + nb && y < x + na;
+}
+}  // namespace
+
+int mbe_evolve_layouts(mbe_env* env, const float* fitness, const int16_t* parent_xy, const int32_t* parent_nbs,
+                       const int32_t* elite_ids, int n_elite, const mbe_evolve_params* p, int16_t* child_xy,
+                       int32_t* child_nbs, void* stream) {
+  if (!env) return fail("null handle");
+  if (!fitness || !parent_xy || !parent_nbs || !p || !child_xy || !child_nbs)
+    return fail("mbe_evolve_layouts: null argument");
+  const mbe_config& cfg = env->cfg;
+  if (cfg.bs_layout != MBE_BS_PER_ENV || cfg.bs_random_max <= 0)
+    return fail("mbe_evolve_layouts: needs random per-env BS layouts (bs_layout=PER_ENV, bs_random_max > 0)");
+  const int E = cfg.num_envs, B = cfg.num_bs;
+  if (n_elite < 0 || n_elite > E) return fail("mbe_evolve_layouts: n_elite=%d outside 0..%d", n_elite, E);
+  if (n_elite > 0 && !elite_ids) return fail("mbe_evolve_layouts: n_elite > 0 needs elite_ids");
+  if (p->tournament < 1 || p->tournament > 4)
+    return fail("mbe_evolve_layouts: tournament=%d outside 1..4", p->tournament);
+  if (p->step < 0 || p->step > 32767) return fail("mbe_evolve_layouts: step=%d outside 0..32767", p->step);
+  const double probs[4] = {p->p_cross, p->p_move, p->p_add, p->p_del};
+  for (double q : probs)
+    if (!std::isfinite(q) || q < 0.0 || q > 1.0)
+      return fail("mbe_evolve_layouts: probability %g is not in [0, 1]", q);
+  const size_t xy_bytes = (size_t)E * B * 4, nbs_bytes = (size_t)E * 4;
+  const void* inputs[4] = {fitness, parent_xy, parent_nbs, elite_ids};
+  const size_t in_bytes[4] = {nbs_bytes, xy_bytes, nbs_bytes, (size_t)n_elite * 4};
+  for (int i = 0; i < 4; ++i)
+    if (ranges_overlap(child_xy, xy_bytes, inputs[i], in_bytes[i]) ||
+        ranges_overlap(child_nbs, nbs_bytes, inputs[i], in_bytes[i]))
+      return fail("mbe_evolve_layouts: child buffers overlap an input");
+  if (ranges_overlap(child_xy, xy_bytes, child_nbs, nbs_bytes))
+    return fail("mbe_evolve_layouts: child_xy and child_nbs overlap");
+  if (((uintptr_t)fitness | (uintptr_t)parent_xy | (uintptr_t)parent_nbs | (uintptr_t)elite_ids |
+       (uintptr_t)child_xy | (uintptr_t)child_nbs) & 3)
+    return fail("mbe_evolve_layouts: buffers must be 4-byte aligned");
+  const mbe::StepArgs& s = env->args;
+  mbe::EvolveArgs a = {};
+  a.fitness = fitness;
+  a.parent = reinterpret_cast<const uint32_t*>(parent_xy);
+  a.parent_nbs = parent_nbs;
+  a.elite_ids = elite_ids;
+  a.child = reinterpret_cast<uint32_t*>(child_xy);
+  a.child_nbs = child_nbs;
+  a.E = E, a.B = B, a.K = n_elite, a.T = p->tournament, a.step = p->step;
+  a.nmin = cfg.bs_random_min, a.nmax = std::min(cfg.bs_random_max, B);
+  a.env_offset = s.env_offset, a.generation = p->generation;
+  a.seed_lo = (unsigned)(p->seed & 0xffffffffu), a.seed_hi = (unsigned)(p->seed >> 32);
+  a.XM = (int)std::ceil(cfg.width) - 1, a.YM = (int)std::ceil(cfg.height) - 1;
+  a.wh_int = s.wh_int, a.wh_int_w = s.wh_int_w, a.wh_int_h = s.wh_int_h;
+  a.width = cfg.width, a.height = cfg.height;
+  a.p_cross = p->p_cross, a.p_move = p->p_move, a.p_add = p->p_add, a.p_del = p->p_del;
+  const size_t smem = (size_t)mbe::kEvolveThreads * B * 4;
+  MBE_ON_DEVICE(cfg.device);
+  mbe::evolve_kernel<<<(unsigned)((E + mbe::kEvolveThreads - 1) / mbe::kEvolveThreads), mbe::kEvolveThreads, smem,
+                       static_cast<cudaStream_t>(stream)>>>(a);
   MBE_CUDA(cudaGetLastError());
   env->launches += 1;
   return 0;
