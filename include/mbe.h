@@ -137,7 +137,13 @@ typedef struct mbe_config {
   mbe_link_class classes[MBE_MAX_CLASSES]; /* [bs class][ue class], ue class fastest */
   const uint8_t* bs_class; /* HOST [B] class id per BS slot, or NULL = all class 0 */
   int32_t num_ue_classes;  /* 0 or 1: all UEs alike (velocity / move_d2max above); else 2..MBE_MAX_UE_CLASSES */
-  int32_t reserved2;
+  /* M: UE trajectories per BS layout.  0 or 1: the flags alone decide (MBE_FLAG_SHARED_TRAJECTORY: one
+     trajectory for all envs).  M >= 2 needs MBE_FLAG_SHARED_TRAJECTORY, M a power of two, M <= num_envs,
+     num_envs % M == 0 and env_offset % M == 0; env of global id g then follows trajectory g mod M (its BS
+     layout draws still use g).  Convention: layout l occupies env rows l*M .. l*M + M-1 and replica m
+     follows trajectory m, on every rank and in every env window.  mbe_evolve_layouts breeds L =
+     num_envs / M layouts on such a handle. */
+  int32_t num_trajectories;
   const uint8_t* ue_class; /* HOST [U] class id per UE (required when num_ue_classes > 1) */
   mbe_ue_class ue_classes[MBE_MAX_UE_CLASSES]; /* used when num_ue_classes > 1 */
 } mbe_config;
@@ -259,7 +265,9 @@ typedef struct mbe_evolve_params {
 /* Breeds child_xy int16 [E,B,2] / child_nbs int32 [E] from parent_xy / parent_nbs and fitness f32 [E]
  * (all DEVICE, 4-byte aligned; E, B and the layout ranges are the handle's, which needs random per-env
  * layouts).  Child c < n_elite copies parent elite_ids[c] verbatim when that id is in 0..E-1.  The
- * child buffers must not overlap any input.  One launch. */
+ * child buffers must not overlap any input.  One launch.  On a handle with num_trajectories = M >= 2 the
+ * population is the L = num_envs / M layouts, not the env rows: every array above is [L, ...], n_elite
+ * lies in 0..L, and the Philox child id is env_offset / M + child. */
 int mbe_evolve_layouts(mbe_env* env, const float* fitness, const int16_t* parent_xy, const int32_t* parent_nbs,
                        const int32_t* elite_ids, int n_elite, const mbe_evolve_params* p, int16_t* child_xy,
                        int32_t* child_nbs, void* stream);

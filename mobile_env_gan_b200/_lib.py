@@ -71,7 +71,7 @@ class Config(C.Structure):
         ("classes", BsClass * MAX_CLASSES),
         ("bs_class", C.POINTER(C.c_uint8)),
         ("num_ue_classes", C.c_int32),
-        ("reserved2", C.c_int32),
+        ("num_trajectories", C.c_int32),
         ("ue_class", C.POINTER(C.c_uint8)),
         ("ue_classes", UeClass * MAX_UE_CLASSES),
     ]

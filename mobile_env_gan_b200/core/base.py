@@ -61,6 +61,7 @@ class Plan:
     utility: tuple
     scheduler: int = 0
     shared_trajectory: bool = False
+    num_trajectories: int = 1  # M: env of global id g follows shared trajectory g mod M
     classes: List[dict] = field(default_factory=list)  # link classes [bs class][ue class], ue class fastest
     bs_class: Optional[np.ndarray] = None
     bs_xy: Optional[np.ndarray] = None  # shared layout [B,2] int16
@@ -117,6 +118,9 @@ class MComCore:
             # "follow_movement": True iff movement_params.reset_rng_episode -- the fork, where that flag
             # makes every epoch replay one UE trajectory (base.py:130-134) and env index = epoch number
             "shared_trajectory": False,
+            # M > 1 (a power of two, with shared_trajectory): env g follows trajectory g mod M, so the M
+            # env rows l*M .. l*M + M-1 score one BS layout over M UE trajectories (scoring.LayoutScorer)
+            "num_trajectories": 1,
             # the fork's collect loop (collectData2.ipynb cell 4) as written: step() dumps the four JSON
             # files of base.py:298-349 and keeps the per-epoch lists for save_epoch_data().  MComCustom
             # (the class that loop drives) defaults to None = on when there is ONE env, like the
@@ -216,14 +220,28 @@ class MComCore:
         shared = config.get("shared_trajectory", False)
         if shared == "follow_movement":
             shared = bool(movement.reset_rng_episode)
+        num_envs, env_offset = int(config["num_envs"]), int(config.get("env_offset", 0))
+        M = int(config.get("num_trajectories", 1))
+        if M < 1:
+            raise ValueError(f"num_trajectories={M} must be >= 1")
+        if M > 1:  # the rules mbe_create enforces (include/mbe.h, mbe_config.num_trajectories)
+            if not shared:
+                raise ValueError(f"num_trajectories={M} needs shared_trajectory (M shared UE trajectories)")
+            if M & (M - 1):
+                raise ValueError(f"num_trajectories={M} must be a power of two")
+            if M > num_envs or num_envs % M:
+                raise ValueError(f"num_envs={num_envs} must be a multiple of num_trajectories={M}")
+            if env_offset % M:
+                raise ValueError(f"env_offset={env_offset} must be a multiple of num_trajectories={M}")
         return Plan(
-            num_envs=int(config["num_envs"]), num_ues=len(users), num_bs=nbs, mode=mode, handler=handler,
+            num_envs=num_envs, num_ues=len(users), num_bs=nbs, mode=mode, handler=handler,
             bs_layout=layout, bs_random=bs_random, autoreset=bool(config.get("autoreset")),
             reset_rng_episode=bool(movement.reset_rng_episode), ep_time=ep_time,
-            env_offset=int(config.get("env_offset", 0)), seed=int(movement.seed),
+            env_offset=env_offset, seed=int(movement.seed),
             width=width, height=height, velocity=mv["velocity"], move_d2max=mv["move_d2max"],
             utility=(float(utility.lower), float(utility.upper), float(w1), float(w2), float(w3)),
-            scheduler=int(scheduler.kernel_id), shared_trajectory=bool(shared), classes=classes, bs_class=bs_class,
+            scheduler=int(scheduler.kernel_id), shared_trajectory=bool(shared), num_trajectories=M,
+            classes=classes, bs_class=bs_class,
             bs_xy=bs_xy, num_bs_classes=len(bs_protos), ue_class=ue_class if len(ue_protos) > 1 else None,
             ue_classes=ue_classes,
         )
@@ -336,6 +354,7 @@ class MComCore:
         cfg.num_classes = p.num_bs_classes
         cfg.flags = (_lib.FLAG_GENERIC_KERNEL if self.config.get("generic_kernel") else 0) | (
             _lib.FLAG_SHARED_TRAJECTORY if p.shared_trajectory else 0)
+        cfg.num_trajectories = p.num_trajectories
         for i, c in enumerate(p.classes):
             lut = np.ascontiguousarray(c["rate_lut"], dtype=np.float64)
             self._keepalive.append(lut)

@@ -220,6 +220,19 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
 
   if (cfg->env_offset < 0 || cfg->env_offset + (int64_t)cfg->num_envs > (int64_t)0xffffffffll)
     return fail("mbe_create: env_offset + num_envs must stay below 2^32 (global env ids are 32-bit Philox counter words)");
+  const int M = cfg->num_trajectories;
+  if (M < 0) return fail("mbe_create: num_trajectories=%d must be >= 0", M);
+  if (M >= 2) {
+    if (!(cfg->flags & MBE_FLAG_SHARED_TRAJECTORY))
+      return fail("mbe_create: num_trajectories=%d needs MBE_FLAG_SHARED_TRAJECTORY", M);
+    if (M & (M - 1)) return fail("mbe_create: num_trajectories=%d must be a power of two", M);
+    if (M > cfg->num_envs) return fail("mbe_create: num_trajectories=%d exceeds num_envs=%d", M, cfg->num_envs);
+    if (cfg->num_envs % M)
+      return fail("mbe_create: num_envs=%d must be a multiple of num_trajectories=%d", cfg->num_envs, M);
+    if (cfg->env_offset % M)
+      return fail("mbe_create: env_offset=%lld must be a multiple of num_trajectories=%d",
+                  (long long)cfg->env_offset, M);
+  }
   MBE_ON_DEVICE(cfg->device);
   mbe_env* env = new (std::nothrow) mbe_env();
   if (!env) return fail("mbe_create: out of host memory");
@@ -237,7 +250,8 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
   a.epw = env->big ? 1 : 32 / a.U;
   a.epb = a.epw * mbe::kWarpsPerBlock;
   a.env_offset = (unsigned)cfg->env_offset;
-  a.traj_gid_mask = (cfg->flags & MBE_FLAG_SHARED_TRAJECTORY) ? 0u : 0xffffffffu;
+  // shared trajectories: env g follows trajectory g & (M - 1), so M = 0 or 1 keeps trajectory 0 for all
+  a.traj_gid_mask = (cfg->flags & MBE_FLAG_SHARED_TRAJECTORY) ? (M >= 2 ? (unsigned)(M - 1) : 0u) : 0xffffffffu;
   a.ep_time = cfg->ep_time;
   a.autoreset = cfg->autoreset;
   a.reset_rng_episode = cfg->reset_rng_episode;
@@ -860,7 +874,9 @@ int mbe_evolve_layouts(mbe_env* env, const float* fitness, const int16_t* parent
   const mbe_config& cfg = env->cfg;
   if (cfg.bs_layout != MBE_BS_PER_ENV || cfg.bs_random_max <= 0)
     return fail("mbe_evolve_layouts: needs random per-env BS layouts (bs_layout=PER_ENV, bs_random_max > 0)");
-  const int E = cfg.num_envs, B = cfg.num_bs;
+  // with M >= 2 trajectories per layout the population is the L = num_envs / M layouts (mbe.h)
+  const int M = cfg.num_trajectories >= 2 ? cfg.num_trajectories : 1;
+  const int E = cfg.num_envs / M, B = cfg.num_bs;
   if (n_elite < 0 || n_elite > E) return fail("mbe_evolve_layouts: n_elite=%d outside 0..%d", n_elite, E);
   if (n_elite > 0 && !elite_ids) return fail("mbe_evolve_layouts: n_elite > 0 needs elite_ids");
   if (p->tournament < 1 || p->tournament > 4)
@@ -892,7 +908,7 @@ int mbe_evolve_layouts(mbe_env* env, const float* fitness, const int16_t* parent
   a.child_nbs = child_nbs;
   a.E = E, a.B = B, a.K = n_elite, a.T = p->tournament, a.step = p->step;
   a.nmin = cfg.bs_random_min, a.nmax = std::min(cfg.bs_random_max, B);
-  a.env_offset = s.env_offset, a.generation = p->generation;
+  a.env_offset = s.env_offset / (unsigned)M, a.generation = p->generation;
   a.seed_lo = (unsigned)(p->seed & 0xffffffffu), a.seed_hi = (unsigned)(p->seed >> 32);
   a.XM = (int)std::ceil(cfg.width) - 1, a.YM = (int)std::ceil(cfg.height) - 1;
   a.wh_int = s.wh_int, a.wh_int_w = s.wh_int_w, a.wh_int_h = s.wh_int_h;

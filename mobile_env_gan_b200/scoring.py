@@ -5,7 +5,11 @@ random layout and ranking them with ``qoeValue`` (mobile_env/chooseBaseStation.i
 
 over all two-decimal per-UE QoE values of the epoch (base.py:269).  With one env per layout the
 whole search is a batch: ``LayoutScorer`` accumulates the statistics on the device after every
-step (``mbe_accumulate_qoe``) and ranks the envs without any file round trip."""
+step (``mbe_accumulate_qoe``) and ranks the envs without any file round trip.
+
+With ``num_trajectories`` = M > 1 (DESIGN.md section 10) a layout is scored over M UE trajectories:
+layout l occupies the env rows l*M .. l*M + M-1, replica m follows trajectory m, and the score is
+``qoeValue`` over all QoE values of the M episodes, so every layout sees the same M trajectories."""
 from __future__ import annotations
 
 import ctypes as C
@@ -17,9 +21,35 @@ import torch
 from . import _lib
 
 
+def check_layouts(plan, bs_xy, nbs, L):
+    """Host check of L layouts for an env with random per-env layouts: shapes bs_xy [L, B, 2] /
+    nbs [L], counts in the scenario's ``bs_random`` range, live BSs on the map.  Returns int16 / int32
+    numpy copies with the slots at or beyond nbs set to (0, 0)."""
+    B = plan.num_bs
+    nmin, nmax = plan.bs_random[0], min(plan.bs_random[1], B)
+    xy = np.asarray(torch.as_tensor(bs_xy).cpu(), dtype=np.int64)
+    n = np.asarray(torch.as_tensor(nbs).cpu(), dtype=np.int64)
+    if xy.shape != (L, B, 2) or n.shape != (L,):
+        raise ValueError(f"a population must be bs_xy [{L}, {B}, 2] and nbs [{L}], got "
+                         f"{tuple(xy.shape)} and {tuple(n.shape)}")
+    if n.min() < nmin or n.max() > nmax:
+        raise ValueError(f"nbs must lie in [{nmin}, {nmax}]")
+    xm, ym = math.ceil(plan.width) - 1, math.ceil(plan.height) - 1
+    live = np.arange(B)[None, :] < n[:, None]
+    x, y = xy[..., 0][live], xy[..., 1][live]
+    if x.size and (x.min() < 0 or x.max() > xm or y.min() < 0 or y.max() > ym):
+        raise ValueError(f"BS coordinates must lie in [0, {xm}] x [0, {ym}]")
+    return np.where(live[..., None], xy, 0).astype(np.int16), n.astype(np.int32)
+
+
 class LayoutScorer:
+    """Scores the env's BS layouts: one per env, or with ``num_trajectories`` = M > 1 one per group of
+    M env rows (``num_layouts`` = num_envs / M), pooled over the M trajectories."""
+
     def __init__(self, env, low_qoe_threshold: float = 0.0, weights=(1.0, 0.1, 10.0)):
         self.env, self.threshold, self.weights = env, float(low_qoe_threshold), weights
+        self.M = env.plan.num_trajectories
+        self.num_layouts = env.num_envs // self.M
         self.acc = torch.zeros(env.num_envs, 4, dtype=torch.float32, device=env.device)
 
     def reset(self):
@@ -38,9 +68,21 @@ class LayoutScorer:
         return env.rollout(env.plan.ep_time if steps is None else steps, qoe_acc=self.acc,
                            threshold=self.threshold, record=record)
 
+    def pooled(self):
+        """The four accumulators per layout, f32 [num_layouts, 4]: the sum over the layout's M replica
+        rows, added left to right over m whatever the layout's index or the batch size, so the same
+        layout scored anywhere gets the same bits."""
+        if self.M == 1:
+            return self.acc
+        rows = self.acc.view(self.num_layouts, self.M, 4)
+        out = rows[:, 0].clone()
+        for m in range(1, self.M):
+            out += rows[:, m]
+        return out
+
     def result(self):
-        """Per-env dict of tensors with the notebook's keys."""
-        s1, s2, neg, n = self.acc.unbind(dim=1)
+        """Per-layout dict of tensors with the notebook's keys (per env when M = 1)."""
+        s1, s2, neg, n = self.pooled().unbind(dim=1)
         mean = s1 / n
         var = s2 / n - mean * mean  # np.var (population variance)
         low = neg / n
@@ -54,28 +96,47 @@ class LayoutScorer:
         top = torch.topk(score, k)
         return top.indices, top.values
 
+    def score_layouts(self, bs_xy, nbs):
+        """Scores ``num_layouts`` given layouts, bs_xy int [L, B, 2] / nbs int [L], with one episode:
+        resets the env and the statistics, writes layout l into its M replica rows, runs the episode
+        and returns the pooled ``Score`` f32 [L].  Scoring winners on an env built with another
+        ``seed`` (the UE trajectories are keyed by the movement seed) is a held-out evaluation."""
+        env, L, M = self.env, self.num_layouts, self.M
+        p = env.plan
+        if p.bs_layout != _lib.BS_PER_ENV or p.bs_random[1] <= 0:
+            raise ValueError("score_layouts needs per-env random BS layouts (config['bs_random'])")
+        xy, n = check_layouts(p, bs_xy, nbs, L)
+        env.reset()
+        env.bs_xy.view(L, M, p.num_bs, 2).copy_(torch.from_numpy(xy).to(env.device)[:, None])
+        env.nbs.view(L, M).copy_(torch.from_numpy(n).to(env.device)[:, None])
+        self.reset()
+        self.run_episode()
+        return self.result()["Score"]
+
 
 class LayoutEvolution:
-    """Genetic search over per-env BS layouts: the population is the env batch (one layout per env),
-    fitness is ``LayoutScorer``'s ``Score`` of one whole episode, and the next population is bred on
-    the GPU by ``mbe_evolve_layouts`` (DESIGN.md section 10): child c < ``elites`` is the c-th best
-    layout copied verbatim, every other child comes from tournament selection (``tournament``
-    candidates), uniform slot crossover (``p_cross``), per-slot moves of at most ``step`` map units
-    per axis (``p_move`` per slot), then at most one added (``p_add``) or deleted (``p_del``) BS within
-    the scenario's ``bs_random`` range.  Operator randomness is Philox keyed by ``seed`` and counted by
-    generation and global env id, so a search is reproducible and ranks sharded with ``env_offset``
-    breed disjoint islands.
+    """Genetic search over per-env BS layouts: the population is the env batch (one layout per env, or
+    one per M env rows with ``num_trajectories`` = M > 1), fitness is ``LayoutScorer``'s (pooled)
+    ``Score`` of one whole episode, and the next population is bred on the GPU by
+    ``mbe_evolve_layouts`` (DESIGN.md section 10): child c < ``elites`` is the c-th best layout copied
+    verbatim, every other child comes from tournament selection (``tournament`` candidates), uniform
+    slot crossover (``p_cross``), per-slot moves of at most ``step`` map units per axis (``p_move`` per
+    slot), then at most one added (``p_add``) or deleted (``p_del``) BS within the scenario's
+    ``bs_random`` range.  Operator randomness is Philox keyed by ``seed`` and counted by generation and
+    global layout id (env_offset / M + layout), so a search is reproducible and ranks sharded with
+    ``env_offset`` breed disjoint islands.
 
     The env must run in FORK mode with per-env layouts and ONE shared UE trajectory
     (``plan.shared_trajectory`` with movement ``reset_rng_episode``, MComCustom's default).  Only then is
     the fitness a function of the layout alone: an elite re-scored at another env index next generation
-    gets bit for bit the score it had, which is what makes keeping elites sound.
+    gets bit for bit the score it had, which is what makes keeping elites sound.  With M > 1 trajectories
+    every layout is scored over the same M trajectories, so the same holds for the pooled score.
 
-    ``bs_xy`` int [E, B, 2] / ``nbs`` int [E] set the initial population (slots at or beyond nbs are
-    ignored and stored as (0, 0)); by default it is the env's own random draw of ``reset()``, so
-    generation 0 is today's random search over ``num_envs`` layouts.  Defaults: tournament 4, p_cross
-    0.5, p_move 0.2, step 10 (5 % of MComCustom's 200 x 200 map), p_add = p_del = 0.1, elites 1/64 of the
-    population; of the tournament sizes 2, 3 and 4 measured in profiles/layout_evolution_bench.json, 4
+    ``bs_xy`` int [L, B, 2] / ``nbs`` int [L] set the initial population of L = num_envs / M layouts
+    (slots at or beyond nbs are ignored and stored as (0, 0)); by default it is the env's own random
+    draw of ``reset()`` (the draw of row l*M for layout l), so generation 0 is today's random search
+    over L layouts.  Defaults: tournament 4, p_cross 0.5, p_move 0.2, step 10 (5 % of MComCustom's
+    200 x 200 map), p_add = p_del = 0.1, elites 1/64 of the population; of the tournament sizes 2, 3 and 4 measured in profiles/layout_evolution_bench.json, 4
     reached the best score."""
 
     def __init__(self, env, *, elites: int = None, tournament: int = 4, p_cross: float = 0.5,
@@ -90,62 +151,47 @@ class LayoutEvolution:
             raise ValueError("LayoutEvolution needs one UE trajectory shared by all envs and episodes "
                              "(shared_trajectory and movement reset_rng_episode): otherwise fitness depends "
                              "on the env index, not on the layout alone")
-        E, B = p.num_envs, p.num_bs
+        M, B = p.num_trajectories, p.num_bs
+        E = p.num_envs // M  # layouts in the population
         elites = max(1, E // 64) if elites is None else int(elites)
         if not 0 <= elites <= E:
             raise ValueError(f"elites={elites} outside 0..{E}")
-        self.env, self.elites = env, elites
+        self.env, self.elites, self.M = env, elites, M
         self.scorer = LayoutScorer(env, low_qoe_threshold, weights)
         self.params = _lib.EvolveParams(seed=(p.seed if seed is None else int(seed)) & 0xFFFFFFFFFFFFFFFF,
                                         generation=0, tournament=int(tournament), step=int(step),
                                         p_cross=float(p_cross), p_move=float(p_move), p_add=float(p_add),
                                         p_del=float(p_del))
-        self.nmin, self.nmax = p.bs_random[0], min(p.bs_random[1], B)
         self._xy = torch.zeros(2, E, B, 2, dtype=torch.int16, device=env.device)
         self._nbs = torch.zeros(2, E, dtype=torch.int32, device=env.device)
         self._cur = 0
         if bs_xy is None and nbs is None:
             env.reset()
-            self._xy[0].copy_(env.bs_xy)
-            self._nbs[0].copy_(env.nbs)
+            self._xy[0].copy_(env.bs_xy.view(E, M, B, 2)[:, 0])
+            self._nbs[0].copy_(env.nbs.view(E, M)[:, 0])
         elif bs_xy is None or nbs is None:
             raise ValueError("an initial population needs both bs_xy and nbs")
         else:
-            xy, n = self._check_population(bs_xy, nbs)
+            xy, n = check_layouts(p, bs_xy, nbs, E)
             self._xy[0].copy_(torch.from_numpy(xy))
             self._nbs[0].copy_(torch.from_numpy(n))
         self.generation = 0
         self.fitness = None  # of the last scored population (self.population())
 
-    def _check_population(self, bs_xy, nbs):
-        p = self.env.plan
-        E, B = p.num_envs, p.num_bs
-        xy = np.asarray(torch.as_tensor(bs_xy).cpu(), dtype=np.int64)
-        n = np.asarray(torch.as_tensor(nbs).cpu(), dtype=np.int64)
-        if xy.shape != (E, B, 2) or n.shape != (E,):
-            raise ValueError(f"initial population must be bs_xy [{E}, {B}, 2] and nbs [{E}], got "
-                             f"{tuple(xy.shape)} and {tuple(n.shape)}")
-        if n.min() < self.nmin or n.max() > self.nmax:
-            raise ValueError(f"nbs must lie in [{self.nmin}, {self.nmax}]")
-        xm, ym = math.ceil(p.width) - 1, math.ceil(p.height) - 1
-        live = np.arange(B)[None, :] < n[:, None]
-        x, y = xy[..., 0][live], xy[..., 1][live]
-        if x.size and (x.min() < 0 or x.max() > xm or y.min() < 0 or y.max() > ym):
-            raise ValueError(f"BS coordinates must lie in [0, {xm}] x [0, {ym}]")
-        return np.where(live[..., None], xy, 0).astype(np.int16), n.astype(np.int32)
-
     def population(self):
-        """(bs_xy [E, B, 2], nbs [E]) that the last ``step()`` scored (the initial one before any step)."""
+        """(bs_xy [L, B, 2], nbs [L]) that the last ``step()`` scored (the initial one before any step)."""
         i = self._cur if self.fitness is None else 1 - self._cur
         return self._xy[i], self._nbs[i]
 
     def step(self):
         """Scores the current population with one episode and breeds the next; returns the fitness
-        tensor f32 [E] of the population just scored."""
-        env, cur = self.env, self._cur
+        tensor f32 [L] of the population just scored."""
+        env, cur, M = self.env, self._cur, self.M
+        L, B = self._nbs.shape[1], env.plan.num_bs
         env.reset()
-        env.bs_xy.copy_(self._xy[cur])  # per-env layouts are read from the bound buffers: no re-bind
-        env.nbs.copy_(self._nbs[cur])
+        # per-env layouts are read from the bound buffers: no re-bind; layout l goes to its M replica rows
+        env.bs_xy.view(L, M, B, 2).copy_(self._xy[cur][:, None])
+        env.nbs.view(L, M).copy_(self._nbs[cur][:, None])
         self.scorer.reset()
         self.scorer.run_episode()
         fit = self.scorer.result()["Score"]
