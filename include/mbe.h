@@ -214,7 +214,11 @@ int mbe_channel(mbe_env* env, float* out_snr, uint32_t* out_elig, void* stream);
 int mbe_observe(mbe_env* env, void* stream);
 
 /* adds this step's two-decimal QoE values (base.py:269) to acc f32 [E,4] = (sum q, sum q^2,
- * #q < threshold, #values): the statistics of chooseBaseStation.ipynb cell 5 `qoeValue` */
+ * #q < threshold, #values): the statistics of chooseBaseStation.ipynb cell 5 `qoeValue`.
+ * The cent k of a value is the exact half-even rounding of its FP32 utility times 100, q is
+ * float32(k / 100), and q counts as low when float32(k / 100) < float32(threshold).  That is Python's
+ * round(u, 2) < t for every cent-valued t; a threshold that rounds to the same float32 as a cent acts as
+ * that cent.  The counts are exact, the sums are FP32 in a fixed order (DESIGN.md section 2). */
 int mbe_accumulate_qoe(mbe_env* env, float* acc, float threshold, void* stream);
 
 /* per-step series of a fused episode: DEVICE pointers, any may be NULL; 16-byte aligned */
@@ -228,7 +232,8 @@ typedef struct mbe_rollout_out {
 
 /* FORK mode: `steps` consecutive MComCore.step calls (base.py:230-296; the fork's collect loop
  * `for s in range(20): env.step(e, s)`) in ONE launch -- state stays on chip between the steps.
- * qoe_acc (f32 [E,4], may be NULL) accumulates the statistics of mbe_accumulate_qoe over all steps;
+ * qoe_acc (f32 [E,4], may be NULL) accumulates the statistics of mbe_accumulate_qoe over all steps,
+ * with the same cents and low-QoE test, bit for bit;
  * `out` (may be NULL) receives the per-step series.  After the call the bound buffers hold exactly
  * what `steps` calls of mbe_step would have left.  Shapes without the fused kernel run the same
  * episode as a sequence of step launches (same results). */

@@ -296,6 +296,25 @@ __device__ __forceinline__ float scaled_utility(const StepArgs& a, double rate) 
   return (rate <= 0.0) ? -1.0f : u;  // rate <= 0 -> lower bound -> scaled -1
 }
 
+// The two-decimal QoE value behind the layout score (base.py:269 stores round(qoe, 2)), shared by
+// qoe_accumulate_kernel and the fused episode so that both keep agreeing bit for bit (include/mbe.h
+// mbe_accumulate_qoe): the cent k is the exact half-even rounding of u * 100 and the value is
+// float32(k / 100).  u * 100 rounded to FP32 lands exactly on a half for some u whose exact product
+// lies off it (u = float32(0.015) = 0.01499999966 gives 1.5); the FMA residual of that product is exact
+// and says on which side.  k * 0.01f is not float32(k / 100) for 60 of the 201 cents (10 * 0.01f =
+// 0.099999994f < 0.1f); one correction with the exact residual k - 100 * q0 gives the correctly rounded
+// quotient for every |k| <= 100.  __fmul_rn keeps the products from being contracted into FMAs.
+__device__ __forceinline__ float qoe_cent_value(float u) {
+  const float p = __fmul_rn(u, 100.0f);
+  float k = rintf(p);
+  if (fabsf(p - k) == 0.5f) {
+    const float e = fmaf(u, 100.0f, -p);
+    if (e != 0.0f) k = p + copysignf(0.5f, e);
+  }
+  const float q0 = __fmul_rn(k, 0.01f);
+  return fmaf(fmaf(-q0, 100.0f, k), 0.01f, q0);
+}
+
 // mean over the connected UEs (metrics.py:18-21): 0 when nobody is connected
 __device__ __forceinline__ float mean_or_zero(float sum, float n) { return n > 0.0f ? __fdividef(sum, n) : 0.0f; }
 

@@ -404,6 +404,7 @@ __global__ void __launch_bounds__(kThreads) channel_kernel(const __grid_constant
 // cell 5 `qoeValue`: mean - 0.1*var - 10*P(qoe < threshold) over all two-decimal QoE values of an
 // epoch, as stored by base.py:269).  One warp per env adds this step's U values to acc[env] =
 // (sum q, sum q^2, #q < threshold, #values); a fixed lane-strided order keeps it deterministic.
+// q is qoe_cent_value (mbe_device.cuh): float32(k / 100) of the exact half-even cent k.
 __global__ void __launch_bounds__(kThreads) qoe_accumulate_kernel(const float* __restrict__ utility, float4* acc, int E,
                                                                   int U, float threshold) {
   const int env = blockIdx.x * (kThreads / 32) + (threadIdx.x >> 5);
@@ -411,7 +412,7 @@ __global__ void __launch_bounds__(kThreads) qoe_accumulate_kernel(const float* _
   if (env >= E) return;
   float s1 = 0.0f, s2 = 0.0f, neg = 0.0f;
   for (int u = lane; u < U; u += 32) {
-    float q = rintf(utility[(size_t)env * U + u] * 100.0f) * 0.01f;  // round(qoe, 2)
+    const float q = qoe_cent_value(utility[(size_t)env * U + u]);  // round(qoe, 2)
     s1 += q;
     s2 = fmaf(q, q, s2);
     neg += (q < threshold) ? 1.0f : 0.0f;

@@ -264,7 +264,7 @@ __global__ void __launch_bounds__(32, ROLLOUT ? MBE_TPE_ROLLOUT_BLOCKS : MBE_TPE
     float q1[U], q2[U], ql[U];
 #pragma unroll
     for (int u = 0; u < U; ++u) {
-      const float q = rintf(s.util[lane * U + u] * 100.0f) * 0.01f;
+      const float q = qoe_cent_value(s.util[lane * U + u]);
       q1[u] = q;
       q2[u] = fmaf(q, q, 0.0f);
       ql[u] = (q < a.qoe_thr) ? 1.0f : 0.0f;

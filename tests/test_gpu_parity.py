@@ -821,8 +821,8 @@ def test_layout_scorer_matches_notebook_formula():
     all_qoe = np.concatenate(qoe, axis=1)  # [E, T*U]
     want = all_qoe.mean(axis=1) - 0.1 * all_qoe.var(axis=1) - 10.0 * (all_qoe < 0.0).mean(axis=1)
     got = scorer.result()
-    # FP32 utilities may round to the neighbouring cent in a few of the 140 values per env
-    np.testing.assert_allclose(got["Score"].cpu().numpy(), want, atol=0.08, rtol=0)
+    # the kernels' cents are the FP64 cents (tests/test_qoe_statistics.py): only FP32 summation differs
+    np.testing.assert_allclose(got["Score"].cpu().numpy(), want, atol=1e-5, rtol=0)
     assert np.abs(got["Score"].cpu().numpy() - want).mean() < 2e-3
     np.testing.assert_allclose(got["Average QoE"].cpu().numpy(), all_qoe.mean(axis=1), atol=2e-4)
     idx, _ = scorer.best(5)

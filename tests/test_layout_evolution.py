@@ -291,7 +291,7 @@ def test_layout_evolution_on_custom():
     qoe = [np.round(mir.step_fork()["utility"], 2) for _ in range(env8.plan.ep_time)]
     q = np.concatenate(qoe, axis=1)
     want = q.mean(axis=1) - 0.1 * q.var(axis=1) - 10.0 * (q < 0.0).mean(axis=1)
-    np.testing.assert_allclose(score.cpu().numpy(), want, atol=0.08, rtol=0)
+    np.testing.assert_allclose(score.cpu().numpy(), want, atol=1e-5, rtol=0)
     assert np.abs(score.cpu().numpy() - want).mean() < 2e-3
     _, fresh = _fresh_score(xy.repeat(4, 1, 1), nbs.repeat(4))  # 32 envs: the same fused kernel
     assert torch.equal(fresh.view(4, 8), score.expand(4, 8))

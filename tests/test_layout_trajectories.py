@@ -191,7 +191,7 @@ def test_assoc_rates_and_pooled_scores_match_the_mirror():
     want = q.mean(axis=1) - 0.1 * q.var(axis=1) - 10.0 * (q < 0.0).mean(axis=1)
     for score in (sc.result()["Score"], LayoutScorer(env).score_layouts(xy, nbs)):
         assert score.shape == (L,)
-        np.testing.assert_allclose(score.cpu().numpy(), want, atol=0.08, rtol=0)
+        np.testing.assert_allclose(score.cpu().numpy(), want, atol=1e-5, rtol=0)
         assert np.abs(score.cpu().numpy() - want).mean() < 2e-3
     idx, top = sc.best(5)
     assert int(idx.max()) < L
