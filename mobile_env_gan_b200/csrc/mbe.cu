@@ -7,6 +7,8 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
+#include <memory>
 #include <new>
 #include <string>
 #include <vector>
@@ -62,6 +64,19 @@ struct DeviceGuard {
   DeviceGuard guard_(dev);                                                                          \
   if (guard_.err != cudaSuccess) return fail("cudaSetDevice(%d): %s", dev, cudaGetErrorString(guard_.err))
 
+// One step-kernel launch: the kernel instance and everything launch() needs to run it.
+struct StepKernel {
+  void (*fn)(mbe::StepArgs) = nullptr;
+  const char* name = "";     // what mbe_step_kernel_name reports
+  int threads = 0, epb = 0;  // CTA size and envs per CTA (grid = ceil(E / epb))
+  size_t smem = 0;           // dynamic shared memory per CTA
+  bool pdl = false;          // launched with programmatic stream serialization
+  bool whole_warps = false;  // thread per env: takes only E % 32 == 0 and 16-byte aligned buffers
+  bool prefetch = false;     // prefetches state slices pf_dist CTAs ahead into L2
+  int pf_dist = 0;           // (prefetch) set at create from the kernel's occupancy
+  bool bound_ok = true;      // (whole_warps) the bound buffers are aligned; set by mbe_bind
+};
+
 }  // namespace
 
 struct mbe_env {
@@ -70,33 +85,22 @@ struct mbe_env {
   bool bound = false;
   mbe::StepArgs args;
   std::vector<void*> luts;  // device tables owned by the handle
-  uint8_t* d_bs_class = nullptr;
-  uint8_t* d_ue_class = nullptr;
-  size_t smem = 0;
-  int grid = 0;
   int64_t launches = 0;
-  // specialised fused kernel for this shape (nullptr: generic kernel only)
-  void (*spec)(mbe::StepArgs) = nullptr;
-  size_t spec_smem = 0;
-  bool big = false;  // block-per-env kernel (wide shapes, ProportionalFair)
-  // several-UEs-per-thread kernel (GYM scenario shapes, shared layout)
-  void (*upt)(mbe::StepArgs) = nullptr;
-  size_t upt_smem = 0;
-  int upt_epb = 0;
-  int upt_pf = 0, spec_pf = 0;  // L2 prefetch distance (CTAs) of the two kernel families, 0 = off
-  bool pf_bound_ok = false;     // the prefetched streams are 16-byte aligned
-  // thread-per-env FORK kernel (per-env layouts, E % 32 == 0, 16-byte aligned buffers)
-  void (*tpe)(mbe::StepArgs) = nullptr;
-  size_t tpe_smem = 0;
-  bool tpe_bound_ok = false;
-  void (*big_fn)(mbe::StepArgs) = nullptr;       // block-per-env kernel instance (UEs per thread by U)
-  size_t big_smem = 0;
-  bool tpe_shared = false;                       // the fused episode of a shared layout (no per-env BS table)
-  void (*tpe_rollout)(mbe::StepArgs) = nullptr;  // the same kernel looping over the steps of an episode
-  size_t tpe_rollout_smem = 0;
+  // general: the generic or the block-per-env kernel, which serves every op.  steps: the whole-step
+  // kernels of this shape in priority order (see pick).  episode: the fused rollout (fn == nullptr: none).
+  StepKernel general, episode;
+  std::vector<StepKernel> steps;
+  bool prefetch_ok = false;  // the prefetched streams (pos, wp, conn, actions) are 16-byte aligned
   // mbe_step_host pipeline: second stream + fork/join events (created on first use)
   cudaStream_t host_stream = nullptr;
   cudaEvent_t host_fork = nullptr, host_join = nullptr;
+
+  template <class F>
+  void each_kernel(F f) {
+    f(general);
+    for (StepKernel& k : steps) f(k);
+    if (episode.fn) f(episode);
+  }
 };
 
 namespace {
@@ -114,8 +118,64 @@ int pdl_mode() {
   }();
   return mode;
 }
-bool pdl_enabled() { return pdl_mode() == 1; }
-bool pdl_enabled_gym() { return pdl_mode() != 0; }
+
+// MBE_UPT=0 / MBE_TPE=0 turn a kernel family off (read at each mbe_create)
+bool family_on(const char* var) {
+  const char* v = std::getenv(var);
+  return !(v && v[0] == '0');
+}
+
+// wide shapes and the schedulers other than ResourceFair run on the block-per-env kernel alone
+bool block_per_env(const mbe_config& c) {
+  return c.num_ues > 32 || c.num_bs > 32 || c.scheduler != MBE_SCHED_RESOURCE_FAIR;
+}
+
+bool aligned16(std::initializer_list<const void*> ptrs) {
+  uintptr_t all = 0;
+  for (const void* p : ptrs) all |= (uintptr_t)p;
+  return (all & 15) == 0;
+}
+
+// Copies count host elements into a new device table that the handle owns (freed by mbe_destroy).
+template <class T>
+cudaError_t upload(mbe_env* env, const T* src, size_t count, T*& dst) {
+  void* p = nullptr;
+  cudaError_t e = cudaMalloc(&p, count * sizeof(T));
+  if (e != cudaSuccess) return e;
+  env->luts.push_back(p);
+  dst = static_cast<T*>(p);
+  return cudaMemcpy(p, src, count * sizeof(T), cudaMemcpyHostToDevice);
+}
+
+// The kernel that runs a launch of E envs: the first whole-step kernel that accepts it, else the
+// general one (reset, observe, the split phases and the debug SNR output only exist there).  A window
+// that is not a whole number of 32-env warps passes over the thread-per-env kernel to the warp-segment
+// kernel, which handles ragged tails.
+const StepKernel& pick(const mbe_env* env, int op, int phases, int E, bool dbg_snr) {
+  if (op == mbe::OP_STEP && phases == MBE_PHASE_ALL && !dbg_snr)
+    for (const StepKernel& k : env->steps)
+      if (k.bound_ok && (!k.whole_warps || E % 32 == 0)) return k;
+  return env->general;
+}
+
+// Launches k over the a.E envs of a on stream.
+int run(mbe_env* env, const StepKernel& k, mbe::StepArgs a, void* stream) {
+  a.epb = k.epb;  // envs per CTA of this mapping (bounds and size of the obs bulk store)
+  a.pf_dist = env->prefetch_ok ? k.pf_dist : 0;
+  cudaLaunchConfig_t lc = {};
+  lc.gridDim = dim3((a.E + k.epb - 1) / k.epb);
+  lc.blockDim = dim3(k.threads);
+  lc.dynamicSmemBytes = k.smem;
+  lc.stream = static_cast<cudaStream_t>(stream);
+  cudaLaunchAttribute pdl;
+  pdl.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  pdl.val.programmaticStreamSerializationAllowed = 1;
+  lc.attrs = &pdl;
+  lc.numAttrs = k.pdl ? 1 : 0;
+  MBE_CUDA(cudaLaunchKernelEx(&lc, k.fn, a));
+  env->launches += 1;
+  return 0;
+}
 
 struct SpecEntry {
   int mode, handler, U, B, per_env;
@@ -236,6 +296,7 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
   MBE_ON_DEVICE(cfg->device);
   mbe_env* env = new (std::nothrow) mbe_env();
   if (!env) return fail("mbe_create: out of host memory");
+  std::unique_ptr<mbe_env, void (*)(mbe_env*)> owned(env, mbe_destroy);  // released on success only
   env->cfg = *cfg;
   std::memset(&env->bufs, 0, sizeof env->bufs);
   mbe::StepArgs& a = env->args;
@@ -244,10 +305,10 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
   a.U = cfg->num_ues;
   a.B = cfg->num_bs;
   const bool gym = cfg->mode == MBE_MODE_GYM, ma = cfg->handler == MBE_HANDLER_MA;
-  env->big = a.U > 32 || a.B > 32 || cfg->scheduler != MBE_SCHED_RESOURCE_FAIR;
+  const bool big = block_per_env(*cfg);
   a.scheduler = cfg->scheduler;
   a.F = gym ? (ma ? 4 * a.B + 1 : 2 * a.B + 1) : 0;
-  a.epw = env->big ? 1 : 32 / a.U;
+  a.epw = big ? 1 : 32 / a.U;
   a.epb = a.epw * mbe::kWarpsPerBlock;
   a.env_offset = (unsigned)cfg->env_offset;
   // shared trajectories: env g follows trajectory g & (M - 1), so M = 0 or 1 keeps trajectory 0 for all
@@ -308,31 +369,19 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
     d.ltab_len = 0;
     if (h.log2snr_lut) {  // log2 snr per d2 (loss not affine in log-distance)
       float* pt = nullptr;
-      size_t bytes = (size_t)h.log2snr_len * sizeof(float);
-      cudaError_t e0 = cudaMalloc(&pt, bytes);
-      if (e0 == cudaSuccess) e0 = cudaMemcpy(pt, h.log2snr_lut, bytes, cudaMemcpyHostToDevice);
-      if (e0 != cudaSuccess) {
-        mbe_destroy(env);
-        return fail("mbe_create: log2snr_lut upload failed: %s", cudaGetErrorString(e0));
-      }
-      env->luts.push_back(pt);
+      if (cudaError_t e = upload(env, h.log2snr_lut, (size_t)h.log2snr_len, pt))
+        return fail("mbe_create: log2snr_lut upload failed: %s", cudaGetErrorString(e));
       d.ltab = pt;
       d.ltab_len = h.log2snr_len;
       any_ltab = true;
     }
     if (h.d2max >= 0) {  // the raw table, for the block-per-env kernel
       double* p0 = nullptr;
-      size_t bytes0 = (size_t)d.stride * sizeof(double);
-      cudaError_t e0 = cudaMalloc(&p0, bytes0);
-      if (e0 == cudaSuccess) e0 = cudaMemcpy(p0, h.rate_lut, bytes0, cudaMemcpyHostToDevice);
-      if (e0 != cudaSuccess) {
-        mbe_destroy(env);
-        return fail("mbe_create: rate_lut upload failed: %s", cudaGetErrorString(e0));
-      }
-      env->luts.push_back(p0);
+      if (cudaError_t e = upload(env, h.rate_lut, (size_t)d.stride, p0))
+        return fail("mbe_create: rate_lut upload failed: %s", cudaGetErrorString(e));
       d.lut0 = p0;
     }
-    if (h.d2max >= 0 && !env->big) {
+    if (h.d2max >= 0 && !big) {
       // device table: [0] = 0.0, then rows n = 1..U of round(rate_lut[d2] / n, 2) in FP64
       // (schedules.py:20-22, base.py:435); kernels index it as lutn[n*stride + d2]
       const int rows = a.U;
@@ -345,39 +394,25 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
           tab[1 + (size_t)(n - 1) * d.stride + i] = std::nearbyint(scaled) / 100.0;
         }
       double* p = nullptr;
-      size_t bytes = tab.size() * sizeof(double);
-      cudaError_t e = cudaMalloc(&p, bytes);
-      if (e == cudaSuccess) e = cudaMemcpy(p, tab.data(), bytes, cudaMemcpyHostToDevice);
-      if (e != cudaSuccess) {
-        mbe_destroy(env);
+      if (cudaError_t e = upload(env, tab.data(), tab.size(), p))
         return fail("mbe_create: rate table upload failed: %s", cudaGetErrorString(e));
-      }
-      env->luts.push_back(p);
       d.lutn = p + 1 - d.stride;  // biased: row n starts at lutn + n*stride, lutn[stride-1] == 0.0
     }
   }
   if (cfg->bs_class) {
     for (int b = 0; b < cfg->num_bs; ++b)
-      if (cfg->bs_class[b] >= cfg->num_classes) {
-        mbe_destroy(env);
+      if (cfg->bs_class[b] >= cfg->num_classes)
         return fail("mbe_create: bs_class[%d]=%d >= num_classes", b, cfg->bs_class[b]);
-      }
-    cudaError_t e = cudaMalloc(&env->d_bs_class, cfg->num_bs);
-    if (e == cudaSuccess) e = cudaMemcpy(env->d_bs_class, cfg->bs_class, cfg->num_bs, cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) {
-      mbe_destroy(env);
+    uint8_t* p = nullptr;
+    if (cudaError_t e = upload(env, cfg->bs_class, (size_t)cfg->num_bs, p))
       return fail("mbe_create: bs_class upload failed: %s", cudaGetErrorString(e));
-    }
-    a.bs_class = env->d_bs_class;
+    a.bs_class = p;
   }
   if (nuc > 1) {
-    cudaError_t e = cudaMalloc(&env->d_ue_class, cfg->num_ues);
-    if (e == cudaSuccess) e = cudaMemcpy(env->d_ue_class, cfg->ue_class, cfg->num_ues, cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) {
-      mbe_destroy(env);
+    uint8_t* p = nullptr;
+    if (cudaError_t e = upload(env, cfg->ue_class, (size_t)cfg->num_ues, p))
       return fail("mbe_create: ue_class upload failed: %s", cudaGetErrorString(e));
-    }
-    a.ue_class = env->d_ue_class;
+    a.ue_class = p;
   }
   for (int b = 0; b < mbe::kMaxSlots; ++b) {
     const int c = (cfg->bs_class && b < cfg->num_bs) ? cfg->bs_class[b] : 0;
@@ -394,129 +429,92 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
   // the specialised kernels assume one UE class, log2 snr affine in log-distance and squared
   // distances exact in FP32; the warp-segment ones take per-BS classes (folded per slot), the
   // UEs-per-thread and thread-per-env ones a single class
-  const bool spec_ok = nuc == 1 && !any_ltab &&
-                       std::floor(cfg->width) * std::floor(cfg->width) + std::floor(cfg->height) * std::floor(cfg->height) <
-                           16777216.0;
-  if (spec_ok && !(cfg->flags & MBE_FLAG_GENERIC_KERNEL)) {
-    for (const SpecEntry& sp : kSpecs)
-      if (sp.mode == cfg->mode && (sp.handler == cfg->handler || !gym) && sp.U == a.U && sp.B == a.B &&
-          sp.per_env == a.bs_per_env) {
-        if (cfg->num_classes > 1 && !sp.mc_fn) break;  // per-env layouts have one class: generic kernel
-        env->spec = cfg->num_classes > 1 ? sp.mc_fn : sp.fn;
-        env->spec_smem = sp.smem;
-        break;
-      }
-  }
-  {
-    const char* v = std::getenv("MBE_UPT");
-    const bool on = !(v && v[0] == '0');
-    if (on && spec_ok && cfg->num_classes == 1 && gym && !a.bs_per_env && !env->big &&
-        !(cfg->flags & MBE_FLAG_GENERIC_KERNEL))
-      for (const UptEntry& t : kUpts)
-        if (t.handler == cfg->handler && t.U == a.U && t.B == a.B) {
-          env->upt = t.fn;
-          env->upt_smem = t.smem;
-          env->upt_epb = (32 / t.K) * MBE_UPT_WARPS;
-        }
-  }
-  {
-    const char* v = std::getenv("MBE_TPE");
-    const bool on = !(v && v[0] == '0');
-    if (on && !gym && a.bs_per_env && spec_ok && cfg->num_classes == 1 && !env->big && a.E % 32 == 0 && a.U == 7 && a.B == 10 &&
-        cfg->width <= 2048 && cfg->height <= 2048 &&
-        !(cfg->flags & MBE_FLAG_GENERIC_KERNEL)) {
-      env->tpe = mbe::step_tpe_fork_kernel<7, 10>;
-      env->tpe_smem = sizeof(mbe::TpeForkSmem<7, 10>);
-      env->tpe_rollout = mbe::step_tpe_fork_kernel<7, 10, true>;
-      env->tpe_rollout_smem = sizeof(mbe::TpeRolloutSmem<7, 10>);
-    }
-    // the scenario shapes in FORK mode (one layout shared by all envs): the fused episode only (5 x 3 and
-    // 15 x 4); their single step stays on the warp-segment kernel
-    if (on && !gym && !a.bs_per_env && spec_ok && cfg->num_classes == 1 && !env->big && a.E % 32 == 0 &&
-        cfg->width <= 2048 && cfg->height <= 2048 && !(cfg->flags & MBE_FLAG_GENERIC_KERNEL)) {
-      env->tpe_shared = true;
-      if (a.U == 5 && a.B == 3) {
-        env->tpe_rollout = mbe::step_tpe_fork_kernel<5, 3, true, true>;
-        env->tpe_rollout_smem = sizeof(mbe::TpeRolloutSmem<5, 3>);
-      } else if (a.U == 15 && a.B == 4) {
-        env->tpe_rollout = mbe::step_tpe_fork_kernel<15, 4, true, true>;
-        env->tpe_rollout_smem = sizeof(mbe::TpeRolloutSmem<15, 4>);
-      } else {
-        // other shapes step episodes launch by launch.  A fused 30 x 13 episode (one env per lane walking
-        // 30 x 13 pairs in scalar code at 208 registers) took 1.43 ms per 20-step episode of 65,536 envs
-        // against 0.83 ms for 20 launches of the warp-segment kernel (profiles/r02_j_fork_rollout.txt);
-        // the small and medium shapes win 7.1x and 1.8x
-        env->tpe_shared = false;
-      }
-    }
-  }
-  if (env->big && std::floor(cfg->width) * std::floor(cfg->width) + std::floor(cfg->height) * std::floor(cfg->height) >=
-                      16777216.0) {
-    mbe_destroy(env);
+  const bool d2_exact =
+      std::floor(cfg->width) * std::floor(cfg->width) + std::floor(cfg->height) * std::floor(cfg->height) < 16777216.0;
+  const bool spec_ok = nuc == 1 && !any_ltab && d2_exact;
+  if (big && !d2_exact)
     return fail("mbe_create: the block-per-env kernel (wide shapes, ProportionalFair / RateFair) needs a map whose "
                 "squared diagonal is below 2^24 (distances are exact FP32 integers)");
-  }
-  env->smem = env->big ? 0 : mbe::smem_bytes(gym, ma, a.epb, a.U, a.B, a.F, a.bs_per_env);
-  env->grid = env->big ? a.E : (a.E + a.epb - 1) / a.epb;
-  if (env->big) env->spec = nullptr;
-  if (env->smem > 200 * 1024) {
-    mbe_destroy(env);
-    return fail("mbe_create: needs %zu bytes of shared memory per block", env->smem);
-  }
-  const void* fn = gym ? (ma ? (const void*)mbe::step_kernel<1, 1> : (const void*)mbe::step_kernel<1, 0>)
-                       : (const void*)mbe::step_kernel<0, 0>;
-  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->smem);
-  if (e == cudaSuccess && env->big) {
+  const size_t smem = big ? 0 : mbe::smem_bytes(gym, ma, a.epb, a.U, a.B, a.F, a.bs_per_env);
+  if (smem > 200 * 1024) return fail("mbe_create: needs %zu bytes of shared memory per block", smem);
+  if (big) {
     // UEs per thread held in registers: 2 (64 registers, 4 CTAs per SM) up to 512 UEs, else 4 (80 registers,
     // 3 CTAs per SM).  With the observation rows leaving as aligned bulk tiles the 2-UEs-per-thread instance
     // is the faster one where both fit: 802 vs 920 us per 16,384-env synthetic step
     // (profiles/r02_zb_variants.txt); while the rows were direct 4-byte stores it was the slower one
     // (1105 vs 1046 us, r02_q): more resident CTAs only meant more contention on misaligned sectors
     const bool two = a.U <= 2 * mbe::kBigThreads;
-    env->big_fn = gym ? (ma ? (two ? mbe::step_big_kernel<1, 1, 2> : mbe::step_big_kernel<1, 1, 4>)
-                            : (two ? mbe::step_big_kernel<1, 0, 2> : mbe::step_big_kernel<1, 0, 4>))
-                      : (two ? mbe::step_big_kernel<0, 0, 2> : mbe::step_big_kernel<0, 0, 4>);
-    env->big_smem = two ? mbe::big_smem_bytes<2>() : mbe::big_smem_bytes<4>();
-    e = cudaFuncSetAttribute((const void*)env->big_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->big_smem);
+    auto fn = gym ? (ma ? (two ? mbe::step_big_kernel<1, 1, 2> : mbe::step_big_kernel<1, 1, 4>)
+                        : (two ? mbe::step_big_kernel<1, 0, 2> : mbe::step_big_kernel<1, 0, 4>))
+                  : (two ? mbe::step_big_kernel<0, 0, 2> : mbe::step_big_kernel<0, 0, 4>);
+    env->general = StepKernel{fn, "step_big_kernel", mbe::kBigThreads, 1,
+                              two ? mbe::big_smem_bytes<2>() : mbe::big_smem_bytes<4>()};
+  } else {
+    auto fn = gym ? (ma ? mbe::step_kernel<1, 1> : mbe::step_kernel<1, 0>) : mbe::step_kernel<0, 0>;
+    env->general = StepKernel{fn, "step_kernel", mbe::kThreads, a.epb, smem};
   }
-  if (e == cudaSuccess && env->spec)
-    e = cudaFuncSetAttribute((const void*)env->spec, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)env->spec_smem);
-  if (e == cudaSuccess && env->upt)
-    e = cudaFuncSetAttribute((const void*)env->upt, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->upt_smem);
-  if (e == cudaSuccess && env->tpe)
-    e = cudaFuncSetAttribute((const void*)env->tpe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->tpe_smem);
-  if (e == cudaSuccess && env->tpe_rollout)
-    e = cudaFuncSetAttribute((const void*)env->tpe_rollout, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)env->tpe_rollout_smem);
-  if (e == cudaSuccess) {
-    // L2 prefetch distance: 0.75 waves of resident CTAs (measured best of 0.25 .. 2 waves on B200,
-    // profiles/README.md); MBE_PREFETCH=0 turns it off, MBE_PREFETCH=n sets the distance in CTAs
-    const char* v = std::getenv("MBE_PREFETCH");
-    const int forced = v ? std::atoi(v) : -1;
-    int sms = 0;
-    e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cfg->device);
-    auto dist = [&](const void* fn, int threads, size_t smem) {
-      int per_sm = 0;
-      if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, threads, smem);
-      return forced >= 0 ? forced : per_sm * sms * 3 / 4;
+  if (!big && spec_ok && !(cfg->flags & MBE_FLAG_GENERIC_KERNEL)) {
+    // the whole-step kernels of this shape, in priority order: thread per env, UEs per thread, warp segment
+    const bool pdl = gym ? pdl_mode() != 0 : pdl_mode() == 1;
+    const bool one_class = cfg->num_classes == 1;
+    auto tpe = [](void (*fn)(mbe::StepArgs), size_t bytes, bool with_pdl) {
+      return StepKernel{fn, "step_tpe_fork_kernel", 32, 32, bytes, with_pdl, /*whole_warps=*/true};
     };
-    if (env->upt) env->upt_pf = dist((const void*)env->upt, 32 * MBE_UPT_WARPS, env->upt_smem);
-    if (env->spec) env->spec_pf = dist((const void*)env->spec, mbe::kThreads, env->spec_smem);
+    if (family_on("MBE_TPE") && !gym && one_class && a.E % 32 == 0 && cfg->width <= 2048 && cfg->height <= 2048) {
+      if (a.bs_per_env && a.U == 7 && a.B == 10) {
+        env->steps.push_back(tpe(mbe::step_tpe_fork_kernel<7, 10>, sizeof(mbe::TpeForkSmem<7, 10>), pdl));
+        env->episode = tpe(mbe::step_tpe_fork_kernel<7, 10, true>, sizeof(mbe::TpeRolloutSmem<7, 10>), false);
+      }
+      // the scenario shapes in FORK mode (one layout shared by all envs): the fused episode only (5 x 3 and
+      // 15 x 4); their single step stays on the warp-segment kernel.  Other shapes step episodes launch by
+      // launch.  A fused 30 x 13 episode (one env per lane walking 30 x 13 pairs in scalar code at 208
+      // registers) took 1.43 ms per 20-step episode of 65,536 envs against 0.83 ms for 20 launches of the
+      // warp-segment kernel (profiles/r02_j_fork_rollout.txt); the small and medium shapes win 7.1x and 1.8x
+      if (!a.bs_per_env && a.U == 5 && a.B == 3)
+        env->episode = tpe(mbe::step_tpe_fork_kernel<5, 3, true, true>, sizeof(mbe::TpeRolloutSmem<5, 3>), false);
+      if (!a.bs_per_env && a.U == 15 && a.B == 4)
+        env->episode = tpe(mbe::step_tpe_fork_kernel<15, 4, true, true>, sizeof(mbe::TpeRolloutSmem<15, 4>), false);
+    }
+    if (family_on("MBE_UPT") && gym && !a.bs_per_env && one_class)
+      for (const UptEntry& t : kUpts)
+        if (t.handler == cfg->handler && t.U == a.U && t.B == a.B) {
+          env->steps.push_back(StepKernel{t.fn, "step_upt_kernel", 32 * MBE_UPT_WARPS, (32 / t.K) * MBE_UPT_WARPS,
+                                          t.smem, pdl, /*whole_warps=*/false, /*prefetch=*/true});
+          break;
+        }
+    for (const SpecEntry& sp : kSpecs)
+      if (sp.mode == cfg->mode && (sp.handler == cfg->handler || !gym) && sp.U == a.U && sp.B == a.B &&
+          sp.per_env == a.bs_per_env) {
+        // several BS classes: the multi-class instance (none for per-env layouts, which have one class)
+        if (void (*fn)(mbe::StepArgs) = one_class ? sp.fn : sp.mc_fn)
+          env->steps.push_back(StepKernel{fn, "step_spec_kernel", mbe::kThreads, a.epb, sp.smem, pdl,
+                                          /*whole_warps=*/false, /*prefetch=*/true});
+        break;
+      }
   }
-  if (e != cudaSuccess) {
-    mbe_destroy(env);
-    return fail("mbe_create: cudaFuncSetAttribute(%zu B smem): %s", env->smem, cudaGetErrorString(e));
-  }
-  *out = env;
+  // L2 prefetch distance: 0.75 waves of resident CTAs (measured best of 0.25 .. 2 waves on B200,
+  // profiles/README.md); MBE_PREFETCH=0 turns it off, MBE_PREFETCH=n sets the distance in CTAs
+  const char* v = std::getenv("MBE_PREFETCH");
+  const int forced = v ? std::atoi(v) : -1;
+  int sms = 0;
+  cudaError_t e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cfg->device);
+  env->each_kernel([&](StepKernel& k) {
+    if (e == cudaSuccess)
+      e = cudaFuncSetAttribute((const void*)k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem);
+    if (!k.prefetch) return;
+    int per_sm = 0;
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)k.fn, k.threads, k.smem);
+    k.pf_dist = forced >= 0 ? forced : per_sm * sms * 3 / 4;
+  });
+  if (e != cudaSuccess)
+    return fail("mbe_create: cudaFuncSetAttribute(%zu B smem): %s", smem, cudaGetErrorString(e));
+  *out = owned.release();
   return 0;
 }
 
 void mbe_destroy(mbe_env* env) {
   if (!env) return;
   for (void* p : env->luts) cudaFree(p);
-  if (env->d_bs_class) cudaFree(env->d_bs_class);
-  if (env->d_ue_class) cudaFree(env->d_ue_class);
   if (env->host_stream) cudaStreamDestroy(env->host_stream);
   if (env->host_fork) cudaEventDestroy(env->host_fork);
   if (env->host_join) cudaEventDestroy(env->host_join);
@@ -560,20 +558,14 @@ int mbe_bind(mbe_env* env, const mbe_buffers* b) {
   a.wp_cnt = b->wp_cnt;
   a.inj_k = b->inj_k;
   a.obs_bulk_ok = b->obs && (((uintptr_t)b->obs & 15) == 0);
-  {
-    uintptr_t all = (uintptr_t)b->pos | (uintptr_t)b->wp | (uintptr_t)b->t | (uintptr_t)b->episode |
-                    (uintptr_t)b->bs_xy | (uintptr_t)b->nbs | (uintptr_t)b->assoc | (uintptr_t)b->rate |
-                    (uintptr_t)b->utility | (uintptr_t)b->done | (uintptr_t)b->metrics;
-    // bulk async copies need 16-byte aligned global addresses; the FORK thread-per-env kernel also needs nbs
-    env->tpe_bound_ok = (all & 15) == 0 && b->nbs != nullptr;
-    if (env->tpe_shared) {
-      all = (uintptr_t)b->pos | (uintptr_t)b->wp | (uintptr_t)b->t | (uintptr_t)b->episode | (uintptr_t)b->assoc |
-            (uintptr_t)b->rate | (uintptr_t)b->utility | (uintptr_t)b->done | (uintptr_t)b->metrics;
-      env->tpe_bound_ok = (all & 15) == 0;
-    }
-    uintptr_t pf = (uintptr_t)b->pos | (uintptr_t)b->wp | (uintptr_t)b->conn | (uintptr_t)b->actions;
-    env->pf_bound_ok = (pf & 15) == 0;
-  }
+  // the thread-per-env kernels move their streams by bulk async copies, which need 16-byte aligned global
+  // addresses; with a per-env layout they also read its BS table and nbs
+  const bool tpe_ok =
+      a.bs_per_env ? aligned16({b->pos, b->wp, b->t, b->episode, b->bs_xy, b->nbs, b->assoc, b->rate, b->utility,
+                                b->done, b->metrics}) && b->nbs != nullptr
+                   : aligned16({b->pos, b->wp, b->t, b->episode, b->assoc, b->rate, b->utility, b->done, b->metrics});
+  env->each_kernel([&](StepKernel& k) { k.bound_ok = !k.whole_warps || tpe_ok; });
+  env->prefetch_ok = aligned16({b->pos, b->wp, b->conn, b->actions});
   if (!a.bs_per_env) {
     // a shared layout is constant for the life of the binding: fold the coordinates into the
     // kernel parameters (constant bank) for the specialised kernels
@@ -630,77 +622,9 @@ static int launch(mbe_env* env, int op, int phases, const uint8_t* mask, void* s
   a.op = op;
   a.phases = phases;
   a.reset_mask = mask;
-  const bool window = window_count > 0;
-  if (window) shift_window(a, env->cfg.handler == MBE_HANDLER_MA && env->cfg.mode == MBE_MODE_GYM, window_first, window_count);
-  const int grid = env->big ? a.E : (a.E + a.epb - 1) / a.epb;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const bool gym = env->cfg.mode == MBE_MODE_GYM, ma = env->cfg.handler == MBE_HANDLER_MA;
-  if (env->big) {
-    env->big_fn<<<grid, mbe::kBigThreads, env->big_smem, st>>>(a);
-    MBE_CUDA(cudaGetLastError());
-    env->launches += 1;
-    return 0;
-  }
-  // (a window that is not a whole number of 32-env warps falls through to the warp-segment kernels,
-  // which handle ragged tails)
-  if (env->tpe && env->tpe_bound_ok && a.E % 32 == 0 && op == mbe::OP_STEP && phases == MBE_PHASE_ALL && !a.dbg_snr) {
-    cudaLaunchConfig_t lc = {};
-    lc.gridDim = dim3(a.E / 32);
-    lc.blockDim = dim3(32);
-    lc.dynamicSmemBytes = env->tpe_smem;
-    lc.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    lc.attrs = attr;
-    lc.numAttrs = pdl_enabled() ? 1 : 0;
-    MBE_CUDA(cudaLaunchKernelEx(&lc, env->tpe, a));
-    env->launches += 1;
-    return 0;
-  }
-  if (env->upt && op == mbe::OP_STEP && phases == MBE_PHASE_ALL && !a.dbg_snr) {
-    a.epb = env->upt_epb;  // envs per CTA of this mapping (bounds and size of the obs bulk store)
-    a.pf_dist = env->pf_bound_ok ? env->upt_pf : 0;
-    cudaLaunchConfig_t lc = {};
-    lc.gridDim = dim3((a.E + a.epb - 1) / a.epb);
-    lc.blockDim = dim3(32 * MBE_UPT_WARPS);
-    lc.dynamicSmemBytes = env->upt_smem;
-    lc.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    lc.attrs = attr;
-    lc.numAttrs = pdl_enabled_gym() ? 1 : 0;
-    MBE_CUDA(cudaLaunchKernelEx(&lc, env->upt, a));
-    env->launches += 1;
-    return 0;
-  }
-  // the debug SNR output only exists in the generic kernel
-  if (env->spec && op == mbe::OP_STEP && phases == MBE_PHASE_ALL && !a.dbg_snr)
-  {
-    const bool pdl = gym ? pdl_enabled_gym() : pdl_enabled();
-    cudaLaunchConfig_t lc = {};
-    a.pf_dist = env->pf_bound_ok ? env->spec_pf : 0;
-    lc.gridDim = dim3(grid);
-    lc.blockDim = dim3(mbe::kThreads);
-    lc.dynamicSmemBytes = env->spec_smem;
-    lc.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    lc.attrs = attr;
-    lc.numAttrs = pdl ? 1 : 0;
-    MBE_CUDA(cudaLaunchKernelEx(&lc, env->spec, a));
-  }
-  else if (!gym)
-    mbe::step_kernel<0, 0><<<grid, mbe::kThreads, env->smem, st>>>(a);
-  else if (!ma)
-    mbe::step_kernel<1, 0><<<grid, mbe::kThreads, env->smem, st>>>(a);
-  else
-    mbe::step_kernel<1, 1><<<grid, mbe::kThreads, env->smem, st>>>(a);
-  MBE_CUDA(cudaGetLastError());
-  env->launches += 1;
-  return 0;
+  if (window_count > 0)
+    shift_window(a, env->cfg.handler == MBE_HANDLER_MA && env->cfg.mode == MBE_MODE_GYM, window_first, window_count);
+  return run(env, pick(env, op, phases, a.E, a.dbg_snr != nullptr), a, stream);
 }
 
 int mbe_reset(mbe_env* env, const uint8_t* env_mask, void* stream) {
@@ -768,8 +692,8 @@ int mbe_rollout(mbe_env* env, int steps, float* qoe_acc, float threshold, const 
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const mbe::StepArgs& a0 = env->args;
   const size_t EU = (size_t)a0.E * a0.U;
-  const uintptr_t series = (uintptr_t)o.pos | (uintptr_t)o.wp | (uintptr_t)o.assoc | (uintptr_t)o.rate | (uintptr_t)o.utility;
-  if (env->tpe_rollout && env->tpe_bound_ok && !a0.dbg_snr && (series & 15) == 0 && (o.rate == nullptr || a0.rate)) {
+  if (env->episode.fn && env->episode.bound_ok && !a0.dbg_snr && aligned16({o.pos, o.wp, o.assoc, o.rate, o.utility}) &&
+      (o.rate == nullptr || a0.rate)) {
     // fused episode: one launch, state read and written once
     mbe::StepArgs a = a0;
     a.op = mbe::OP_STEP;
@@ -783,10 +707,7 @@ int mbe_rollout(mbe_env* env, int steps, float* qoe_acc, float threshold, const 
     a.ro_assoc = o.assoc;
     a.ro_rate = o.rate;
     a.ro_util = o.utility;
-    env->tpe_rollout<<<a.E / 32, 32, env->tpe_rollout_smem, st>>>(a);
-    MBE_CUDA(cudaGetLastError());
-    env->launches += 1;
-    return 0;
+    return run(env, env->episode, a, stream);
   }
   // other shapes: the same episode as a sequence of step launches
   if ((o.pos || o.wp) && env->cfg.autoreset)
@@ -925,13 +846,9 @@ int mbe_evolve_layouts(mbe_env* env, const float* fitness, const int16_t* parent
 
 int64_t mbe_launch_count(const mbe_env* env) { return env ? env->launches : 0; }
 
-const char* mbe_step_kernel_name(const mbe_env* env) {  // mirrors the dispatch order of launch()
+const char* mbe_step_kernel_name(const mbe_env* env) {
   if (!env) return "";
-  if (env->big) return "step_big_kernel";
-  if (env->tpe && (!env->bound || env->tpe_bound_ok) && !env->args.dbg_snr) return "step_tpe_fork_kernel";
-  if (env->upt && !env->args.dbg_snr) return "step_upt_kernel";
-  if (env->spec && !env->args.dbg_snr) return "step_spec_kernel";
-  return "step_kernel";
+  return pick(env, mbe::OP_STEP, MBE_PHASE_ALL, env->cfg.num_envs, env->args.dbg_snr != nullptr).name;
 }
 
 int mbe_step_host(mbe_env* env, const int32_t* actions_host, float* obs_host, float* reward_host,
@@ -953,7 +870,7 @@ int mbe_step_host(mbe_env* env, const int32_t* actions_host, float* obs_host, fl
   const char* wv = std::getenv("MBE_HOST_WINDOWS");
   const int want = wv ? std::max(1, std::atoi(wv)) : (obs_host ? 4 : 1);
   constexpr int kAlign = 384;  // multiple of every kernel's envs-per-CTA and of 32 (16-byte aligned slices)
-  int windows = std::min(want, std::max(1, a.E / (env->big ? kAlign : 8 * kAlign)));
+  int windows = std::min(want, std::max(1, a.E / (block_per_env(env->cfg) ? kAlign : 8 * kAlign)));
   const int per = ((a.E + windows - 1) / windows + kAlign - 1) / kAlign * kAlign;
   windows = (a.E + per - 1) / per;
   if (windows > 1 && !env->host_stream) {

@@ -389,13 +389,23 @@ def test_bs_isolines_uses_the_reference_outline():
 
 def test_step_kernel_name_reports_the_dispatched_family():
     import mobile_env_gan_b200 as mbe
+    from mobile_env_gan_b200.core.schedules import ProportionalFair
+    from mobile_env_gan_b200.scenarios import MComSmall
     from mobile_env_gan_b200.scenarios.custom import MComCustom
 
     assert mbe.make("mobile-medium-central-v0", num_envs=64).step_kernel_name == "step_upt_kernel"
     assert mbe.make("mobile-large-ma-v0", num_envs=64).step_kernel_name == "step_spec_kernel"
     assert mbe.make("mobile-synthetic-central-v0", num_envs=4).step_kernel_name == "step_big_kernel"
+    # a shape with a warp-segment instance still runs on the block-per-env kernel under ProportionalFair
+    pf = mbe.make("mobile-medium-central-v0", num_envs=64, config={"scheduler": ProportionalFair})
+    assert pf.step_kernel_name == "step_big_kernel"
     assert MComCustom(config={"num_envs": 64}).step_kernel_name == "step_tpe_fork_kernel"
     assert MComCustom(config={"num_envs": 40}).step_kernel_name == "step_spec_kernel"  # E % 32 != 0
+    snr = MComCustom(config={"num_envs": 64})
+    snr.enable_debug_snr()  # the debug SNR output only exists in the generic kernel
+    assert snr.step_kernel_name == "step_kernel"
+    # a shared layout in FORK mode: only the fused episode is thread-per-env, the step is warp-segment
+    assert MComSmall(config={"num_envs": 64, "mode": "fork"}).step_kernel_name == "step_spec_kernel"
     generic = mbe.make("mobile-medium-central-v0", num_envs=64, config={"generic_kernel": True})
     assert generic.step_kernel_name == "step_kernel"
 
