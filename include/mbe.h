@@ -288,7 +288,7 @@ const char* mbe_step_kernel_name(const mbe_env* env);
 /* Host-buffer convenience: H2D actions, step, D2H obs/reward/done, then synchronises the
  * stream.  Host pointers should be pinned.  NULL pointers are skipped.  Large batches with
  * observations are processed as env windows on two streams so uploads and the step overlap the
- * download (MBE_HOST_WINDOWS=n overrides the window count). */
+ * download. */
 int mbe_step_host(mbe_env* env, const int32_t* actions_host, float* obs_host,
                   float* reward_host, uint8_t* done_host, void* stream);
 

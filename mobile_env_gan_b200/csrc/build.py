@@ -32,7 +32,7 @@ def is_stale() -> bool:
     return any(os.path.getmtime(d) > t for d in deps())
 
 
-def build(force: bool = False, verbose: bool = False, out: str = None, defines=()) -> str:
+def build(force: bool = False, verbose: bool = False, out: str = None) -> str:
     if out is None and not force and not is_stale():
         return LIB
     cmd = [
@@ -41,7 +41,7 @@ def build(force: bool = False, verbose: bool = False, out: str = None, defines=(
         "--expt-relaxed-constexpr", "--extended-lambda",
         "-Xptxas", "-v" if verbose else "-O3",
         "-o", out or LIB,
-    ] + [f"-D{d}" for d in defines] + [os.path.join(HERE, s) for s in SOURCES]
+    ] + [os.path.join(HERE, s) for s in SOURCES]
     res = subprocess.run(cmd, capture_output=True, text=True)
     if res.returncode != 0:
         raise RuntimeError("nvcc failed:\n" + res.stdout + res.stderr)

@@ -5,7 +5,6 @@
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <initializer_list>
 #include <memory>
@@ -105,26 +104,6 @@ struct mbe_env {
 
 namespace {
 
-// Programmatic dependent launch (the next step's CTAs become resident while this grid drains and
-// prefetch their state slices into L2 before the dependency wait).  Measured on B200
-// (profiles/README.md): 3-7% (graph replay) to 10% (plain launches) faster for the medium GYM
-// kernels, 14% for the small shape, neutral for the large one, 2% slower for the FORK kernels (no
-// prefetch there) -> default on for the GYM step kernels only; MBE_PDL=0 turns it off everywhere,
-// MBE_PDL=1 on everywhere.
-int pdl_mode() {
-  static const int mode = []() {
-    const char* v = std::getenv("MBE_PDL");
-    return !v ? -1 : (v[0] == '1' ? 1 : 0);
-  }();
-  return mode;
-}
-
-// MBE_UPT=0 / MBE_TPE=0 turn a kernel family off (read at each mbe_create)
-bool family_on(const char* var) {
-  const char* v = std::getenv(var);
-  return !(v && v[0] == '0');
-}
-
 // wide shapes and the schedulers other than ResourceFair run on the block-per-env kernel alone
 bool block_per_env(const mbe_config& c) {
   return c.num_ues > 32 || c.num_bs > 32 || c.scheduler != MBE_SCHED_RESOURCE_FAIR;
@@ -179,16 +158,16 @@ int run(mbe_env* env, const StepKernel& k, mbe::StepArgs a, void* stream) {
 
 struct SpecEntry {
   int mode, handler, U, B, per_env;
-  void (*fn)(mbe::StepArgs);
+  void (*fn)(mbe::StepArgs);     // one BS class (nullptr: not compiled, ONE = 0 below)
   size_t smem;
   void (*mc_fn)(mbe::StepArgs);  // several BS classes in a shared layout (nullptr for per-env layouts)
 };
 
-#define MBE_SPEC(MODE, HANDLER, U, B, PE)                                             \
-  SpecEntry {                                                                         \
-    MODE, HANDLER, U, B, PE, mbe::step_spec_kernel<MODE, HANDLER, U, B, (PE != 0)>,   \
-        mbe::spec_smem_bytes<HANDLER, U, B, (PE != 0)>(MODE == 1),                    \
-        mbe::spec_mc_kernel<MODE, HANDLER, U, B, (PE != 0)>()                         \
+#define MBE_SPEC(MODE, HANDLER, U, B, PE, ONE)                                                      \
+  SpecEntry {                                                                                       \
+    MODE, HANDLER, U, B, PE, mbe::spec_kernel<MODE, HANDLER, U, B, (PE != 0), false, (ONE != 0)>(), \
+        mbe::spec_smem_bytes<HANDLER, U, B, (PE != 0)>(MODE == 1),                                  \
+        mbe::spec_kernel<MODE, HANDLER, U, B, (PE != 0), true>()                                    \
   }
 
 // shapes with a compile-time specialisation: the scenario sizes of BASELINE.json (small 3x5,
@@ -203,10 +182,11 @@ struct UptEntry {
 // (small 5x3 with K=1 and large 30x13 with K=10 were measured slower than one thread per UE)
 const UptEntry kUpts[] = {MBE_UPT(0, 15, 4, 5), MBE_UPT(1, 15, 4, 5)};
 
+// ONE = 0: no one-class instance; the shared 15 x 4 GYM layout with one BS class always runs on kUpts
 const SpecEntry kSpecs[] = {
-    MBE_SPEC(1, 0, 5, 3, 0),  MBE_SPEC(1, 1, 5, 3, 0),  MBE_SPEC(1, 0, 15, 4, 0),  MBE_SPEC(1, 1, 15, 4, 0),
-    MBE_SPEC(1, 0, 30, 13, 0), MBE_SPEC(1, 1, 30, 13, 0), MBE_SPEC(0, 0, 7, 10, 1), MBE_SPEC(0, 0, 5, 3, 0),
-    MBE_SPEC(0, 0, 15, 4, 0), MBE_SPEC(0, 0, 30, 13, 0), MBE_SPEC(1, 0, 7, 10, 1),  MBE_SPEC(1, 1, 7, 10, 1),
+    MBE_SPEC(1, 0, 5, 3, 0, 1),   MBE_SPEC(1, 1, 5, 3, 0, 1),   MBE_SPEC(1, 0, 15, 4, 0, 0),  MBE_SPEC(1, 1, 15, 4, 0, 0),
+    MBE_SPEC(1, 0, 30, 13, 0, 1), MBE_SPEC(1, 1, 30, 13, 0, 1), MBE_SPEC(0, 0, 7, 10, 1, 1),  MBE_SPEC(0, 0, 5, 3, 0, 1),
+    MBE_SPEC(0, 0, 15, 4, 0, 1),  MBE_SPEC(0, 0, 30, 13, 0, 1), MBE_SPEC(1, 0, 7, 10, 1, 1),  MBE_SPEC(1, 1, 7, 10, 1, 1),
 };
 
 }  // namespace
@@ -455,12 +435,17 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
   }
   if (!big && spec_ok && !(cfg->flags & MBE_FLAG_GENERIC_KERNEL)) {
     // the whole-step kernels of this shape, in priority order: thread per env, UEs per thread, warp segment
-    const bool pdl = gym ? pdl_mode() != 0 : pdl_mode() == 1;
+    // Programmatic dependent launch (the next step's CTAs become resident while this grid drains and
+    // prefetch their state slices into L2 before the dependency wait).  Measured on B200
+    // (profiles/README.md): 3-7% (graph replay) to 10% (plain launches) faster for the medium GYM
+    // kernels, 14% for the small shape, neutral for the large one, 2% slower for the FORK kernels (no
+    // prefetch there) -> on for the GYM step kernels only.
+    const bool pdl = gym;
     const bool one_class = cfg->num_classes == 1;
     auto tpe = [](void (*fn)(mbe::StepArgs), size_t bytes, bool with_pdl) {
       return StepKernel{fn, "step_tpe_fork_kernel", 32, 32, bytes, with_pdl, /*whole_warps=*/true};
     };
-    if (family_on("MBE_TPE") && !gym && one_class && a.E % 32 == 0 && cfg->width <= 2048 && cfg->height <= 2048) {
+    if (!gym && one_class && a.E % 32 == 0 && cfg->width <= 2048 && cfg->height <= 2048) {
       if (a.bs_per_env && a.U == 7 && a.B == 10) {
         env->steps.push_back(tpe(mbe::step_tpe_fork_kernel<7, 10>, sizeof(mbe::TpeForkSmem<7, 10>), pdl));
         env->episode = tpe(mbe::step_tpe_fork_kernel<7, 10, true>, sizeof(mbe::TpeRolloutSmem<7, 10>), false);
@@ -475,17 +460,18 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
       if (!a.bs_per_env && a.U == 15 && a.B == 4)
         env->episode = tpe(mbe::step_tpe_fork_kernel<15, 4, true, true>, sizeof(mbe::TpeRolloutSmem<15, 4>), false);
     }
-    if (family_on("MBE_UPT") && gym && !a.bs_per_env && one_class)
+    if (gym && !a.bs_per_env && one_class)
       for (const UptEntry& t : kUpts)
         if (t.handler == cfg->handler && t.U == a.U && t.B == a.B) {
-          env->steps.push_back(StepKernel{t.fn, "step_upt_kernel", 32 * MBE_UPT_WARPS, (32 / t.K) * MBE_UPT_WARPS,
+          env->steps.push_back(StepKernel{t.fn, "step_upt_kernel", 32 * mbe::kUptWarps, (32 / t.K) * mbe::kUptWarps,
                                           t.smem, pdl, /*whole_warps=*/false, /*prefetch=*/true});
           break;
         }
     for (const SpecEntry& sp : kSpecs)
       if (sp.mode == cfg->mode && (sp.handler == cfg->handler || !gym) && sp.U == a.U && sp.B == a.B &&
           sp.per_env == a.bs_per_env) {
-        // several BS classes: the multi-class instance (none for per-env layouts, which have one class)
+        // several BS classes: the multi-class instance (none for per-env layouts, which have one class);
+        // one class: the one-class instance where one is compiled
         if (void (*fn)(mbe::StepArgs) = one_class ? sp.fn : sp.mc_fn)
           env->steps.push_back(StepKernel{fn, "step_spec_kernel", mbe::kThreads, a.epb, sp.smem, pdl,
                                           /*whole_warps=*/false, /*prefetch=*/true});
@@ -493,9 +479,7 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
       }
   }
   // L2 prefetch distance: 0.75 waves of resident CTAs (measured best of 0.25 .. 2 waves on B200,
-  // profiles/README.md); MBE_PREFETCH=0 turns it off, MBE_PREFETCH=n sets the distance in CTAs
-  const char* v = std::getenv("MBE_PREFETCH");
-  const int forced = v ? std::atoi(v) : -1;
+  // profiles/README.md)
   int sms = 0;
   cudaError_t e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cfg->device);
   env->each_kernel([&](StepKernel& k) {
@@ -504,7 +488,7 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
     if (!k.prefetch) return;
     int per_sm = 0;
     if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)k.fn, k.threads, k.smem);
-    k.pf_dist = forced >= 0 ? forced : per_sm * sms * 3 / 4;
+    k.pf_dist = per_sm * sms * 3 / 4;
   });
   if (e != cudaSuccess)
     return fail("mbe_create: cudaFuncSetAttribute(%zu B smem): %s", smem, cudaGetErrorString(e));
@@ -866,9 +850,8 @@ int mbe_step_host(mbe_env* env, const int32_t* actions_host, float* obs_host, fl
   // download: plain FP32 rows by DMA straight into obs_host (48 GB/s on the B200 box, no host thread
   // touches them).  A compact wire format (a third fewer bytes, expanded into obs_host by host threads)
   // measured 0.52-0.70x this DMA path on the 16-vCPU B200 box (profiles/README.md): the host must still
-  // write the FP32 rows.  MBE_HOST_WINDOWS overrides the number of windows.
-  const char* wv = std::getenv("MBE_HOST_WINDOWS");
-  const int want = wv ? std::max(1, std::atoi(wv)) : (obs_host ? 4 : 1);
+  // write the FP32 rows.
+  const int want = obs_host ? 4 : 1;
   constexpr int kAlign = 384;  // multiple of every kernel's envs-per-CTA and of 32 (16-byte aligned slices)
   int windows = std::min(want, std::max(1, a.E / (block_per_env(env->cfg) ? kAlign : 8 * kAlign)));
   const int per = ((a.E + windows - 1) / windows + kAlign - 1) / kAlign * kAlign;

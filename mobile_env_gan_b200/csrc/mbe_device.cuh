@@ -6,10 +6,7 @@
 
 namespace mbe {
 
-#ifndef MBE_WARPS_PER_BLOCK
-#define MBE_WARPS_PER_BLOCK 4
-#endif
-constexpr int kWarpsPerBlock = MBE_WARPS_PER_BLOCK;
+constexpr int kWarpsPerBlock = 4;
 constexpr int kThreads = kWarpsPerBlock * 32;
 constexpr unsigned kFull = 0xffffffffu;
 constexpr int kMaxSlots = 32;
@@ -280,7 +277,6 @@ __device__ __forceinline__ float log2_snr(const ClassDev& c, int d2) {
 __device__ __forceinline__ float log2_snr_obs_f(float k, float l0, float d2f) {
   return fmaf(-k, lg2_sfu(fmaxf(d2f, 1e-32f)), l0);
 }
-__device__ __forceinline__ float log2_snr_obs(float k, float l0, int d2) { return log2_snr_obs_f(k, l0, (float)d2); }
 // the same for any link class (runtime-shape kernels)
 __device__ __forceinline__ float log2_snr_obs(const ClassDev& c, int d2) {
   if (c.ltab) return c.ltab[min(d2, c.ltab_len - 1)];
@@ -321,16 +317,6 @@ __device__ __forceinline__ float mean_or_zero(float sum, float n) { return n > 0
 // Sum over the lanes of one env (contiguous segment of U lanes inside the warp), result
 // broadcast to every lane of the segment.  Fixed tree order => deterministic.
 __device__ __forceinline__ float seg_sum(float v, int u, int U, int lane) {
-  for (int off = 1; off < U; off <<= 1) {
-    float o = __shfl_down_sync(kFull, v, off);
-    if (u + off < U) v += o;
-  }
-  return __shfl_sync(kFull, v, lane - u);
-}
-
-template <int U>
-__device__ __forceinline__ float seg_sum_c(float v, int u, int lane) {
-#pragma unroll
   for (int off = 1; off < U; off <<= 1) {
     float o = __shfl_down_sync(kFull, v, off);
     if (u + off < U) v += o;

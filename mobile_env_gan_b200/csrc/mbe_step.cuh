@@ -1,6 +1,6 @@
 // Fused step kernel, "warp-segment" mapping (U <= 32, B <= 32):
 //   one thread per (env, UE); the U lanes of an env are a contiguous segment of a warp,
-//   floor(32/U) envs per warp, 8 warps per block.  Global index of a lane = env*U + ue, so
+//   floor(32/U) envs per warp, 4 warps per block.  Global index of a lane = env*U + ue, so
 //   every [E,U] stream is read/written fully coalesced; per-env reductions are warp
 //   ballots / match / segmented shuffles; the observation block [envs of the CTA, U, F] is
 //   staged in shared memory and leaves with ONE bulk async copy (TMA, UBLKCP in SASS).

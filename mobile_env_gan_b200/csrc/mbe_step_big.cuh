@@ -18,23 +18,16 @@
 #include <type_traits>
 #include "mbe_device.cuh"
 
-#ifndef MBE_BIG_MIN_BLOCKS
-#define MBE_BIG_MIN_BLOCKS 3
-#endif
-
 namespace mbe {
 
 constexpr int kBigThreads = 256;
 constexpr int kBigWarps = kBigThreads / 32;
 constexpr int kBigMaxI = 4;     // UEs per thread  => U <= 1024
-constexpr int kBigMaxU = kBigMaxI * kBigThreads;
 constexpr int kBigMaxB = 64;    // BS slots        => two 32-bit mask words
+constexpr int kBigMinBlocks = 3;  // resident CTAs per SM at 4 UEs per thread (one more at 2)
 // per-warp shared-memory tile of whole observation rows on their way out (floats): 8 rows of the 64-BS
 // central shape (8 x 129), 4 of the multi-agent one (4 x 257); 16-byte multiple
-#ifndef MBE_BIG_TILE_FLOATS
-#define MBE_BIG_TILE_FLOATS 1056
-#endif
-constexpr int kBigTileFloats = MBE_BIG_TILE_FLOATS;
+constexpr int kBigTileFloats = 1056;
 
 template <int MAXU>
 struct BigSmemT {
@@ -103,7 +96,7 @@ __device__ __forceinline__ double link_share(const StepArgs& a, const ClassDev& 
 // MAXI = UEs per thread held in registers (U <= MAXI * 256): 2 covers the synthetic 512-UE shape with 64
 // registers and 4 resident CTAs per SM, 4 (U <= 1024) needs 80 registers / 3 CTAs
 template <int MODE, int HANDLER, int MAXI = kBigMaxI>
-__global__ void __launch_bounds__(kBigThreads, MAXI <= 2 ? MBE_BIG_MIN_BLOCKS + 1 : MBE_BIG_MIN_BLOCKS) step_big_kernel(const __grid_constant__ StepArgs a) {
+__global__ void __launch_bounds__(kBigThreads, MAXI <= 2 ? kBigMinBlocks + 1 : kBigMinBlocks) step_big_kernel(const __grid_constant__ StepArgs a) {
   constexpr int kBigMaxI = MAXI;  // shadows the namespace constant inside this kernel
   constexpr bool GYM = (MODE == 1);
   constexpr bool MA = (HANDLER == 1);

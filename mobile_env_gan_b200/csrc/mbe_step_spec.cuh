@@ -9,25 +9,15 @@
 #pragma once
 #include "mbe_device.cuh"
 
+namespace mbe {
+
 // Resident CTAs (128 threads) per SM the register allocation is held to, tuned per kernel on B200
 // (profiles/README.md): the small central shapes run at full occupancy with 32 registers (10..16 CTAs
 // measure the same within noise), the multi-agent and wide shapes need more registers for their
 // per-BS arrays (large central 9 CTAs = 56 registers, large multi-agent 8 = 64).
-#ifndef MBE_SPEC_MIN_BLOCKS
-#define MBE_SPEC_MIN_BLOCKS(MODE, HANDLER, B) \
-  ((B) <= 4 ? ((HANDLER) == 1 ? 12 : MBE_SMALL_C_BLOCKS) : (B) <= 10 ? ((MODE) == 0 ? 11 : 10) : ((HANDLER) == 1 ? MBE_LARGE_MA_BLOCKS : MBE_LARGE_C_BLOCKS))
-#endif
-#ifndef MBE_SMALL_C_BLOCKS
-#define MBE_SMALL_C_BLOCKS 16
-#endif
-#ifndef MBE_LARGE_C_BLOCKS
-#define MBE_LARGE_C_BLOCKS 9
-#endif
-#ifndef MBE_LARGE_MA_BLOCKS
-#define MBE_LARGE_MA_BLOCKS 8
-#endif
-
-namespace mbe {
+constexpr int spec_min_blocks(int mode, int handler, int B) {
+  return B <= 4 ? (handler == 1 ? 12 : 16) : B <= 10 ? (mode == 0 ? 11 : 10) : (handler == 1 ? 8 : 9);
+}
 
 template <int HANDLER, int U, int B, bool PER_ENV>
 __host__ __device__ constexpr size_t spec_smem_bytes(bool gym) {
@@ -49,7 +39,9 @@ struct ChunkMem {
 };
 
 // One fused step of the EPB envs starting at env_base, state straight from global memory.  The
-// observation block is left in m.obs; the caller stores it.
+// observation block is left in m.obs; the caller stores it.  (Written inline in the kernel, the same
+// body compiles differently: the compiler then bounds threadIdx.x by the launch bounds and allocates
+// registers of the multi-agent instances anew, one of them with a spill.)
 template <int MODE, int HANDLER, int U, int B, bool PER_ENV, bool MC = false>
 __device__ __forceinline__ void step_chunk(const StepArgs& a, const int env_base, const ChunkMem& m) {
   constexpr bool GYM = (MODE == 1);
@@ -338,7 +330,7 @@ __device__ __forceinline__ void step_chunk(const StepArgs& a, const int env_base
 
 // ---- one chunk per CTA (works for any E) ----
 template <int MODE, int HANDLER, int U, int B, bool PER_ENV, bool MC = false>
-__global__ void __launch_bounds__(kThreads, MBE_SPEC_MIN_BLOCKS(MODE, HANDLER, B)) step_spec_kernel(const __grid_constant__ StepArgs a) {
+__global__ void __launch_bounds__(kThreads, spec_min_blocks(MODE, HANDLER, B)) step_spec_kernel(const __grid_constant__ StepArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr bool GYM = (MODE == 1);
   constexpr bool MA = (HANDLER == 1);
@@ -368,11 +360,13 @@ __global__ void __launch_bounds__(kThreads, MBE_SPEC_MIN_BLOCKS(MODE, HANDLER, B
   if (GYM) store_obs_block(a, m.obs, env_base, threadIdx.x, true);
 }
 
-// the multi-class instantiation of a shape (shared layouts only)
-template <int MODE, int HANDLER, int U, int B, bool PER_ENV>
-constexpr auto spec_mc_kernel() -> void (*)(StepArgs) {
-  if constexpr (PER_ENV) return nullptr;
-  else return step_spec_kernel<MODE, HANDLER, U, B, false, true>;
+// The instance of a shape for one BS class (MC = false) or several (MC = true), nullptr where none is
+// compiled: several classes need a shared layout, and WANTED = false leaves out a one-class case that
+// another kernel family always takes.
+template <int MODE, int HANDLER, int U, int B, bool PER_ENV, bool MC, bool WANTED = true>
+constexpr auto spec_kernel() -> void (*)(StepArgs) {
+  if constexpr (!WANTED || (MC && PER_ENV)) return nullptr;
+  else return step_spec_kernel<MODE, HANDLER, U, B, PER_ENV, MC>;
 }
 
 }  // namespace mbe

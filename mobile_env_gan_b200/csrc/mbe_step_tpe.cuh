@@ -109,12 +109,8 @@ __device__ __forceinline__ void bulk_store(void* gdst, const void* ssrc, uint32_
 }
 
 // resident one-warp CTAs per SM the register allocation is held to (step / fused episode)
-#ifndef MBE_TPE_BLOCKS
-#define MBE_TPE_BLOCKS 20
-#endif
-#ifndef MBE_TPE_ROLLOUT_BLOCKS
-#define MBE_TPE_ROLLOUT_BLOCKS 16
-#endif
+constexpr int kTpeBlocks = 20;
+constexpr int kTpeRolloutBlocks = 16;
 
 // |connections(b)| of one env, 4 bits per BS in one 64-bit word
 template <int U, int B>
@@ -127,7 +123,7 @@ struct TpeCounts {
 };
 
 template <int U, int B, bool ROLLOUT = false, bool SHARED = false>
-__global__ void __launch_bounds__(32, ROLLOUT ? MBE_TPE_ROLLOUT_BLOCKS : MBE_TPE_BLOCKS) step_tpe_fork_kernel(const __grid_constant__ StepArgs a) {
+__global__ void __launch_bounds__(32, ROLLOUT ? kTpeRolloutBlocks : kTpeBlocks) step_tpe_fork_kernel(const __grid_constant__ StepArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   using S = typename std::conditional<ROLLOUT, TpeRolloutSmem<U, B>, TpeForkSmem<U, B>>::type;
   static_assert(B <= 16, "the nearest-BS key keeps the BS index in 4 bits");

@@ -13,38 +13,30 @@
 #pragma once
 #include "mbe_device.cuh"
 
+namespace mbe {
+
 // resident CTAs per SM x 2 (register budget), tuned on B200: 7 for both handlers (72 registers, no
 // forced cap; 8 = 64 registers was best before the L2 prefetch, 3.5% slower with it)
-#ifndef MBE_UPT_BLOCKS_SMALL
-#define MBE_UPT_BLOCKS_SMALL 7
-#endif
-#ifndef MBE_UPT_BLOCKS_MA
-#define MBE_UPT_BLOCKS_MA 7
-#endif
-#define MBE_UPT_MIN_BLOCKS(HANDLER, B) ((B) <= 4 ? ((HANDLER) == 1 ? MBE_UPT_BLOCKS_MA : MBE_UPT_BLOCKS_SMALL) : 6)
+constexpr int kUptBlocks = 7;
 // warps per CTA of this mapping: 2 measured best (finer CTA granularity; 1 would break the 16-byte
 // size rule of the observation bulk store for U=15)
-#ifndef MBE_UPT_WARPS
-#define MBE_UPT_WARPS 2
-#endif
-
-namespace mbe {
+constexpr int kUptWarps = 2;
 
 template <int HANDLER, int U, int B, int K>
 __host__ __device__ constexpr size_t upt_smem_bytes() {
-  constexpr int EPB = (32 / K) * MBE_UPT_WARPS;
+  constexpr int EPB = (32 / K) * kUptWarps;
   constexpr int F = (HANDLER == 1 ? 4 : 2) * B + 1;
   return (((size_t)EPB * U * F * 4) + 15) & ~(size_t)15;
 }
 
 template <int HANDLER, int U, int B, int K>
-__global__ void __launch_bounds__(32 * MBE_UPT_WARPS, MBE_UPT_MIN_BLOCKS(HANDLER, B) * 4 / MBE_UPT_WARPS) step_upt_kernel(const __grid_constant__ StepArgs a) {
+__global__ void __launch_bounds__(32 * kUptWarps, kUptBlocks * 4 / kUptWarps) step_upt_kernel(const __grid_constant__ StepArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   static_assert(U % K == 0, "U must be a multiple of K");
   constexpr bool MA = (HANDLER == 1);
   constexpr int UPT = U / K;
   constexpr int EPW = 32 / K;
-  constexpr int EPB = EPW * MBE_UPT_WARPS;
+  constexpr int EPB = EPW * kUptWarps;
   constexpr int F = (MA ? 4 : 2) * B + 1;
   constexpr int NW = (B + 3) / 4;  // packed count words (8 bits per BS)
   float* s_obs = reinterpret_cast<float*>(smem_raw);
@@ -300,7 +292,7 @@ __global__ void __launch_bounds__(32 * MBE_UPT_WARPS, MBE_UPT_MIN_BLOCKS(HANDLER
     }
     if (k == 0) a.t[env] = t_e;
   }
-  store_obs_block<32 * MBE_UPT_WARPS>(a, s_obs, env_base, tid, true);
+  store_obs_block<32 * kUptWarps>(a, s_obs, env_base, tid, true);
 }
 
 }  // namespace mbe

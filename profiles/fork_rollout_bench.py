@@ -1,11 +1,9 @@
 #!/usr/bin/env python
-"""Fused episode (mbe_rollout, one launch) against the same episode as 20 step launches + score updates for the
-scenario shapes in FORK mode.  MBE_TPE=0 disables the thread-per-env kernels (the stepping path).
+"""Fused episode (``LayoutScorer.run_episode``: mbe_rollout, one launch where a fused kernel exists) against the
+same episode as 20 ``env.step`` + ``scorer.update`` calls, for the scenario shapes in FORK mode.
     python profiles/fork_rollout_bench.py [envs]"""
 import os
-import subprocess
 import sys
-import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -21,24 +19,27 @@ def main(E):
         env = cls(config={"num_envs": E, "autoreset": True, "mode": "fork"})
         sc = LayoutScorer(env)
         env.reset()
-        sc.run_episode(20)
-        torch.cuda.synchronize()
-        before = env.launch_count
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(10):
-            sc.run_episode(20)
-        e1.record()
-        torch.cuda.synchronize()
-        ms = e0.elapsed_time(e1) / 10
-        print(f"MBE_TPE={os.environ.get('MBE_TPE', '1')} {name:6s} E={E}: {ms:8.3f} ms per 20-step episode, "
-              f"{E * 20 / (ms * 1e-3) / 1e9:7.2f} G env-steps/s, {(env.launch_count - before) // 10} launches per episode", flush=True)
+
+        def stepped():
+            for s in range(20):
+                env.step(0, s)
+                sc.update()
+
+        for arm, episode in (("rollout", lambda: sc.run_episode(20)), ("step", stepped)):
+            episode()
+            torch.cuda.synchronize()
+            before = env.launch_count
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            for _ in range(10):
+                episode()
+            e1.record()
+            torch.cuda.synchronize()
+            ms = e0.elapsed_time(e1) / 10
+            print(f"{arm:7s} {name:6s} E={E}: {ms:8.3f} ms per 20-step episode, "
+                  f"{E * 20 / (ms * 1e-3) / 1e9:7.2f} G env-steps/s, {(env.launch_count - before) // 10} launches per episode",
+                  flush=True)
 
 
 if __name__ == "__main__":
-    E = int(sys.argv[1]) if len(sys.argv) > 1 else 65536
-    if os.environ.get("_CHILD"):
-        main(E)
-    else:
-        for tpe in ("1", "0"):
-            subprocess.run([sys.executable, __file__, str(E)], env=dict(os.environ, MBE_TPE=tpe, _CHILD="1"))
+    main(int(sys.argv[1]) if len(sys.argv) > 1 else 65536)

@@ -641,13 +641,12 @@ def test_step_host_roundtrip():
         ("mobile-large-ma-v0", 6500),
     ],
 )
-def test_step_host_windows_match_device_step(env_id, E, monkeypatch):
-    """mbe_step_host can split a batch into env windows on two streams (copy/step overlap), and
-    mbe_step_window steps a sub-range: both must reproduce the single whole-batch launch exactly,
-    over a full episode + autoreset."""
+def test_step_host_windows_match_device_step(env_id, E):
+    """mbe_step_host splits a batch with observations into env windows on two streams (copy/step
+    overlap), and mbe_step_window steps a sub-range: both must reproduce the single whole-batch launch
+    exactly, over a full episode + autoreset."""
     import mobile_env_gan_b200 as mbe
 
-    monkeypatch.setenv("MBE_HOST_WINDOWS", "3")
     a = mbe.make(env_id, num_envs=E, autoreset=True)  # host windows
     b = mbe.make(env_id, num_envs=E, autoreset=True)  # one launch
     c = mbe.make(env_id, num_envs=E, autoreset=True)  # explicit windows on two streams
@@ -677,19 +676,20 @@ def test_step_host_windows_match_device_step(env_id, E, monkeypatch):
         for name in ("pos", "wp", "t", "episode", "conn", "rate", "utility_scaled", "metrics", "obs", "reward", "done"):
             assert torch.equal(getattr(a, name), getattr(b, name)), name
             assert torch.equal(getattr(c, name), getattr(b, name)), name
-    assert a.launch_count - first_launches == min(3, E // 3072) * steps  # windows hold >= 3072 envs
+    assert a.launch_count - first_launches == min(4, E // 3072) * steps  # windows hold >= 3072 envs
 
 
-def test_step_host_windows_fork_custom(monkeypatch):
-    """Same for the fork's own scenario (thread-per-env FORK kernel, per-env random layouts)."""
+def test_step_host_matches_device_step_fork_custom():
+    """mbe_step_host in FORK mode (one window: no observations to download) reproduces the device step
+    for the fork's own scenario (thread-per-env FORK kernel, per-env random layouts)."""
     from mobile_env_gan_b200.scenarios.custom import MComCustom
 
-    monkeypatch.setenv("MBE_HOST_WINDOWS", "2")
     E = 8192
     a = MComCustom(config={"num_envs": E, "autoreset": True})
     b = MComCustom(config={"num_envs": E, "autoreset": True})
     a.reset(), b.reset()
     done_h = torch.empty(E, dtype=torch.uint8).pin_memory()
+    first_launches = a.launch_count
     for s in range(23):
         a.step_host(None, None, None, done_h)
         b.step(0, s)
@@ -697,6 +697,7 @@ def test_step_host_windows_fork_custom(monkeypatch):
         assert torch.equal(done_h, b.done.cpu())
         for name in ("pos", "wp", "t", "episode", "assoc", "rate", "utility_scaled", "metrics", "bs_xy", "nbs"):
             assert torch.equal(getattr(a, name), getattr(b, name)), name
+    assert a.launch_count - first_launches == 23
 
 
 # ------------------------------------------------- wide shapes / ProportionalFair (block-per-env)
