@@ -156,38 +156,76 @@ int run(mbe_env* env, const StepKernel& k, mbe::StepArgs a, void* stream) {
   return 0;
 }
 
-struct SpecEntry {
-  int mode, handler, U, B, per_env;
-  void (*fn)(mbe::StepArgs);     // one BS class (nullptr: not compiled, ONE = 0 below)
-  size_t smem;
-  void (*mc_fn)(mbe::StepArgs);  // several BS classes in a shared layout (nullptr for per-env layouts)
+// One compiled whole-step or fused-episode instance, the handles it serves (mode, handler: any in FORK mode,
+// U, B, BS layout, several BS classes or one) and its launch record, read from the kernel's header.
+// k.whole_warps also limits it to E % 32 == 0 and a map of at most 2048 x 2048 (packed nearest-BS key).
+struct Instance {
+  int mode, handler, U, B;
+  bool per_env, multi_class;
+  bool episode;  // the fused episode of mbe_rollout, else a whole step
+  StepKernel k;
 };
 
-#define MBE_SPEC(MODE, HANDLER, U, B, PE, ONE)                                                      \
-  SpecEntry {                                                                                       \
-    MODE, HANDLER, U, B, PE, mbe::spec_kernel<MODE, HANDLER, U, B, (PE != 0), false, (ONE != 0)>(), \
-        mbe::spec_smem_bytes<HANDLER, U, B, (PE != 0)>(MODE == 1),                                  \
-        mbe::spec_kernel<MODE, HANDLER, U, B, (PE != 0), true>()                                    \
-  }
+// Programmatic dependent launch (the next step's CTAs become resident while this grid drains and
+// prefetch their state slices into L2 before the dependency wait).  Measured on B200
+// (profiles/README.md): 3-7% (graph replay) to 10% (plain launches) faster for the medium GYM
+// kernels, 14% for the small shape, neutral for the large one, 2% slower for the FORK kernels (no
+// prefetch there) -> on for the GYM step kernels only.
+template <int MODE, int HANDLER, int U, int B, bool PER_ENV, bool MC>
+constexpr Instance spec() {
+  using L = mbe::SpecLayout<MODE, HANDLER, U, B, PER_ENV>;
+  return {MODE, HANDLER, U, B, PER_ENV, MC, false,
+          {mbe::step_spec_kernel<MODE, HANDLER, U, B, PER_ENV, MC>, "step_spec_kernel", mbe::kThreads, L::EPB, L::BYTES,
+           /*pdl=*/MODE == MBE_MODE_GYM, /*whole_warps=*/false, /*prefetch=*/true}};
+}
+template <int HANDLER, int U, int B, int K>
+constexpr Instance upt() {
+  using L = mbe::UptLayout<HANDLER, U, B, K>;
+  return {MBE_MODE_GYM, HANDLER, U, B, false, false, false,
+          {mbe::step_upt_kernel<HANDLER, U, B, K>, "step_upt_kernel", mbe::kUptThreads, L::EPB, L::BYTES,
+           /*pdl=*/true, /*whole_warps=*/false, /*prefetch=*/true}};
+}
+template <int U, int B, bool ROLLOUT, bool SHARED>
+constexpr Instance tpe() {
+  return {MBE_MODE_FORK, 0, U, B, !SHARED, false, ROLLOUT,
+          {mbe::step_tpe_fork_kernel<U, B, ROLLOUT, SHARED>, "step_tpe_fork_kernel", mbe::kTpeThreads,
+           mbe::kTpeEnvsPerCta, sizeof(mbe::TpeSmem<U, B, ROLLOUT>), /*pdl=*/false, /*whole_warps=*/true}};
+}
 
-// shapes with a compile-time specialisation: the scenario sizes of BASELINE.json (small 3x5,
-// medium 4x15, large 13x30) and the fork's MComCustom (7 UEs, <= 10 random BSs per env)
-struct UptEntry {
-  int handler, U, B, K;
-  void (*fn)(mbe::StepArgs);
-  size_t smem;
+// Every compiled instance.  A handle's whole-step kernels are the matching step rows in this order,
+// which is their priority (see pick): thread per env, UEs per thread, warp segment.  Shapes: the
+// scenario sizes of BASELINE.json (small 5 x 3, medium 15 x 4, large 30 x 13) and the fork's MComCustom
+// (7 UEs, <= 10 random BSs per env).
+constexpr Instance kInstances[] = {
+    // thread per env <U, B, fused episode, shared layout>: MComCustom's FORK step and fused episode.  The
+    // scenario shapes in FORK mode have the fused episode only; their single step stays on the warp-segment
+    // kernel.  A fused 30 x 13 episode (one env per lane walking 30 x 13 pairs in scalar code at 208
+    // registers) took 1.43 ms per 20-step episode of 65,536 envs against 0.83 ms for 20 launches of the
+    // warp-segment kernel (profiles/r02_j_fork_rollout.txt); the small and medium shapes win 7.1x and 1.8x.
+    tpe<7, 10, false, false>(), tpe<7, 10, true, false>(), tpe<5, 3, true, true>(), tpe<15, 4, true, true>(),
+    // UEs per thread <handler, U, B, K>: the shared 15 x 4 GYM layout with one BS class, which therefore
+    // has no one-class warp-segment instance (small 5 x 3 with K = 1 and large 30 x 13 with K = 10 were
+    // measured slower than one thread per UE)
+    upt<0, 15, 4, 5>(), upt<1, 15, 4, 5>(),
+    // warp segment <mode, handler, U, B, per-env layout, several BS classes>
+    spec<1, 0, 5, 3, false, false>(), spec<1, 1, 5, 3, false, false>(), spec<1, 0, 5, 3, false, true>(),
+    spec<1, 1, 5, 3, false, true>(), spec<1, 0, 15, 4, false, true>(), spec<1, 1, 15, 4, false, true>(),
+    spec<1, 0, 30, 13, false, false>(), spec<1, 1, 30, 13, false, false>(), spec<1, 0, 30, 13, false, true>(),
+    spec<1, 1, 30, 13, false, true>(), spec<1, 0, 7, 10, true, false>(), spec<1, 1, 7, 10, true, false>(),
+    spec<0, 0, 5, 3, false, false>(), spec<0, 0, 5, 3, false, true>(), spec<0, 0, 15, 4, false, false>(),
+    spec<0, 0, 15, 4, false, true>(), spec<0, 0, 30, 13, false, false>(), spec<0, 0, 30, 13, false, true>(),
+    spec<0, 0, 7, 10, true, false>(),
 };
-#define MBE_UPT(HANDLER, U, B, K) \
-  UptEntry { HANDLER, U, B, K, mbe::step_upt_kernel<HANDLER, U, B, K>, mbe::upt_smem_bytes<HANDLER, U, B, K>() }
-// (small 5x3 with K=1 and large 30x13 with K=10 were measured slower than one thread per UE)
-const UptEntry kUpts[] = {MBE_UPT(0, 15, 4, 5), MBE_UPT(1, 15, 4, 5)};
 
-// ONE = 0: no one-class instance; the shared 15 x 4 GYM layout with one BS class always runs on kUpts
-const SpecEntry kSpecs[] = {
-    MBE_SPEC(1, 0, 5, 3, 0, 1),   MBE_SPEC(1, 1, 5, 3, 0, 1),   MBE_SPEC(1, 0, 15, 4, 0, 0),  MBE_SPEC(1, 1, 15, 4, 0, 0),
-    MBE_SPEC(1, 0, 30, 13, 0, 1), MBE_SPEC(1, 1, 30, 13, 0, 1), MBE_SPEC(0, 0, 7, 10, 1, 1),  MBE_SPEC(0, 0, 5, 3, 0, 1),
-    MBE_SPEC(0, 0, 15, 4, 0, 1),  MBE_SPEC(0, 0, 30, 13, 0, 1), MBE_SPEC(1, 0, 7, 10, 1, 1),  MBE_SPEC(1, 1, 7, 10, 1, 1),
-};
+// mbe_step_host starts its env windows at multiples of kAlign envs: a multiple of 32 (16-byte aligned
+// slices) and of every instance's envs per CTA.  The generic kernel's 4 * floor(32 / U) envs per CTA need
+// not divide it (40 at U = 3): a window is a launch of its own, so only its last CTA may be partial.
+constexpr int kAlign = 384;
+static_assert([] {
+  for (const Instance& r : kInstances)
+    if (kAlign % r.k.epb) return false;
+  return kAlign % 32 == 0;
+}(), "kAlign must be a multiple of 32 and of every instance's envs per CTA");
 
 }  // namespace
 
@@ -288,8 +326,8 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
   const bool big = block_per_env(*cfg);
   a.scheduler = cfg->scheduler;
   a.F = gym ? (ma ? 4 * a.B + 1 : 2 * a.B + 1) : 0;
-  a.epw = big ? 1 : 32 / a.U;
-  a.epb = a.epw * mbe::kWarpsPerBlock;
+  a.epw = big ? 1 : mbe::envs_per_warp(a.U);  // the generic kernel's warp-segment mapping
+  a.epb = big ? 1 : mbe::segment_envs_per_cta(a.U);
   a.env_offset = (unsigned)cfg->env_offset;
   // shared trajectories: env g follows trajectory g & (M - 1), so M = 0 or 1 keeps trajectory 0 for all
   a.traj_gid_mask = (cfg->flags & MBE_FLAG_SHARED_TRAJECTORY) ? (M >= 2 ? (unsigned)(M - 1) : 0u) : 0xffffffffu;
@@ -434,48 +472,15 @@ int mbe_create(const mbe_config* cfg, mbe_env** out) {
     env->general = StepKernel{fn, "step_kernel", mbe::kThreads, a.epb, smem};
   }
   if (!big && spec_ok && !(cfg->flags & MBE_FLAG_GENERIC_KERNEL)) {
-    // the whole-step kernels of this shape, in priority order: thread per env, UEs per thread, warp segment
-    // Programmatic dependent launch (the next step's CTAs become resident while this grid drains and
-    // prefetch their state slices into L2 before the dependency wait).  Measured on B200
-    // (profiles/README.md): 3-7% (graph replay) to 10% (plain launches) faster for the medium GYM
-    // kernels, 14% for the small shape, neutral for the large one, 2% slower for the FORK kernels (no
-    // prefetch there) -> on for the GYM step kernels only.
-    const bool pdl = gym;
-    const bool one_class = cfg->num_classes == 1;
-    auto tpe = [](void (*fn)(mbe::StepArgs), size_t bytes, bool with_pdl) {
-      return StepKernel{fn, "step_tpe_fork_kernel", 32, 32, bytes, with_pdl, /*whole_warps=*/true};
-    };
-    if (!gym && one_class && a.E % 32 == 0 && cfg->width <= 2048 && cfg->height <= 2048) {
-      if (a.bs_per_env && a.U == 7 && a.B == 10) {
-        env->steps.push_back(tpe(mbe::step_tpe_fork_kernel<7, 10>, sizeof(mbe::TpeForkSmem<7, 10>), pdl));
-        env->episode = tpe(mbe::step_tpe_fork_kernel<7, 10, true>, sizeof(mbe::TpeRolloutSmem<7, 10>), false);
-      }
-      // the scenario shapes in FORK mode (one layout shared by all envs): the fused episode only (5 x 3 and
-      // 15 x 4); their single step stays on the warp-segment kernel.  Other shapes step episodes launch by
-      // launch.  A fused 30 x 13 episode (one env per lane walking 30 x 13 pairs in scalar code at 208
-      // registers) took 1.43 ms per 20-step episode of 65,536 envs against 0.83 ms for 20 launches of the
-      // warp-segment kernel (profiles/r02_j_fork_rollout.txt); the small and medium shapes win 7.1x and 1.8x
-      if (!a.bs_per_env && a.U == 5 && a.B == 3)
-        env->episode = tpe(mbe::step_tpe_fork_kernel<5, 3, true, true>, sizeof(mbe::TpeRolloutSmem<5, 3>), false);
-      if (!a.bs_per_env && a.U == 15 && a.B == 4)
-        env->episode = tpe(mbe::step_tpe_fork_kernel<15, 4, true, true>, sizeof(mbe::TpeRolloutSmem<15, 4>), false);
-    }
-    if (gym && !a.bs_per_env && one_class)
-      for (const UptEntry& t : kUpts)
-        if (t.handler == cfg->handler && t.U == a.U && t.B == a.B) {
-          env->steps.push_back(StepKernel{t.fn, "step_upt_kernel", 32 * mbe::kUptWarps, (32 / t.K) * mbe::kUptWarps,
-                                          t.smem, pdl, /*whole_warps=*/false, /*prefetch=*/true});
-          break;
-        }
-    for (const SpecEntry& sp : kSpecs)
-      if (sp.mode == cfg->mode && (sp.handler == cfg->handler || !gym) && sp.U == a.U && sp.B == a.B &&
-          sp.per_env == a.bs_per_env) {
-        // several BS classes: the multi-class instance (none for per-env layouts, which have one class);
-        // one class: the one-class instance where one is compiled
-        if (void (*fn)(mbe::StepArgs) = one_class ? sp.fn : sp.mc_fn)
-          env->steps.push_back(StepKernel{fn, "step_spec_kernel", mbe::kThreads, a.epb, sp.smem, pdl,
-                                          /*whole_warps=*/false, /*prefetch=*/true});
-        break;
+    const bool whole_warps = a.E % 32 == 0 && cfg->width <= 2048 && cfg->height <= 2048;
+    for (const Instance& r : kInstances)
+      if (r.mode == cfg->mode && (!gym || r.handler == cfg->handler) && r.U == a.U && r.B == a.B &&
+          r.per_env == (a.bs_per_env != 0) && r.multi_class == (cfg->num_classes > 1) &&
+          (!r.k.whole_warps || whole_warps)) {
+        if (r.episode)
+          env->episode = r.k;
+        else
+          env->steps.push_back(r.k);
       }
   }
   // L2 prefetch distance: 0.75 waves of resident CTAs (measured best of 0.25 .. 2 waves on B200,
@@ -852,7 +857,6 @@ int mbe_step_host(mbe_env* env, const int32_t* actions_host, float* obs_host, fl
   // measured 0.52-0.70x this DMA path on the 16-vCPU B200 box (profiles/README.md): the host must still
   // write the FP32 rows.
   const int want = obs_host ? 4 : 1;
-  constexpr int kAlign = 384;  // multiple of every kernel's envs-per-CTA and of 32 (16-byte aligned slices)
   int windows = std::min(want, std::max(1, a.E / (block_per_env(env->cfg) ? kAlign : 8 * kAlign)));
   const int per = ((a.E + windows - 1) / windows + kAlign - 1) / kAlign * kAlign;
   windows = (a.E + per - 1) / per;

@@ -11,6 +11,12 @@ constexpr int kThreads = kWarpsPerBlock * 32;
 constexpr unsigned kFull = 0xffffffffu;
 constexpr int kMaxSlots = 32;
 
+// Envs per warp when an env takes `lanes` adjacent lanes of it (the lanes past the last env idle).
+__host__ __device__ constexpr int envs_per_warp(int lanes) { return 32 / lanes; }
+// Envs per CTA of the warp-segment mapping (generic and specialised kernels): U lanes per env,
+// kWarpsPerBlock warps per CTA.
+__host__ __device__ constexpr int segment_envs_per_cta(int U) { return envs_per_warp(U) * kWarpsPerBlock; }
+
 enum Op : int { OP_STEP = 0, OP_RESET = 1, OP_OBSERVE = 2 };
 enum Purpose : unsigned { P_WAYPOINT = 0, P_INITPOS = 1, P_BSLAYOUT = 2 };
 

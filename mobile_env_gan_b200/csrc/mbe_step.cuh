@@ -17,6 +17,8 @@ struct Smem {
   uint8_t* cls;    // [B]
 };
 
+// Size of step_kernel's shared-memory carve-up for epb envs per CTA.  The kernel carves inline: through a
+// layout function shared with this one its three instances compile to different code (register order).
 __host__ __device__ inline size_t smem_bytes(int mode_gym, int handler_ma, int epb, int U, int B, int F,
                                             int bs_per_env) {
   size_t n = 0;

@@ -19,16 +19,18 @@ constexpr int spec_min_blocks(int mode, int handler, int B) {
   return B <= 4 ? (handler == 1 ? 12 : 16) : B <= 10 ? (mode == 0 ? 11 : 10) : (handler == 1 ? 8 : 9);
 }
 
-template <int HANDLER, int U, int B, bool PER_ENV>
-__host__ __device__ constexpr size_t spec_smem_bytes(bool gym) {
-  constexpr int EPB = (32 / U) * kWarpsPerBlock;
-  constexpr int F = (HANDLER == 1 ? 4 : 2) * B + 1;
-  size_t n = gym ? (size_t)EPB * U * F * 4 : 0;
-  n = (n + 15) & ~(size_t)15;
-  if (PER_ENV) n += (size_t)EPB * B * 4;
-  if (gym && HANDLER == 1) n += (size_t)EPB * B * 8;
-  return (n + 15) & ~(size_t)15;
-}
+// Envs per CTA of an instance and its dynamic shared memory: the observation staging block (GYM) at 0,
+// then the per-env BS table (PER_ENV), then the multi-agent BS utilities and counts (GYM, multi-agent).
+// The host sizes the launch with EPB and BYTES, the kernel carves its shared memory with the offsets.
+template <int MODE, int HANDLER, int U, int B, bool PER_ENV>
+struct SpecLayout {
+  static constexpr int EPB = segment_envs_per_cta(U);
+  static constexpr int F = MODE == 1 ? (HANDLER == 1 ? 4 : 2) * B + 1 : 0;
+  static constexpr size_t BS = ((size_t)EPB * U * F * 4 + 15) & ~(size_t)15;
+  static constexpr size_t BSU = BS + (PER_ENV ? (size_t)EPB * B * 4 : 0);
+  static constexpr size_t BSN = BSU + (size_t)EPB * B * 4;
+  static constexpr size_t BYTES = ((MODE == 1 && HANDLER == 1 ? BSN + (size_t)EPB * B * 4 : BSU) + 15) & ~(size_t)15;
+};
 
 // Shared / staged memory one chunk of envs (the envs of one CTA iteration) works on.
 struct ChunkMem {
@@ -46,9 +48,10 @@ template <int MODE, int HANDLER, int U, int B, bool PER_ENV, bool MC = false>
 __device__ __forceinline__ void step_chunk(const StepArgs& a, const int env_base, const ChunkMem& m) {
   constexpr bool GYM = (MODE == 1);
   constexpr bool MA = (HANDLER == 1);
-  constexpr int EPW = 32 / U;
-  constexpr int EPB = EPW * kWarpsPerBlock;
-  constexpr int F = GYM ? ((MA ? 4 : 2) * B + 1) : 0;
+  using L = SpecLayout<MODE, HANDLER, U, B, PER_ENV>;
+  constexpr int EPW = envs_per_warp(U);
+  constexpr int EPB = L::EPB;
+  constexpr int F = L::F;
   constexpr unsigned SEG = (U == 32) ? kFull : ((1u << U) - 1u);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   float* s_obs = m.obs;
@@ -333,22 +336,19 @@ template <int MODE, int HANDLER, int U, int B, bool PER_ENV, bool MC = false>
 __global__ void __launch_bounds__(kThreads, spec_min_blocks(MODE, HANDLER, B)) step_spec_kernel(const __grid_constant__ StepArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr bool GYM = (MODE == 1);
-  constexpr bool MA = (HANDLER == 1);
-  constexpr int EPB = (32 / U) * kWarpsPerBlock;
-  constexpr int F = GYM ? ((MA ? 4 : 2) * B + 1) : 0;
+  using L = SpecLayout<MODE, HANDLER, U, B, PER_ENV>;
+  constexpr int EPB = L::EPB;
   // Programmatic dependent launch: let the next launch in the stream become resident while this
   // grid drains, and (as the dependent) wait for the previous grid's memory before touching state.
   // Both are no-ops when the launch does not carry the attribute.
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   prefetch_ahead<EPB, U, GYM>(a);
   asm volatile("griddepcontrol.wait;" ::: "memory");
-  constexpr size_t OBS_BYTES = (((size_t)(GYM ? EPB * U * F * 4 : 0)) + 15) & ~(size_t)15;
-  constexpr size_t BS_BYTES = PER_ENV ? (size_t)EPB * B * 4 : 0;
   ChunkMem m = {};
   m.obs = reinterpret_cast<float*>(smem_raw);
-  m.bs = reinterpret_cast<uint32_t*>(smem_raw + OBS_BYTES);
-  m.bsu = reinterpret_cast<float*>(smem_raw + OBS_BYTES + BS_BYTES);
-  m.bsn = reinterpret_cast<int*>(smem_raw + OBS_BYTES + BS_BYTES + (size_t)EPB * B * 4);
+  m.bs = reinterpret_cast<uint32_t*>(smem_raw + L::BS);
+  m.bsu = reinterpret_cast<float*>(smem_raw + L::BSU);
+  m.bsn = reinterpret_cast<int*>(smem_raw + L::BSN);
   const int env_base = blockIdx.x * EPB;
   if (PER_ENV) {
     const int n = min(EPB, a.E - env_base) * B;
@@ -358,15 +358,6 @@ __global__ void __launch_bounds__(kThreads, spec_min_blocks(MODE, HANDLER, B)) s
   }
   step_chunk<MODE, HANDLER, U, B, PER_ENV, MC>(a, env_base, m);
   if (GYM) store_obs_block(a, m.obs, env_base, threadIdx.x, true);
-}
-
-// The instance of a shape for one BS class (MC = false) or several (MC = true), nullptr where none is
-// compiled: several classes need a shared layout, and WANTED = false leaves out a one-class case that
-// another kernel family always takes.
-template <int MODE, int HANDLER, int U, int B, bool PER_ENV, bool MC, bool WANTED = true>
-constexpr auto spec_kernel() -> void (*)(StepArgs) {
-  if constexpr (!WANTED || (MC && PER_ENV)) return nullptr;
-  else return step_spec_kernel<MODE, HANDLER, U, B, PER_ENV, MC>;
 }
 
 }  // namespace mbe

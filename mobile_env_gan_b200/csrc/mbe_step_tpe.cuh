@@ -47,6 +47,14 @@ struct TpeRolloutSmem : TpeForkSmem<U, B> {
   alignas(16) uint32_t wp_out[32 * U];   // waypoints after the move ((-1,-1): arrived this step, movement.py:54-56)
 };
 
+// the dynamic shared memory of an instance
+template <int U, int B, bool ROLLOUT>
+using TpeSmem = typename std::conditional<ROLLOUT, TpeRolloutSmem<U, B>, TpeForkSmem<U, B>>::type;
+
+// a CTA is one warp and owns as many consecutive envs, one per lane
+constexpr int kTpeThreads = 32;
+constexpr int kTpeEnvsPerCta = kTpeThreads;
+
 // the lane-strided accumulation + shfl_down tree of qoe_accumulate_kernel (mbe_step.cuh) for one env
 // on a thread-local array: lane 0's result after off = 16, 8, 4, 2, 1 with zeros in lanes >= U.
 // Adding those zeros only ever turns a -0 into +0, which no later sum can see, so they are skipped.
@@ -123,14 +131,14 @@ struct TpeCounts {
 };
 
 template <int U, int B, bool ROLLOUT = false, bool SHARED = false>
-__global__ void __launch_bounds__(32, ROLLOUT ? kTpeRolloutBlocks : kTpeBlocks) step_tpe_fork_kernel(const __grid_constant__ StepArgs a) {
+__global__ void __launch_bounds__(kTpeThreads, ROLLOUT ? kTpeRolloutBlocks : kTpeBlocks) step_tpe_fork_kernel(const __grid_constant__ StepArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  using S = typename std::conditional<ROLLOUT, TpeRolloutSmem<U, B>, TpeForkSmem<U, B>>::type;
+  using S = TpeSmem<U, B, ROLLOUT>;
   static_assert(B <= 16, "the nearest-BS key keeps the BS index in 4 bits");
   static_assert(U <= 32, "the QoE tree replays a 32-lane reduction");
   S& s = *reinterpret_cast<S*>(smem_raw);
   const int lane = threadIdx.x;
-  const size_t e0 = (size_t)blockIdx.x * 32;  // first env of this warp
+  const size_t e0 = (size_t)blockIdx.x * kTpeEnvsPerCta;  // first env of this warp
   const int env = (int)e0 + lane;
   const unsigned gid = a.env_offset + (unsigned)env;
   const SlotDev& C0 = a.slot[0];  // the single BS class

@@ -21,23 +21,27 @@ constexpr int kUptBlocks = 7;
 // warps per CTA of this mapping: 2 measured best (finer CTA granularity; 1 would break the 16-byte
 // size rule of the observation bulk store for U=15)
 constexpr int kUptWarps = 2;
+constexpr int kUptThreads = 32 * kUptWarps;
+
+// Envs per CTA of an instance and its dynamic shared memory, the observation staging block.
+template <int HANDLER, int U, int B, int K>
+struct UptLayout {
+  static constexpr int EPW = envs_per_warp(K);
+  static constexpr int EPB = EPW * kUptWarps;
+  static constexpr int F = (HANDLER == 1 ? 4 : 2) * B + 1;
+  static constexpr size_t BYTES = ((size_t)EPB * U * F * 4 + 15) & ~(size_t)15;
+};
 
 template <int HANDLER, int U, int B, int K>
-__host__ __device__ constexpr size_t upt_smem_bytes() {
-  constexpr int EPB = (32 / K) * kUptWarps;
-  constexpr int F = (HANDLER == 1 ? 4 : 2) * B + 1;
-  return (((size_t)EPB * U * F * 4) + 15) & ~(size_t)15;
-}
-
-template <int HANDLER, int U, int B, int K>
-__global__ void __launch_bounds__(32 * kUptWarps, kUptBlocks * 4 / kUptWarps) step_upt_kernel(const __grid_constant__ StepArgs a) {
+__global__ void __launch_bounds__(kUptThreads, kUptBlocks * 4 / kUptWarps) step_upt_kernel(const __grid_constant__ StepArgs a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   static_assert(U % K == 0, "U must be a multiple of K");
+  using L = UptLayout<HANDLER, U, B, K>;
   constexpr bool MA = (HANDLER == 1);
   constexpr int UPT = U / K;
-  constexpr int EPW = 32 / K;
-  constexpr int EPB = EPW * kUptWarps;
-  constexpr int F = (MA ? 4 : 2) * B + 1;
+  constexpr int EPW = L::EPW;
+  constexpr int EPB = L::EPB;
+  constexpr int F = L::F;
   constexpr int NW = (B + 3) / 4;  // packed count words (8 bits per BS)
   float* s_obs = reinterpret_cast<float*>(smem_raw);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -292,7 +296,7 @@ __global__ void __launch_bounds__(32 * kUptWarps, kUptBlocks * 4 / kUptWarps) st
     }
     if (k == 0) a.t[env] = t_e;
   }
-  store_obs_block<32 * kUptWarps>(a, s_obs, env_base, tid, true);
+  store_obs_block<kUptThreads>(a, s_obs, env_base, tid, true);
 }
 
 }  // namespace mbe

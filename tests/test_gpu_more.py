@@ -410,6 +410,131 @@ def test_step_kernel_name_reports_the_dispatched_family():
     assert generic.step_kernel_name == "step_kernel"
 
 
+def _dispatch_env(shape, mode, handler="central", classes=1, E=64, **extra):
+    """An env of one scenario shape ("custom": 7 UEs on per-env random layouts of 10 slots); classes=2
+    gives BS 1 a lower transmit power, i.e. a second BS class."""
+    from mobile_env_gan_b200.core.base import MComCore
+    from mobile_env_gan_b200.core.entities import BaseStation, UserEquipment
+    from mobile_env_gan_b200.core.util import deep_dict_merge
+    from test_gpu_parity import SCENARIOS
+
+    config = dict({"num_envs": E, "mode": mode, "handler": handler}, **extra)
+    if shape == "custom":
+        bs, U = [], 7
+        config.update({"bs_random": (5, 10), "max_bs": 10, "ue": {"velocity": 10}})
+    else:
+        bs, U = SCENARIOS[shape]
+    cfg = deep_dict_merge(MComCore.default_config(), config)
+    stations = [BaseStation(i, tuple(xy), **dict(cfg["bs"], **({"tx": 30} if classes == 2 and i == 1 else {})))
+                for i, xy in enumerate(bs)]
+    env = MComCore(stations, [UserEquipment(i, **cfg["ue"]) for i in range(U)], config)
+    assert len(env.plan.classes) == classes
+    return env
+
+
+def _step_kernels_launched(fn):
+    """The libmbe step kernels fn launches, as 'name<template arguments>' without casts or blanks."""
+    import re
+
+    from torch.profiler import ProfilerActivity, profile
+
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    found = set()
+    for ev in prof.events():
+        m = re.search(r"mbe::(step_\w+<[^>]*>)", ev.name)
+        if m:
+            name = re.sub(r"\s+|\(int\)", "", m.group(1))
+            found.add(name.replace("(bool)0", "false").replace("(bool)1", "true"))
+    return found
+
+
+def _shape(shape, mode, **kw):
+    return lambda: _dispatch_env(shape, mode, **kw)
+
+
+def _debug_snr_custom():
+    from mobile_env_gan_b200.scenarios.custom import MComCustom
+
+    env = MComCustom(config={"num_envs": 64})
+    env.enable_debug_snr()  # the debug SNR output only exists in the generic kernel
+    return env
+
+
+def _registered(env_id, E=64, **config):
+    import mobile_env_gan_b200 as mbe
+
+    return lambda: mbe.make(env_id, num_envs=E, config=config)
+
+
+def _proportional_fair():
+    from mobile_env_gan_b200.core.schedules import ProportionalFair
+
+    return _registered("mobile-medium-central-v0", scheduler=ProportionalFair)()
+
+
+# (env factory, kernel of one step, kernel of a 2-step rollout or None for GYM).  One case per compiled
+# whole-step or fused-episode instance, then the calls that fall back to another instance or family.
+_SPEC = "step_spec_kernel<{},{},{},{},{},{}>"
+_DISPATCH_CASES = {
+    # thread per env: MComCustom's step and episode; the scenario shapes' FORK episodes
+    "custom-fork": (_shape("custom", "fork"), "step_tpe_fork_kernel<7,10,false,false>",
+                    "step_tpe_fork_kernel<7,10,true,false>"),
+    "small-fork": (_shape("small", "fork"), _SPEC.format(0, 0, 5, 3, "false", "false"),
+                   "step_tpe_fork_kernel<5,3,true,true>"),
+    "medium-fork": (_shape("medium", "fork"), _SPEC.format(0, 0, 15, 4, "false", "false"),
+                    "step_tpe_fork_kernel<15,4,true,true>"),
+    # UEs per thread
+    "medium-gym-central": (_shape("medium", "gym"), "step_upt_kernel<0,15,4,5>", None),
+    "medium-gym-ma": (_shape("medium", "gym", handler="ma"), "step_upt_kernel<1,15,4,5>", None),
+    # warp segment, shared layouts, one BS class
+    "small-gym-central": (_shape("small", "gym"), _SPEC.format(1, 0, 5, 3, "false", "false"), None),
+    "small-gym-ma": (_shape("small", "gym", handler="ma"), _SPEC.format(1, 1, 5, 3, "false", "false"), None),
+    "large-gym-central": (_shape("large", "gym"), _SPEC.format(1, 0, 30, 13, "false", "false"), None),
+    "large-gym-ma": (_shape("large", "gym", handler="ma"), _SPEC.format(1, 1, 30, 13, "false", "false"), None),
+    "large-fork": (_shape("large", "fork"), _SPEC.format(0, 0, 30, 13, "false", "false"),
+                   _SPEC.format(0, 0, 30, 13, "false", "false")),
+    # warp segment, shared layouts, several BS classes (no one-class episode applies)
+    **{f"{s}-gym-{h}-2cls": (_shape(s, "gym", handler=h, classes=2), _SPEC.format(1, int(h == "ma"), U, B, "false", "true"),
+                             None)
+       for s, U, B in (("small", 5, 3), ("medium", 15, 4), ("large", 30, 13)) for h in ("central", "ma")},
+    **{f"{s}-fork-2cls": (_shape(s, "fork", classes=2), _SPEC.format(0, 0, U, B, "false", "true"),
+                          _SPEC.format(0, 0, U, B, "false", "true"))
+       for s, U, B in (("small", 5, 3), ("medium", 15, 4), ("large", 30, 13))},
+    # warp segment, per-env layouts; FORK with E % 32 != 0 (the thread-per-env kernels take whole warps)
+    "custom-fork-40": (_shape("custom", "fork", E=40), _SPEC.format(0, 0, 7, 10, "true", "false"),
+                       _SPEC.format(0, 0, 7, 10, "true", "false")),
+    "custom-gym-central": (_shape("custom", "gym"), _SPEC.format(1, 0, 7, 10, "true", "false"), None),
+    "custom-gym-ma": (_shape("custom", "gym", handler="ma"), _SPEC.format(1, 1, 7, 10, "true", "false"), None),
+    # fallbacks: no fused episode without whole warps, block-per-env, generic
+    "small-fork-40": (_shape("small", "fork", E=40), _SPEC.format(0, 0, 5, 3, "false", "false"),
+                      _SPEC.format(0, 0, 5, 3, "false", "false")),
+    "synthetic": (_registered("mobile-synthetic-central-v0", E=4), "step_big_kernel<1,0,2>", None),
+    "medium-proportional-fair": (_proportional_fair, "step_big_kernel<1,0,2>", None),
+    "custom-debug-snr": (_debug_snr_custom, "step_kernel<0,0>", "step_kernel<0,0>"),
+    "medium-generic-flag": (_registered("mobile-medium-central-v0", generic_kernel=True), "step_kernel<1,0>", None),
+}
+
+
+@pytest.mark.parametrize("case", list(_DISPATCH_CASES))
+def test_step_and_rollout_launch_the_dispatched_instance(case):
+    """The kernel instance, template arguments included, that one step (and a FORK rollout) launches."""
+    from mobile_env_gan_b200 import _lib
+
+    factory, step_kernel, rollout_kernel = _DISPATCH_CASES[case]
+    env = factory()
+    env.reset()
+    assert step_kernel.startswith(env.step_kernel_name + "<")
+    if env.plan.mode == _lib.MODE_GYM:
+        actions = torch.zeros((env.num_envs, env.NUM_USERS), dtype=torch.int32, device=env.device)
+        assert _step_kernels_launched(lambda: env.step(actions)) == {step_kernel}
+    else:
+        assert _step_kernels_launched(lambda: env.step(0, 0)) == {step_kernel}
+        assert _step_kernels_launched(lambda: env.rollout(2)) == {rollout_kernel}
+
+
 def test_fork_step_window_ragged_tail_and_tiny_window():
     """A window that is not a whole number of 32-env warps (or holds fewer than 32 envs) must still
     step exactly its envs: the thread-per-env FORK kernel only takes whole warps, so such windows
