@@ -7,6 +7,7 @@ whole 20-step epoch is one kernel launch (mbe_rollout) and the score statistics 
     torchrun --nproc-per-node 8 examples/layout_search.py --layouts 8388608   # layouts sharded over the GPUs
     python examples/layout_search.py --layouts 1048576 --generations 50       # genetic search (LayoutEvolution)
     python examples/layout_search.py --layouts 65536 --generations 10 --trajectories 8 --holdout 1024
+    python examples/layout_search.py --layouts 65536 --generations 10 --holdout 1024 --map-stride 4
 
 Multi-GPU: every rank scores its own contiguous slice of the global layout range (Philox layouts are
 keyed by the global env id, so the candidates do not depend on the number of GPUs); the only exchange
@@ -21,7 +22,9 @@ the ranks' winners are gathered as above.
 random rounds and in the genetic search: layout l runs in the M env rows l*M .. l*M + M-1 and its score is
 the notebook's qoeValue over the QoE values of all M episodes (DESIGN.md section 10).  --holdout M' then
 re-scores the final top layouts on M' trajectories of another movement seed (--holdout-seed) that the
-search never saw, and prints the training score next to the held-out score.
+search never saw, and prints the training score next to the held-out score.  --map-stride S adds each
+top layout's map statistics over every S-th map point (DESIGN.md section 10.2): the score of a UE alone
+at each point, the share of points with at least one and with at least two connectable BSs.
 """
 import argparse
 import os
@@ -48,6 +51,8 @@ def main():
                     "held-out trajectories (a power of two)")
     ap.add_argument("--holdout-seed", type=int, default=1, help="scenario seed of the held-out trajectories "
                     "(the search runs MComCustom's default seed)")
+    ap.add_argument("--map-stride", type=int, default=0, help="> 0: print the top layouts' map statistics "
+                    "(coverage, overlap, map score) over the grid of this stride")
     args = ap.parse_args()
     M = args.trajectories
     world, rank, local = (int(os.environ.get(k, d)) for k, d in (("WORLD_SIZE", 1), ("RANK", 0), ("LOCAL_RANK", 0)))
@@ -103,25 +108,34 @@ def gather_rows(rows, world):
 
 
 def report(best, args, env, rank):
-    """Prints the top layouts (rank 0), with --holdout their scores on held-out trajectories beside."""
+    """Prints the top layouts (rank 0), with --holdout their scores on held-out trajectories beside, and with
+    --map-stride their map statistics (LayoutScorer.map_result: map score, coverage, overlap)."""
     if rank != 0:
         return
-    if args.holdout <= 0:
+    if args.holdout <= 0 and args.map_stride <= 0:
         for s, xy in best:
             print(f"{s:+.4f}  {xy}")
         return
-    K, Mh, B = len(best), args.holdout, env.plan.num_bs
+    K, Mh, B = len(best), max(args.holdout, 1), env.plan.num_bs
     held = MComCustom(config={"device": env.device, "seed": args.holdout_seed, "num_envs": K * Mh,
                               "num_trajectories": Mh})
     xy = torch.zeros(K, B, 2, dtype=torch.int16)
     for i, (_, pts) in enumerate(best):
         xy[i, :len(pts)] = torch.tensor(pts, dtype=torch.int16)
     nbs = torch.tensor([len(pts) for _, pts in best], dtype=torch.int32)
-    score = LayoutScorer(held).score_layouts(xy, nbs).cpu().tolist()
-    print(f"training score ({args.trajectories} trajectories) | held-out score ({Mh} trajectories, "
-          f"seed {args.holdout_seed}) | layout")
-    for (s, pts), h in zip(best, score):
-        print(f"{s:+.4f}  {h:+.4f}  {pts}")
+    scorer = LayoutScorer(held)
+    score = scorer.score_layouts(xy, nbs).cpu().tolist()  # also writes layout l into rows l*Mh ..
+    head, cols = [f"training score ({args.trajectories} trajectories)"], [[s for s, _ in best]]
+    if args.holdout > 0:
+        head.append(f"held-out score ({Mh} trajectories, seed {args.holdout_seed})")
+        cols.append(score)
+    if args.map_stride > 0:
+        r = scorer.map_result(stride=args.map_stride)
+        head += [f"map score (stride {args.map_stride})", "coverage", "overlap"]
+        cols += [r["Score"].cpu().tolist(), r["Coverage"].cpu().tolist(), r["Overlap"].cpu().tolist()]
+    print(" | ".join(head) + " | layout")
+    for i, (_, pts) in enumerate(best):
+        print("  ".join(f"{c[i]:+.4f}" for c in cols) + f"  {pts}")
 
 
 def evolve(env, args, world, rank, total):

@@ -179,7 +179,8 @@ int mbe_abi_version(void);
 const char* mbe_build_info(void);
 const char* mbe_last_error(void);
 /* sizeof of the ABI structs as the library was compiled (0 mbe_config, 1 mbe_buffers, 2 mbe_link_class,
- * 3 mbe_ue_class, 4 mbe_rollout_out, 5 mbe_render_style, 6 mbe_evolve_params; -1 otherwise): lets a
+ * 3 mbe_ue_class, 4 mbe_rollout_out, 5 mbe_render_style, 6 mbe_evolve_params, 7 mbe_map_params; -1
+ * otherwise): lets a
  * binding in another language check its layout */
 int mbe_struct_size(int which);
 
@@ -276,6 +277,36 @@ typedef struct mbe_evolve_params {
 int mbe_evolve_layouts(mbe_env* env, const float* fitness, const int16_t* parent_xy, const int32_t* parent_nbs,
                        const int32_t* elite_ids, int n_elite, const mbe_evolve_params* p, int16_t* child_xy,
                        int32_t* child_nbs, void* stream);
+
+/* Layout maps (DESIGN.md section 10.2) of envs env_ids[0..n) (DEVICE int32, NULL = envs 0..n-1), with the
+ * layout the step kernels see: the coordinates a shared layout had at mbe_bind, or the bound bs_xy[e] with
+ * the live slots b < clamp(nbs[e], 0, B).  The grid points are (x, y) = (i*stride, j*stride) with
+ * 0 <= x <= XM = ceil(width) - 1 and 0 <= y <= YM = ceil(height) - 1 (the range UE positions are drawn
+ * from): GX = XM / stride + 1 columns, GY = YM / stride + 1 rows, row j is y = j*stride (y ascends with the
+ * row, unlike a render frame), point index j*GX + i.  Per point, with d2 the exact integer squared
+ * distance to a live BS and a BS connectable iff d2 <= d2max of link class (bs_class[b], ue_class):
+ *   coverage  uint8 [n, GY, GX]  connectable BSs, saturated at 255;
+ *   serving   int8  [n, GY, GX]  the connectable BS of smallest d2, ties to the lower slot (the FORK
+ *                                association), -1 = none;
+ *   qoe       int8  [n, GY, GX]  the cent k in [-100, 100] of a UE served there that shares its BS with
+ *                                load - 1 others: the exact half-even rounding of 100 * scaled utility
+ *                                (FP32, as the step kernels compute it) of the rate
+ *                                nearbyint(rate_lut[d2] / load * 100) / 100 (FP64); -100 without a server.
+ * stats int64 [n, 6] = (points, covered (>= 1 BS), overlap (>= 2 BSs), sum k, sum k^2, low), where a point is
+ * low iff float32(k / 100) < float32(threshold), the test of mbe_accumulate_qoe; area int32 [n, B] = points
+ * each slot serves.  An env id outside 0..E-1 gives zero stats and area, coverage 0, serving -1, qoe -128.
+ * Every output may be NULL; stats 8-byte and area 4-byte aligned (DEVICE).  Two launches; leaves every bound
+ * buffer untouched. */
+typedef struct mbe_map_params {
+  int32_t stride;   /* grid step in map units, >= 1 */
+  int32_t ue_class; /* UE class of the map's UE, 0..num_ue_classes-1 */
+  int32_t load;     /* UEs sharing the serving BS, >= 1 */
+  int32_t reserved;
+  float threshold;  /* low-QoE threshold, finite */
+} mbe_map_params;
+
+int mbe_layout_map(mbe_env* env, const int32_t* env_ids, int n, const mbe_map_params* p, int64_t* stats,
+                   int32_t* area, uint8_t* coverage, int8_t* serving, int8_t* qoe, void* stream);
 
 /* number of kernel launches this handle has enqueued so far */
 int64_t mbe_launch_count(const mbe_env* env);

@@ -124,6 +124,13 @@ class EvolveParams(C.Structure):
                 ("p_del", C.c_double)]
 
 
+class MapParams(C.Structure):
+    """mbe_map_params: grid stride, the map UE's class, UEs sharing the serving BS, low-QoE threshold."""
+
+    _fields_ = [("stride", C.c_int32), ("ue_class", C.c_int32), ("load", C.c_int32), ("reserved", C.c_int32),
+                ("threshold", C.c_float)]
+
+
 # every symbol include/mbe.h declares: (name, restype, argtypes)
 SYMBOLS = [
     ("mbe_abi_version", C.c_int, []),
@@ -145,6 +152,8 @@ SYMBOLS = [
                              C.POINTER(RenderStyle), C.c_void_p, C.c_void_p]),
     ("mbe_evolve_layouts", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                      C.POINTER(EvolveParams), C.c_void_p, C.c_void_p, C.c_void_p]),
+    ("mbe_layout_map", C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(MapParams), C.c_void_p, C.c_void_p,
+                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     ("mbe_launch_count", C.c_int64, [C.c_void_p]),
     ("mbe_step_kernel_name", C.c_char_p, [C.c_void_p]),
     ("mbe_step_host", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -174,7 +183,8 @@ def load():
         fn.argtypes = args
     if lib.mbe_abi_version() != MBE_ABI_VERSION:
         raise MbeError(f"libmbe ABI {lib.mbe_abi_version()} != binding {MBE_ABI_VERSION}")
-    for which, struct in enumerate((Config, Buffers, BsClass, UeClass, RolloutOut, RenderStyle, EvolveParams)):
+    for which, struct in enumerate((Config, Buffers, BsClass, UeClass, RolloutOut, RenderStyle, EvolveParams,
+                                          MapParams)):
         if lib.mbe_struct_size(which) != C.sizeof(struct):
             raise MbeError(f"struct layout mismatch: {struct.__name__} is {C.sizeof(struct)} bytes here, "
                            f"{lib.mbe_struct_size(which)} in {LIB_PATH}")

@@ -17,6 +17,7 @@ Two step semantics behind one kernel set (SURVEY.md section 0):
 from __future__ import annotations
 
 import ctypes as C
+import math
 import os
 from dataclasses import dataclass, field
 from typing import Dict, List, Optional
@@ -36,6 +37,32 @@ from .util import deep_dict_merge
 from .utilities import BoundedLogUtility
 
 MAX_COORD = 32767
+
+
+@dataclass
+class LayoutMap:
+    """What ``MComCore.layout_map`` computed, as device tensors (DESIGN.md section 10.2): ``stats`` int64
+    ``[n, 6]`` = (points, covered, overlap, sum k, sum k^2, low) and ``area`` int32 ``[n, B]`` per requested
+    env, and with ``maps`` the grids ``coverage`` uint8, ``serving`` int8 and ``qoe`` int8 ``[n, GY, GX]``,
+    row j at y = j * stride, column i at x = i * stride."""
+
+    stats: torch.Tensor
+    area: torch.Tensor
+    coverage: Optional[torch.Tensor]
+    serving: Optional[torch.Tensor]
+    qoe: Optional[torch.Tensor]
+
+    def result(self, weights=(1.0, 0.1, 10.0)):
+        """Per env dict of FP64 tensors: ``LayoutScorer.result()``'s keys over the map's QoE values
+        k / 100 (``Score`` with ``weights``), plus ``Coverage`` and ``Overlap``, the shares of the points
+        with at least one and at least two connectable BSs."""
+        pts, cov, ovl, sk, sk2, low = self.stats.double().unbind(dim=1)
+        mean = sk / (100 * pts)
+        var = sk2 / (10000 * pts) - mean * mean
+        p = low / pts
+        w1, w2, w3 = weights
+        return {"Average QoE": mean, "QoE Variance": var, "Low QoE Proportion": p,
+                "Score": w1 * mean - w2 * var - w3 * p, "Coverage": cov / pts, "Overlap": ovl / pts}
 
 
 @dataclass
@@ -682,6 +709,32 @@ class MComCore:
                                         None if ro is None else C.byref(ro), int(steps), C.byref(st),
                                         C.c_void_p(out.data_ptr()), self._stream()))
         return out if series is not None else out[0]
+
+    def layout_map(self, envs=None, *, stride: int = 1, load: int = 1, ue_class: int = 0, threshold: float = 0.0,
+                   maps: bool = True) -> LayoutMap:
+        """Coverage, serving BS and QoE cent at every ``stride``-th integer map point of the BS layout of
+        ``envs`` (index tensor or list, default all; an id outside 0..E-1 gives an empty map and zero
+        statistics), and their map-wide statistics, in two launches (``mbe_layout_map``, DESIGN.md section
+        10.2).  ``load``: UEs sharing the serving BS (1 = a UE alone); ``ue_class``: the map UE's class;
+        ``threshold``: the low-QoE threshold of ``LayoutScorer``; ``maps=False``: statistics only."""
+        if envs is None:
+            n, ids = self.num_envs, None
+        else:
+            ids = torch.as_tensor(envs).to(device=self.device, dtype=torch.int32).reshape(-1).contiguous()
+            n = ids.numel()
+        gx = (math.ceil(self.plan.width) - 1) // max(int(stride), 1) + 1
+        gy = (math.ceil(self.plan.height) - 1) // max(int(stride), 1) + 1
+        dev = self.device
+        out = LayoutMap(torch.empty(n, 6, dtype=torch.int64, device=dev),
+                        torch.empty(n, self.plan.num_bs, dtype=torch.int32, device=dev),
+                        *((torch.empty(n, gy, gx, dtype=dt, device=dev) if maps else None)
+                          for dt in (torch.uint8, torch.int8, torch.int8)))
+        ptr = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
+        prm = _lib.MapParams(stride=int(stride), ue_class=int(ue_class), load=int(load), threshold=float(threshold))
+        _lib.check(self._lib.mbe_layout_map(self._handle, ptr(ids), int(n), C.byref(prm), ptr(out.stats),
+                                            ptr(out.area), ptr(out.coverage), ptr(out.serving), ptr(out.qoe),
+                                            self._stream()))
+        return out
 
     @property
     def launch_count(self) -> int:

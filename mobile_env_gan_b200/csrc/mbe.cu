@@ -20,6 +20,7 @@
 #include "mbe_step_tpe.cuh"
 #include "mbe_render.cuh"
 #include "mbe_evolve.cuh"
+#include "mbe_map.cuh"
 
 namespace {
 
@@ -89,6 +90,7 @@ struct mbe_env {
   // kernels of this shape in priority order (see pick).  episode: the fused rollout (fn == nullptr: none).
   StepKernel general, episode;
   std::vector<StepKernel> steps;
+  uint32_t bound_xy[mbe::kMapMaxB] = {};  // a shared layout as mbe_bind read it (int16 pairs), for layout maps
   bool prefetch_ok = false;  // the prefetched streams (pos, wp, conn, actions) are 16-byte aligned
   // mbe_step_host pipeline: second stream + fork/join events (created on first use)
   cudaStream_t host_stream = nullptr;
@@ -248,6 +250,7 @@ int mbe_struct_size(int which) {
     case 4: return (int)sizeof(mbe_rollout_out);
     case 5: return (int)sizeof(mbe_render_style);
     case 6: return (int)sizeof(mbe_evolve_params);
+    case 7: return (int)sizeof(mbe_map_params);
     default: return -1;
   }
 }
@@ -566,6 +569,7 @@ int mbe_bind(mbe_env* env, const mbe_buffers* b) {
       a.slot[i].xf = (float)xy[2 * i];
       a.slot[i].yf = (float)xy[2 * i + 1];
     }
+    for (int i = 0; i < a.B; ++i) env->bound_xy[i] = (uint16_t)xy[2 * i] | ((uint32_t)(uint16_t)xy[2 * i + 1] << 16);
   }
   env->bound = true;
   return 0;
@@ -831,6 +835,78 @@ int mbe_evolve_layouts(mbe_env* env, const float* fitness, const int16_t* parent
   MBE_CUDA(cudaGetLastError());
   env->launches += 1;
   return 0;
+}
+
+int mbe_layout_map(mbe_env* env, const int32_t* env_ids, int n, const mbe_map_params* p, int64_t* stats,
+                   int32_t* area, uint8_t* coverage, int8_t* serving, int8_t* qoe, void* stream) {
+  static_assert(mbe::kMapMaxB == mbe::kBigMaxB, "a layout map stages every BS slot of a handle");
+  if (!env) return fail("mbe_layout_map: null handle");
+  if (!env->bound) return fail("mbe_bind has not been called");
+  if (!p) return fail("mbe_layout_map: null params");
+  const mbe::StepArgs& s = env->args;
+  if (n < 0) return fail("mbe_layout_map: n=%d must be >= 0", n);
+  if (p->stride < 1) return fail("mbe_layout_map: stride=%d must be >= 1", p->stride);
+  if (p->load < 1) return fail("mbe_layout_map: load=%d must be >= 1", p->load);
+  if (p->ue_class < 0 || p->ue_class >= s.n_ue_classes)
+    return fail("mbe_layout_map: ue_class=%d outside 0..%d", p->ue_class, s.n_ue_classes - 1);
+  if (!std::isfinite(p->threshold)) return fail("mbe_layout_map: threshold must be finite");
+  if ((uintptr_t)stats & 7) return fail("mbe_layout_map: stats must be 8-byte aligned");
+  if ((uintptr_t)area & 3) return fail("mbe_layout_map: area must be 4-byte aligned");
+  if (n == 0) return 0;
+  const mbe_config& cfg = env->cfg;
+  mbe::MapArgs m = {};
+  m.bs_xy = s.bs_per_env ? s.bs_xy : nullptr;
+  m.nbs = s.nbs;
+  m.env_ids = env_ids;
+  m.bs_class = s.bs_class;
+  m.stats = reinterpret_cast<long long*>(stats);
+  m.area = area;
+  m.coverage = coverage;
+  m.serving = serving;
+  m.qoe = qoe;
+  m.E = s.E, m.B = s.B, m.n = n, m.s = p->stride;
+  const int XM = (int)std::ceil(cfg.width) - 1, YM = (int)std::ceil(cfg.height) - 1;
+  m.GX = XM / p->stride + 1;
+  const int GY = YM / p->stride + 1;
+  m.G = m.GX * GY;  // <= 32767^2
+  m.bands = (m.G + mbe::kMapPoints - 1) / mbe::kMapPoints;
+  if ((long long)n * m.bands > 0x7fffffffll) return fail("mbe_layout_map: %lld CTAs exceed one launch", (long long)n * m.bands);
+  // a cent k is low iff float32(k / 100) < float32(threshold); float32(k / 100) increases with k
+  m.k_low = 101;
+  for (int k = 100; k >= -100; --k)
+    if ((float)((double)k / 100.0) >= p->threshold) m.k_low = k;
+  m.vec = m.G % 4 == 0 && (((uintptr_t)coverage | (uintptr_t)serving | (uintptr_t)qoe) & 3) == 0;
+  m.n_classes = cfg.num_classes;
+  m.load = (double)p->load;
+  long long tab = 0;
+  for (int c = 0; c < cfg.num_classes; ++c) {
+    m.link[c] = c * s.n_ue_classes + p->ue_class;
+    m.d2max[c] = s.cls[m.link[c]].d2max;
+    m.off[c] = (int)tab;
+    if (m.d2max[c] >= 0) tab += (long long)m.d2max[c] + 1;
+    if (tab > 0x7fffffffll) return fail("mbe_layout_map: cent table of %lld entries is too large", tab);
+  }
+  m.tab_len = (int)tab;
+  std::memcpy(m.xy, env->bound_xy, sizeof m.xy);
+  MBE_ON_DEVICE(cfg.device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (m.tab_len > 0) MBE_CUDA(cudaMallocAsync((void**)&m.cent, (size_t)m.tab_len, st));
+  const long long prep = std::max({(long long)m.tab_len, stats ? (long long)n * mbe::kMapStats : 0ll,
+                                   area ? (long long)n * m.B : 0ll});
+  int rc = 0;
+  if (prep > 0) {
+    mbe::map_prep_kernel<<<(unsigned)((prep + mbe::kMapThreads - 1) / mbe::kMapThreads), mbe::kMapThreads, 0, st>>>(
+        s, m);
+    env->launches += 1;
+    if (cudaError_t e = cudaGetLastError()) rc = fail("mbe_layout_map: map_prep_kernel: %s", cudaGetErrorString(e));
+  }
+  if (rc == 0) {
+    mbe::map_kernel<<<(unsigned)(n * m.bands), mbe::kMapThreads, 0, st>>>(m);
+    env->launches += 1;
+    if (cudaError_t e = cudaGetLastError()) rc = fail("mbe_layout_map: map_kernel: %s", cudaGetErrorString(e));
+  }
+  if (m.cent) MBE_CUDA(cudaFreeAsync(m.cent, st));
+  return rc;
 }
 
 int64_t mbe_launch_count(const mbe_env* env) { return env ? env->launches : 0; }

@@ -317,6 +317,18 @@ __device__ __forceinline__ float qoe_cent_value(float u) {
   return fmaf(fmaf(-q0, 100.0f, k), 0.01f, q0);
 }
 
+// The cent k itself, as an integer: the same exact half-even rounding of u * 100 as qoe_cent_value
+// (layout maps, mbe_map.cuh, tabulate it per squared distance).
+__device__ __forceinline__ int qoe_cent(float u) {
+  const float p = __fmul_rn(u, 100.0f);
+  float k = rintf(p);
+  if (fabsf(p - k) == 0.5f) {
+    const float e = fmaf(u, 100.0f, -p);
+    if (e != 0.0f) k = p + copysignf(0.5f, e);
+  }
+  return (int)k;
+}
+
 // mean over the connected UEs (metrics.py:18-21): 0 when nobody is connected
 __device__ __forceinline__ float mean_or_zero(float sum, float n) { return n > 0.0f ? __fdividef(sum, n) : 0.0f; }
 

@@ -96,6 +96,16 @@ class LayoutScorer:
         top = torch.topk(score, k)
         return top.indices, top.values
 
+    def map_result(self, stride: int = 1, load: int = 1, ue_class: int = 0):
+        """Map statistics of every layout (``MComCore.layout_map`` of env row l*M for layout l: all M replica
+        rows hold the same layout): dict of FP64 tensors [num_layouts] with ``result()``'s keys, over the
+        grid points instead of the trajectories, plus ``Coverage`` and ``Overlap``; same threshold and
+        weights."""
+        env = self.env
+        rows = torch.arange(0, env.num_envs, self.M, dtype=torch.int32, device=env.device)
+        m = env.layout_map(rows, stride=stride, load=load, ue_class=ue_class, threshold=self.threshold, maps=False)
+        return m.result(self.weights)
+
     def score_layouts(self, bs_xy, nbs):
         """Scores ``num_layouts`` given layouts, bs_xy int [L, B, 2] / nbs int [L], with one episode:
         resets the env and the statistics, writes layout l into its M replica rows, runs the episode
